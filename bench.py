@@ -9,7 +9,10 @@ forward field w_n streamed to HBM) + residual + 5000 adjoint steps with the imag
 scaling: every rank runs its own shots (BASELINE config 3's shot-parallel layout) and the timed region ends with
 the NCCL all-reduce of the gradient.  `value` counts wavefield point-updates (2 * nt * nz * nx per shot).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--nt 5000] [--grid 1000x3000]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--nt 5000] [--grid 1000x3000] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the timed steps computed, the FWI gradient summed over their shots, as DIR/gradient.npy
+(float32), so that two builds can be compared output for output; the inputs depend only on the arguments.
 
 Extra objects in the same JSON line:
   track_a        the reference-pinned Monte-Carlo source inversion (BASELINE configs 1 and 5), with its own reference
@@ -59,7 +62,28 @@ def parse():
                          "GPU ~5 %% slower for a few seconds (SM clocks and throttle reasons unchanged); see DESIGN 5")
     ap.add_argument("--force-dist", action="store_true", help="diagnostic: initialise NCCL even with one rank")
     ap.add_argument("--no-graphs", action="store_true", help="diagnostic: individual launches instead of CUDA-graph replay of the time loops")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the gradient of the timed steps to DIR/gradient.npy (a fixed sample of it above %d MB)" % (DUMP_LIMIT >> 20))
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 arm")
+    return args
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy.  Arrays over their share of DUMP_LIMIT are replaced by the same seeded
+    sample of their elements on every run (flat, in index order)."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT // len(arrays)
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.unique(np.random.default_rng(0).integers(0, a.size, share // a.itemsize))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload(args):
@@ -619,6 +643,8 @@ def run_b200(args):
         dist.all_reduce(grad)                       # one FWI gradient = sum over every rank's shots
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"gradient": grad.cpu().numpy()})
     ms = marks[0].elapsed_time(e1)
     shot_ms = [marks[k].elapsed_time(marks[k + 1]) for k in range(args.steps)]
     launches = prop.launch_count() - l0

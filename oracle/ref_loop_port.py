@@ -6,8 +6,8 @@ script that cannot be imported, and /root/reference does not exist on the GPU bo
 times THIS restatement there.  Unlike oracle/mc_oracle.py (vectorised, ~3x faster than the reference) this file keeps
 the reference's OPERATION STRUCTURE, because that structure is what its speed is made of:
   * the sampler makes the same scalar NumPy / `random` calls in the same order (FWI:448-510, 320-331, 226-232, 206-208),
-    so with the same seeds it produces the reference's samples bit for bit (checked against the live reference by
-    tests/test_ref_loop_port.py whenever /root/reference is present);
+    so with the same seeds it produces the reference's samples bit for bit (tests/test_ref_loop_port.py replays the
+    draws stored with the reference's results in tests/golden/track_a_reference.npz);
   * the forward model is the K x C double loop of slice multiply-adds (FWI:260-263);
   * the misfit is one VR call per trace, three NumPy reductions each, then np.average (FWI:664-668, 682, 512-520);
   * likelihood and Bayes normalisation as FWI:774, 811, 847-848; worker fan-out as FWI:822-830 (one OS process per
