@@ -43,58 +43,20 @@ struct Step2DArgs {
     float* rec_out;
 };
 
-#ifndef FWI_PREFETCH_ROW0
 // rows of u_{n-1} / m requested before the dependency wait.  ms per 1000-step gradient at 1000x3000: 0 rows 17.0, 1 row
 // 16.2, 2 rows 16.0 (80 registers, still 6 CTAs per SM); prefetching the adjoint's snapshot row as well: 16.5 - 19.0
-#define FWI_PREFETCH_ROW0 2
-#endif
-#ifndef FWI_PDL_TRIGGER
-// Where a step lets its successor's CTAs become resident: 0 = implicit, when its own CTAs exit (default), 1 = top,
-// 2 = after the dense part, 3 = after the TMA wait.  Measured on the bench workload (ms per 5000-step gradient):
-// no PDL 85.5, 0: 84.5, 2: 88.6, 1: 101 - an early trigger parks the whole next grid at its dependency wait and releases
-// all CTAs in the same instant, which lines up their load / compute / store phases and costs L2 bandwidth; with the
-// implicit trigger only the launch latency and the prologue overlap and the CTAs stay staggered.
-#define FWI_PDL_TRIGGER 0
-#endif
-#ifndef FWI_ROW_PIPE
-// rows of u_{n-1} / m requested AHEAD of the row being computed (rolling, on top of FWI_PREFETCH_ROW0 = depth).  Without it the
-// loads of row r + 1 sit behind the store of row r in program order (the compiler cannot prove the rows disjoint), so a warp
-// pays one L2 round trip per row.  0 = off
-#define FWI_ROW_PIPE 0
-#endif
-#ifndef FWI_L1_PREFETCH
-// rows of u_{n-1} / m (beyond the FWI_PREFETCH_ROW0 rows held in registers) requested into L1 with prefetch.global.L1 before the
-// dependency wait: no registers, and the row loop's loads then hit L1 instead of paying an L2 round trip each.  0 = off
-#define FWI_L1_PREFETCH 0
-#endif
-#ifndef FWI_STEP_MINB
-#define FWI_STEP_MINB 0           // > 0: __launch_bounds__ min CTAs per SM of the step kernel (caps the registers)
-#endif
-#if FWI_STEP_MINB > 0
-#define FWI_STEP_BOUNDS(nthreads) __launch_bounds__(nthreads, FWI_STEP_MINB)
-#else
-// no minimum given: ptxas settles at 80 registers (3 CTAs of 256 threads per SM); with an explicit minimum of 1 it takes 110
-#define FWI_STEP_BOUNDS(nthreads) __launch_bounds__(nthreads)
-#endif
-#ifndef FWI_M_SMEM
-// 1: the tile's rows of m (static inside a sweep) are staged in shared memory by a TMA load issued BEFORE the dependency wait
-#define FWI_M_SMEM 0
-#endif
-constexpr size_t step_tile_floats(int bz) { return ((size_t)(128 + 2 * kHalo) * (bz + 2 * kHalo) + 31) / 32 * 32; }    // [SZ][SX] rounded up to a 128-byte multiple
+constexpr int kPrefetchRows = 2;
+// The PDL trigger is left implicit (when this grid's CTAs exit): an explicit early griddepcontrol.launch_dependents parks the
+// whole next grid at its dependency wait and releases all CTAs in the same instant, which lines up their load / compute /
+// store phases and costs L2 bandwidth (ms per 5000-step gradient: no PDL 85.5, implicit 84.5, after the dense part 88.6,
+// at the top 101).
+// No minimum-blocks bound: ptxas settles at 80 registers (3 CTAs of 256 threads per SM); with an explicit minimum of 1 it takes 110.
 template <int BZ, int NW, int MODE>
-__global__ void FWI_STEP_BOUNDS(NW * 32) fd2d_step_kernel(const __grid_constant__ CUtensorMap tm_cur,
-#if FWI_M_SMEM
-                                                             const __grid_constant__ CUtensorMap tm_m,
-#endif
-                                                             Step2DArgs a) {
+__global__ void __launch_bounds__(NW * 32) fd2d_step_kernel(const __grid_constant__ CUtensorMap tm_cur, Step2DArgs a) {
     constexpr int BX = 128, SX = BX + 2 * kHalo, SZ = BZ + 2 * kHalo, RPW = BZ / NW;
     static_assert(BZ % NW == 0, "rows must split evenly over warps");
-    extern __shared__ __align__(128) float tile[];          // [SZ][SX] (+ [BZ][BX] of m)
+    extern __shared__ __align__(128) float tile[];          // [SZ][SX]
     __shared__ __align__(8) uint64_t bar;
-#if FWI_M_SMEM
-    __shared__ __align__(8) uint64_t bar_m;
-    float* sM = tile + step_tile_floats(BZ);
-#endif
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int tx0 = blockIdx.x * BX, tz0 = blockIdx.y * BZ;
@@ -105,49 +67,27 @@ __global__ void FWI_STEP_BOUNDS(NW * 32) fd2d_step_kernel(const __grid_constant_
     //      step n+1 runs while step n is still draining (the launch latency and the tail of a 6 us kernel overlap)
     if (threadIdx.x == 0) {
         mbar_init(&bar, 1);
-#if FWI_M_SMEM
-        mbar_init(&bar_m, 1);
-#endif
         fence_mbar_init();
         fence_proxy_async();
-#if FWI_M_SMEM
-        mbar_expect_tx(&bar_m, BZ * BX * (uint32_t)sizeof(float));
-        tma_load_2d(sM, &tm_m, tx0, tz0, &bar_m);
-#endif
     }
     float4 gx4 = make_float4(1.f, 1.f, 1.f, 1.f);
     if (col_ok) gx4 = ld4(a.gx + x);
     // (prefetching the adjoint's snapshot rows into L2 from here was measured: 17.3 vs 17.0 ms per 1000-step gradient, not kept;
     //  so was a bulk L2 prefetch, cp.async.bulk.prefetch.L2, of the two snapshot tiles of the NEXT deferred-imaging launch
     //  issued by the propagate-only step before it: 16.5 vs 15.6 us per forward+adjoint step pair at 1000 x 3000)
-#if FWI_PREFETCH_ROW0
     // u_{n-1} and m of this warp's first rows: neither is written by the step this launch is chained to (u_{n-1} is the
     // output of step n-2, which completed before step n-1 passed its own wait), and requesting them here takes one L2
     // round trip off the serial chain  TMA wait -> row loads -> compute
-    float4 o4p[FWI_PREFETCH_ROW0], m4p[FWI_PREFETCH_ROW0];
+    float4 o4p[kPrefetchRows], m4p[kPrefetchRows];
 #pragma unroll
-    for (int r = 0; r < FWI_PREFETCH_ROW0; ++r) {
+    for (int r = 0; r < kPrefetchRows; ++r) {
         o4p[r] = make_float4(0.f, 0.f, 0.f, 0.f); m4p[r] = o4p[r];
         if (col_ok && zw + r < a.nz) {
             o4p[r] = ld4(a.oldnew + (size_t)(zw + r) * a.px + x);
-#if !FWI_M_SMEM
             m4p[r] = ld4(a.m + (size_t)(zw + r) * a.px + x);
-#endif
         }
     }
-#endif
-#if FWI_L1_PREFETCH
-#pragma unroll
-    for (int r = FWI_PREFETCH_ROW0; r < RPW && r < FWI_PREFETCH_ROW0 + FWI_L1_PREFETCH; ++r)
-        if (col_ok && zw + r < a.nz) {
-            prefetch_l1(a.oldnew + (size_t)(zw + r) * a.px + x);
-            prefetch_l1(a.m + (size_t)(zw + r) * a.px + x);
-        }
-#endif
     griddep_wait();                 // step n complete and visible (no-op for a plain launch)
-#if FWI_PDL_TRIGGER == 1
-    griddep_launch_dependents();    // every CTA of this grid is resident once all have passed here: step n+2's may queue up
-#endif
     if (threadIdx.x == 0) {
         mbar_expect_tx(&bar, SX * SZ * (uint32_t)sizeof(float));
         tma_load_2d(tile, &tm_cur, tx0 - kHalo, tz0 - kHalo, &bar);
@@ -155,12 +95,6 @@ __global__ void FWI_STEP_BOUNDS(NW * 32) fd2d_step_kernel(const __grid_constant_
     __syncthreads();        // barrier init visible to every waiter
 
     mbar_wait(&bar, 0);
-#if FWI_M_SMEM
-    mbar_wait(&bar_m, 0);
-#endif
-#if FWI_PDL_TRIGGER == 3
-    griddep_launch_dependents();
-#endif
 
     if (col_ok && zw < a.nz) {
         // register window over z: win[k] holds row (z - 4 + k) of this lane's float4 column
@@ -183,27 +117,8 @@ __global__ void FWI_STEP_BOUNDS(NW * 32) fd2d_step_kernel(const __grid_constant_
 #pragma unroll
                 for (int k = 0; k < 9; ++k) { zc[k][0] = win[k].x; zc[k][1] = win[k].y; zc[k][2] = win[k].z; zc[k][3] = win[k].w; }
                 const size_t off = (size_t)z * a.px + x;
-#if FWI_ROW_PIPE
-                // queue: o4p[k] / m4p[k] hold row r + k; row r + FWI_PREFETCH_ROW0 is requested now, before row r's store
-                const float4 o4 = o4p[0], m4 = m4p[0];
-                float4 o4n = make_float4(0.f, 0.f, 0.f, 0.f), m4n = o4n;
-                if (r + FWI_PREFETCH_ROW0 < RPW && z + FWI_PREFETCH_ROW0 < a.nz) {
-                    o4n = ld4(a.oldnew + off + (size_t)FWI_PREFETCH_ROW0 * a.px);
-                    m4n = ld4(a.m + off + (size_t)FWI_PREFETCH_ROW0 * a.px);
-                }
-#pragma unroll
-                for (int k = 0; k + 1 < FWI_PREFETCH_ROW0; ++k) { o4p[k] = o4p[k + 1]; m4p[k] = m4p[k + 1]; }
-                o4p[FWI_PREFETCH_ROW0 - 1] = o4n; m4p[FWI_PREFETCH_ROW0 - 1] = m4n;
-#elif FWI_M_SMEM
-                const float4 o4 = (r < FWI_PREFETCH_ROW0) ? o4p[r < FWI_PREFETCH_ROW0 ? r : 0] : ld4(a.oldnew + off);
-                const float4 m4 = ld4(sM + (warp * RPW + r) * BX + 4 * lane);
-#elif FWI_PREFETCH_ROW0
-                const float4 o4 = (r < FWI_PREFETCH_ROW0) ? o4p[r < FWI_PREFETCH_ROW0 ? r : 0] : ld4(a.oldnew + off);
-                const float4 m4 = (r < FWI_PREFETCH_ROW0) ? m4p[r < FWI_PREFETCH_ROW0 ? r : 0] : ld4(a.m + off);
-#else
-                const float4 o4 = ld4(a.oldnew + off);
-                const float4 m4 = ld4(a.m + off);
-#endif
+                const float4 o4 = (r < kPrefetchRows) ? o4p[r < kPrefetchRows ? r : 0] : ld4(a.oldnew + off);
+                const float4 m4 = (r < kPrefetchRows) ? m4p[r < kPrefetchRows ? r : 0] : ld4(a.m + off);
                 const float gzv = __ldg(a.gz + z);
                 const float ov[4] = {o4.x, o4.y, o4.z, o4.w}, mv[4] = {m4.x, m4.y, m4.z, m4.w};
                 const float gv[4] = {gx4.x * gzv, gx4.y * gzv, gx4.z * gzv, gx4.w * gzv};
@@ -239,9 +154,6 @@ __global__ void FWI_STEP_BOUNDS(NW * 32) fd2d_step_kernel(const __grid_constant_
         }
     }
 
-#if FWI_PDL_TRIGGER == 2
-    griddep_launch_dependents();
-#endif
     // ---- sparse fix-ups for the points this tile owns: injection, then receiver sampling ----------
     const int tid = blockIdx.y * gridDim.x + blockIdx.x;
     const int i0 = a.inj.tile_ptr ? a.inj.tile_ptr[tid] : 0, i1 = a.inj.tile_ptr ? a.inj.tile_ptr[tid + 1] : 0;
@@ -339,12 +251,8 @@ int encode_tiled_f32(CUtensorMap* out, void* base, int rank, const uint64_t* dim
     cuuint64_t d[5]; cuuint64_t s[5]; cuuint32_t b[5]; cuuint32_t es[5];
     for (int i = 0; i < rank; ++i) { d[i] = dims[i]; b[i] = box[i]; es[i] = 1; }
     for (int i = 0; i < rank - 1; ++i) s[i] = strides_bytes[i];
-    static int promo = -1;
-    if (promo < 0) { const char* e = getenv("FWI_TMA_L2PROMO"); promo = e ? atoi(e) : 2; }      // 0 none, 1 64B, 2 128B, 3 256B
-    const CUtensorMapL2promotion pr = promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : (promo == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B :
-                                      (promo == 3 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
     CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, base, d, s, b, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_NONE, pr, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d", (int)r); return FWI_ECUDA; }
     return FWI_OK;
 }
@@ -378,6 +286,10 @@ struct PointList {
 };
 
 constexpr int kBX = 128;
+// The one-step kernel is built for exactly these (rows, warps per CTA): the round-1 sweep's winner and three heights of 7 rows
+// per warp among which one has tiles that fill whole waves.  pick_tile() breaks ties by this order.
+// (5 and 7 warps per CTA measured 1.5x slower at 1000 x 3000)
+constexpr int kStepTiles[][2] = {{32, 4}, {28, 4}, {42, 6}, {56, 8}};
 
 struct GraphEntry {
     int kind, nt, nsrc, nrec, seg, nseg;
@@ -411,10 +323,9 @@ struct fwi_fd2d {
     CUtensorMap tb_cur[8], tb_old[8], tb_m;     // temporally blocked kernel (variant 2)
     int cz = 32, tb_nw = 8, tiles_x2 = 0, tiles_z2 = 0;
     float *m = nullptr, *vp = nullptr, *gx = nullptr, *gz = nullptr;
-    void* arena = nullptr; size_t l2_persist_bytes = 0;
+    void* arena = nullptr;
     float* fld[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // forward 0..3, adjoint 4..7 (one-step kernels use 0/1 and 4/5)
     CUtensorMap tmap[8];
-    CUtensorMap tmap_m;               // FWI_M_SMEM: 128 x bz box of m
     float* acc = nullptr;
     float* snap = nullptr; size_t snap_steps = 0;
     float* ckpt = nullptr; size_t ckpt_slots = 0;
@@ -465,20 +376,16 @@ static int make_tmaps3(fwi_fd2d* p) {
         // (measured on 8 GPUs, 64 planes per rank, us per launch: one chunk 93.0 / 95.7 with 14- / 16-row tiles, two chunks
         // 97.9 / 100.1 - a single chunk re-reads 8 instead of 16 halo planes, which outweighs pushing the lower boundary
         // at the end of the launch; the model charges that late push 3 %; 4 GPUs, 128 planes per rank: 152.4 vs 157.2 us)
-        int min_ch = 1;
-        int force_by = 0, force_ch = 0;
+        int force_by = 0;
         if (const char* e = getenv("FWI_FD3D_BY")) force_by = atoi(e);
-        if (const char* e = getenv("FWI_FD3D_NZCH")) force_ch = atoi(e);       // tuning aid: fixed chunk count (1 = the lower boundary is pushed last)
-        if (force_ch >= 1) min_ch = std::min(force_ch, std::max(1, nzo / 8));
         int best_by = 16, best = 1;
         double best_cost = 1e300;
         for (int by : {16, 14}) {
             if (force_by ? by != force_by : (by != 16 && !p->peers())) continue;
             const int txy = p->tiles_x * ((p->ny + by - 1) / by);
-            for (int nzch = min_ch; nzch <= (force_ch >= 1 ? min_ch : std::max(min_ch, nzo / 8)); ++nzch) {
+            for (int nzch = 1; nzch <= std::max(1, nzo / 8); ++nzch) {
                 const int zc = (nzo + nzch - 1) / nzch;
                 const int real = (nzo + zc - 1) / zc;
-                if (real < min_ch) continue;
                 if (p->peers() && nzo - (real - 1) * zc < kHalo) continue;
                 const double waves = std::ceil((double)txy * real / p->sm_count);
                 const double late_push = (p->peer_arena[1] && real == 1) ? 1.03 : 1.0;
@@ -531,13 +438,6 @@ static int make_tmaps(fwi_fd2d* p) {
         const uint64_t strides[1] = {(uint64_t)p->px * sizeof(float)};
         const uint32_t box[2] = {(uint32_t)(kBX + 2 * kHalo), (uint32_t)(p->bz + 2 * kHalo)};
         int rc = encode_tiled_f32(&p->tmap[i], p->fld[i], 2, dims, strides, box);
-        if (rc) return rc;
-    }
-    {
-        const uint64_t dims_p[2] = {(uint64_t)p->px, (uint64_t)p->nz};
-        const uint64_t strides[1] = {(uint64_t)p->px * sizeof(float)};
-        const uint32_t box_m[2] = {(uint32_t)kBX, (uint32_t)p->bz};
-        int rc = encode_tiled_f32(&p->tmap_m, p->m, 2, dims_p, strides, box_m);
         if (rc) return rc;
     }
     return FWI_OK;
@@ -667,21 +567,7 @@ static int launch_step_cfg(fwi_fd2d* p, int mode, int cur, float* oldnew, const 
     a.rec = (rec && rec->n) ? rec->dev() : PointListDev{nullptr, nullptr, nullptr};
     a.rec_out = rec_out;
     const dim3 grid(p->tiles_x, p->tiles_z), block(NW * 32);
-#if FWI_M_SMEM
-    const size_t smem = (step_tile_floats(BZ) + (size_t)BZ * kBX) * sizeof(float);
-#define STEP_TMAPS p->tmap[cur], p->tmap_m
-    static bool smem_attr_set = false;          // per <BZ, NW> instantiation: tile + m rows exceed the 48 KB default
-    if (!smem_attr_set) {
-        FWI_CUDA(cudaFuncSetAttribute(fd2d_step_kernel<BZ, NW, STEP_FWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        FWI_CUDA(cudaFuncSetAttribute(fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        FWI_CUDA(cudaFuncSetAttribute(fd2d_step_kernel<BZ, NW, STEP_ADJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        FWI_CUDA(cudaFuncSetAttribute(fd2d_step_kernel<BZ, NW, STEP_ADJ2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        smem_attr_set = true;
-    }
-#else
     const size_t smem = (size_t)(kBX + 2 * kHalo) * (BZ + 2 * kHalo) * sizeof(float);
-#define STEP_TMAPS p->tmap[cur]
-#endif
     // Programmatic dependent launch: consecutive steps are chained with a programmatic edge (also inside captured graphs),
     // the kernel orders itself behind its predecessor with griddepcontrol.wait.
     cudaLaunchConfig_t cfg{};
@@ -691,11 +577,10 @@ static int launch_step_cfg(fwi_fd2d* p, int mode, int cur, float* oldnew, const 
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = (p->pdl && p->pdl_chain) ? 1 : 0;
     p->pdl_chain = true;
-    if (mode == STEP_FWD) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_FWD>, STEP_TMAPS, a));
-    else if (mode == STEP_FWD_SAVE) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, STEP_TMAPS, a));
-    else if (mode == STEP_ADJ2) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_ADJ2>, STEP_TMAPS, a));
-    else FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_ADJ>, STEP_TMAPS, a));
-#undef STEP_TMAPS
+    if (mode == STEP_FWD) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_FWD>, p->tmap[cur], a));
+    else if (mode == STEP_FWD_SAVE) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, p->tmap[cur], a));
+    else if (mode == STEP_ADJ2) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_ADJ2>, p->tmap[cur], a));
+    else FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_ADJ>, p->tmap[cur], a));
     return FWI_OK;
 }
 
@@ -722,7 +607,7 @@ static int launch_step3(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poi
     a.timeout_cycles = p->slab_timeout_cycles;
     const dim3 grid(p->tiles_x, p->tiles_y, p->nzch);
     // (programmatic dependent launch was measured on this kernel too: 2 % at 128^3, nothing from 256^3 up - not used)
-#define FD3_LAUNCH(BYV)                                                                                                         \
+#define LAUNCH3(BYV)                                                                                                         \
     do {                                                                                                                        \
         const dim3 block(T3<BYV>::Threads);                                                                                     \
         const size_t smem = T3<BYV>::Smem;                                                                                      \
@@ -731,8 +616,8 @@ static int launch_step3(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poi
         else if (mode == STEP_ADJ2) fd3d_step_kernel<STEP_ADJ2, BYV><<<grid, block, smem, st>>>(p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);        \
         else fd3d_step_kernel<STEP_ADJ, BYV><<<grid, block, smem, st>>>(p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);                               \
     } while (0)
-    if (p->by == 14) FD3_LAUNCH(14); else FD3_LAUNCH(16);
-#undef FD3_LAUNCH
+    if (p->by == 14) LAUNCH3(14); else LAUNCH3(16);
+#undef LAUNCH3
     return FWI_OK;
 }
 
@@ -741,8 +626,7 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
     p->launches++;
     if (p->ny > 1) return launch_step3(p, mode, cur, oldnew, inj, inj_vals, rec, rec_out, snap, st, snap_prev);
 #define CFG(BZV, NWV) if (p->bz == BZV && p->nw == NWV) return launch_step_cfg<BZV, NWV>(p, mode, cur, oldnew, inj, inj_vals, rec, rec_out, snap, st, snap_prev)
-    CFG(32, 4); CFG(64, 8); CFG(16, 2);      // the round-1 sweep's winner, and one taller / one flatter tile for tests
-    CFG(28, 4); CFG(42, 6); CFG(56, 8);      // 7 rows per warp: heights among which pick_tile() finds one whose tiles fill whole waves
+    CFG(32, 4); CFG(28, 4); CFG(42, 6); CFG(56, 8);      // every entry of kStepTiles
 #undef CFG
     set_error("fd2d: unsupported tile configuration bz=%d nw=%d", p->bz, p->nw);
     return FWI_EINVAL;
@@ -815,7 +699,7 @@ static int launch_tb2(fwi_fd2d* p, int mode, const State& s, int jc, int jd, con
                       cudaStream_t st) {
     p->launches++;
 #define TB(CZV, NWV) if (p->cz == CZV && p->tb_nw == NWV) return launch_tb2_cfg<CZV, NWV>(p, mode, s, jc, jd, inj_ext, inj_own, inj1, inj2, rec, rec1, rec2, snap1, snap2, st)
-    TB(32, 8); TB(24, 8); TB(16, 8);
+    TB(32, 8); TB(24, 8);
 #undef TB
     set_error("fd2d: unsupported temporal-blocking tile cz=%d", p->cz);
     return FWI_EINVAL;
@@ -1063,8 +947,8 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
     FWI_CUDA(cudaEventCreateWithFlags(&p->ev_in, cudaEventDisableTiming));
     FWI_CUDA(cudaEventCreateWithFlags(&p->ev_out, cudaEventDisableTiming));
     FWI_CUDA(cudaEventCreateWithFlags(&p->ev_geom, cudaEventDisableTiming));
-    // one arena for everything the step kernels re-read every step, hottest first, so that a single L2
-    // access-policy window can keep it resident while the snapshots stream past:
+    // one arena for everything the step kernels re-read every step, hottest first; its layout decides where the
+    // fields land in the L2, and the step timings were measured with exactly this order:
     //   [m, acc, fld0, fld1, fld4, fld5 | fld2, fld3, fld6, fld7, vp]
     const size_t plb = (pl * sizeof(float) + 255) & ~(size_t)255;
     FWI_CUDA(cudaMalloc(&p->arena, 11 * plb + 256));
@@ -1077,27 +961,7 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
         for (int k = 0; k < 8; ++k) p->fld[order[k]] = (float*)(a + (2 + k) * plb);
         p->vp = (float*)(a + 10 * plb);
     }
-    {
-        cudaDeviceProp prop;
-        FWI_CUDA(cudaGetDeviceProperties(&prop, device));
-        { const char* e = getenv("FWI_PDL"); if (e && e[0] == '0') p->pdl = false; }
-        const char* env = getenv("FWI_L2_PERSIST");
-        const bool want = env && env[0] == '1';       // opt-in: measured no gain on B200 (profiles/), the .cs stores suffice
-        if (want && prop.persistingL2CacheMaxSize > 0 && prop.accessPolicyMaxWindowSize > 0) {
-            const size_t hot = 6 * plb;                                  // m, acc and the four one-step buffers
-            const size_t setaside = std::min<size_t>((size_t)prop.persistingL2CacheMaxSize, hot);
-            if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, setaside) == cudaSuccess) {
-                cudaStreamAttrValue at{};
-                at.accessPolicyWindow.base_ptr = p->arena;
-                at.accessPolicyWindow.num_bytes = std::min<size_t>(hot, (size_t)prop.accessPolicyMaxWindowSize);
-                at.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)setaside / (double)at.accessPolicyWindow.num_bytes);
-                at.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-                at.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-                if (cudaStreamSetAttribute(p->work, cudaStreamAttributeAccessPolicyWindow, &at) != cudaSuccess) cudaGetLastError();
-                p->l2_persist_bytes = setaside;
-            } else cudaGetLastError();
-        }
-    }
+    { const char* e = getenv("FWI_PDL"); if (e && e[0] == '0') p->pdl = false; }
     FWI_CUDA(cudaMalloc(&p->gx, p->px * sizeof(float)));
     FWI_CUDA(cudaMalloc(&p->gz, nz * sizeof(float)));
     FWI_CUDA(cudaMalloc(&p->gy, ny * sizeof(float)));
@@ -1120,14 +984,14 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
     cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, device);
     int rc = make_tmaps(p);
     if (rc) return rc;
-    if ((rc = tb2_attrs<32, 8>()) || (rc = tb2_attrs<24, 8>()) || (rc = tb2_attrs<16, 8>())) return rc;
-#define FD3_ATTR(BYV)                                                                                                                        \
+    if ((rc = tb2_attrs<32, 8>()) || (rc = tb2_attrs<24, 8>())) return rc;
+#define ATTR3(BYV)                                                                                                                        \
     FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_FWD, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem));        \
     FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_FWD_SAVE, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem));   \
     FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_ADJ, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem));        \
     FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_ADJ2, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem))
-    FD3_ATTR(16); FD3_ATTR(14);
-#undef FD3_ATTR
+    ATTR3(16); ATTR3(14);
+#undef ATTR3
     return FWI_OK;
 }
 
@@ -1138,10 +1002,9 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
 // forward+adjoint step pair: 32 rows 16.67, 28: 15.34, 42: 15.50, 56: 15.56 (forward step 6.77 / 5.83 / 5.94 / 5.85); at
 // 1500 x 3000: 27.9 / 25.9 / 26.1 / 26.8.  The kernels are bit-identical, only the decomposition differs.
 static void pick_tile(int nz, int nx, int sms, int* bz, int* nw) {
-    const int cand[][2] = {{32, 4}, {28, 4}, {42, 6}, {56, 8}};          // (5 and 7 warps per CTA measured 1.5x slower at 1000 x 3000)
     const long tx = (nx + kBX - 1) / kBX;
     double best = 1e300;
-    for (const auto& c : cand) {
+    for (const auto& c : kStepTiles) {
         const long tiles = tx * ((nz + c[0] - 1) / c[0]);
         const double cost = (double)((tiles + sms - 1) / sms) * (c[0] + 4);
         if (cost < best - 1e-9) { best = cost; *bz = c[0]; *nw = c[1]; }
@@ -1167,7 +1030,6 @@ int fwi_fd2d_create(int device, int nz, int nx, float h, float dt, int nabs, flo
     if ((*out)->variant == 0 && nz >= 32) {
         int bz = 32, nw = 4;
         pick_tile(nz, nx, (*out)->sm_count, &bz, &nw);
-        if (const char* t = getenv("FWI_FD2D_BZ")) { const int v = atoi(t); if (v == 28 || v == 42 || v == 56) { bz = v; nw = v / 7; } else if (v == 32) { bz = 32; nw = 4; } }   // tuning aid
         rc = fwi_fd2d_set_tile(*out, bz, nw);
         if (rc) { fwi_fd2d_destroy(*out); *out = nullptr; }
     }
@@ -1205,7 +1067,8 @@ int fwi_fd2d_destroy(fwi_fd2d* p) {
 
 int fwi_fd2d_set_tile(fwi_fd2d* p, int bz, int nw) {
     FWI_REQUIRE(p, "fwi_fd2d_set_tile: NULL plan");
-    const bool ok = (bz == 32 && nw == 4) || (bz == 64 && nw == 8) || (bz == 16 && nw == 2) || (bz == 28 && nw == 4) || (bz == 42 && nw == 6) || (bz == 56 && nw == 8);
+    bool ok = false;
+    for (const auto& c : kStepTiles) ok = ok || (bz == c[0] && nw == c[1]);
     FWI_REQUIRE(ok, "fwi_fd2d_set_tile: unsupported (bz=%d, nw=%d)", bz, nw);
     FWI_REQUIRE(p->ny == 1, "fwi_fd2d_set_tile: 2-D plans only");
     DeviceGuard g(p->device);
@@ -1219,7 +1082,7 @@ int fwi_fd2d_set_tile(fwi_fd2d* p, int bz, int nw) {
 
 int fwi_fd2d_set_tb2(fwi_fd2d* p, int cz) {
     FWI_REQUIRE(p, "fwi_fd2d_set_tb2: NULL plan");
-    FWI_REQUIRE(cz == 16 || cz == 24 || cz == 32, "fwi_fd2d_set_tb2: unsupported core rows %d (16, 24, 32)", cz);
+    FWI_REQUIRE(cz == 24 || cz == 32, "fwi_fd2d_set_tb2: unsupported core rows %d (24, 32)", cz);
     FWI_REQUIRE(p->ny == 1, "fwi_fd2d_set_tb2: 2-D plans only");
     DeviceGuard g(p->device);
     FWI_CUDA(cudaStreamSynchronize(p->work));

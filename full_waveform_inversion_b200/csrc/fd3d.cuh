@@ -19,25 +19,10 @@
 
 namespace fwi {
 
-#ifndef FD3_RPW
-#define FD3_RPW 2
-#endif
-#ifndef FD3_NP
-#define FD3_NP 8
-#endif
-#ifndef FD3_NO
-#define FD3_NO 4
-#endif
-#ifndef FD3_OMLEAD
-#define FD3_OMLEAD 5
-#endif
-#ifndef FD3_SPLIT
-#define FD3_SPLIT 1
-#endif
-constexpr int k3BX = 128, k3NP = FD3_NP;                            // tile width, u_n ring depth
-constexpr int k3RPW = FD3_RPW;                                      // y rows per consumer warp
+constexpr int k3BX = 128, k3NP = 8;                                // tile width, u_n ring depth
+constexpr int k3RPW = 2;                                            // y rows per consumer warp
 constexpr int k3SX = k3BX + 2 * kHalo;                              // 136
-constexpr int k3NO = FD3_NO, k3OmLead = FD3_OMLEAD, k3Prod = 1 + FD3_SPLIT;   // u_{n-1}/m plane ring depth; issued 3 planes before use
+constexpr int k3NO = 4, k3OmLead = 5, k3Prod = 2;                   // u_{n-1}/m plane ring depth; issued 3 planes before use; producer warps
 // The tile height BY is a template parameter: 16 rows (8 consumer warps) or 14 rows (7 consumer warps).  512-wide planes
 // give 4 x 32 = 128 tiles of 16 rows but 4 x 37 = 148 tiles of 14 rows - exactly one per SM, which removes the 25 % tail of
 // a second wave that only 108 CTAs fill (measured on 4-GPU slabs: 0.78 -> see DESIGN.md); fwi_fd2d picks per plan.

@@ -53,13 +53,11 @@ __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* tm) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(tm) : "memory");
 }
 
-// programmatic dependent launch: wait for the grid this launch was chained to / let the next grid's CTAs become resident
+// programmatic dependent launch: wait for the grid this launch was chained to
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void st4(float* p, const float4& v) { *reinterpret_cast<float4*>(p) = v; }
-__device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
 // streaming (evict-first) accesses for the wavefield snapshots: written once / read once, must not evict the
 // L2-resident wavefields
 __device__ __forceinline__ void st4_stream(float* p, const float4& v) { __stcs(reinterpret_cast<float4*>(p), v); }

@@ -27,10 +27,6 @@ void set_error(const char* fmt, ...) {
     va_end(ap);
 }
 
-#ifndef MC_MIN_BLOCKS
-#define MC_MIN_BLOCKS 3
-#endif
-
 struct EvalParams {
     const float* rows;
     const float* gbar;
@@ -69,7 +65,7 @@ __device__ __forceinline__ void make_coef(float (&coef)[C * NM], const float (&m
 constexpr int kMcAcc = 5;      // running sums per sample: 3 accumulators + the two boundary-patch carries of flattened CC-shift
 
 template <int C, int NM, int S, int MODE>
-__global__ void __launch_bounds__(S * NM >= 8 ? 128 : 256, S * NM >= 8 ? 3 : MC_MIN_BLOCKS) mc_eval_kernel(EvalParams p) {
+__global__ void __launch_bounds__(S * NM >= 8 ? 128 : 256, 3) mc_eval_kernel(EvalParams p) {
     constexpr int CC = C * NM;
     constexpr int RW = row_width(CC);
     constexpr int RW4 = RW / 4;
@@ -1243,7 +1239,6 @@ int fwi_mc_eval(fwi_mc_ctx* c, const float* M, int64_t ldm, const float* frac, i
     int nw = (S == 8) ? 4 : 8, ks = 1;
     if (!big && !boundary_fix) { nw = pick_warps(c->K); ks = nw; }
     else if (!boundary_fix && S == 8) ks = 2;     // measured at N = 2e6 / 4e6: ks 1: 175, 2: 215, 4: 189 M samples/s (finer CTA tail)
-    { const char* e = getenv("FWI_MC_KS"); if (e && big && !boundary_fix && (atoi(e) == 1 || atoi(e) == 2 || atoi(e) == 4)) ks = atoi(e); }   // tuning aid (nw = 4 or 8 here)
     p.ks = ks;
     cudaStream_t st = (cudaStream_t)stream;
     if (c->NM == 1) {

@@ -45,43 +45,10 @@ namespace fwi {
 
 constexpr int kUK = 32;                 // padded K (floats per operand row = one 128-byte swizzle row)
 constexpr int kUM = 128;                // samples per MMA tile (TMEM lanes)
-#ifndef FWI_UMMA_PIPES
-#define FWI_UMMA_PIPES 2
-#endif
 constexpr int kUN = 256;                // time samples per resident B'' tile (one TMA box)
-constexpr int kUPipes = FWI_UMMA_PIPES; // independent pipelines per CTA (sample groups in flight).  2 x 256 columns: 5.7 ms for N = 4e6 (VR);
+constexpr int kUPipes = 2;              // independent pipelines per CTA (sample groups in flight).  2 x 256 columns: 5.7 ms for N = 4e6 (VR);
                                         // 4 x 128: 9.2 ms - the single MMA-issuing lane pays ~0.45 us per accumulator use whatever its size
-#ifndef FWI_UMMA_EXP
-#define FWI_UMMA_EXP 0                      // timing experiments: 1 = TMEM loads without folds, 2 = folds without TMEM loads
-#endif
-#ifndef FWI_UMMA_TRACE
-#define FWI_UMMA_TRACE 0                    // timing experiment: CTA (0,0) prints the clock at the handshake events of pipeline 0
-#endif
-#ifndef FWI_UMMA_LDPIPE
-#define FWI_UMMA_LDPIPE 1                   // full chunks: next piece's tcgen05.ld in flight while the current piece is folded
-#endif
-#ifndef FWI_UMMA_FUSEPACK
-#define FWI_UMMA_FUSEPACK 0                 // 1: the producer warp builds the A'' tile in shared memory from the samples (no pack kernel, no
-                                            // 128 B per sample A'' array).  Measured at N = 4e6: VR 767 M samples/s against 919 with the pack kernel
-                                            // + TMA (the warp's ~600 instructions per tile compete with the epilogue warps of its sub-partition
-                                            // and follow the stage's release; a TMA load is one instruction) - kept as a memory-saving option
-#endif
-#ifndef FWI_UMMA_F32X2
-#define FWI_UMMA_F32X2 0                    // 1: sum of squares with the packed fma.rn.f32x2 (FFMA2, two accumulator elements per instruction).
-                                            // Measured, M samples/s at N = 4e6 (0 / 1): VR 919 / 863, normalised VR 539 / 500, PCC 721 / 742,
-                                            // gau 752 / 797, CC-shift 543 / 548, normalised CC-shift 408 / 399 - not the default
-#endif
-#ifndef FWI_UMMA_LDUNROLL
-#define FWI_UMMA_LDUNROLL 4                 // unroll factor of the pipelined piece loop (2 pieces per iteration; 4 = a whole 256-column chunk)
-#endif
-#ifndef FWI_UMMA_ISSUERS
-#define FWI_UMMA_ISSUERS 1                  // MMA-issuing warps: 1 (round robin over the pipelines) or one per pipeline
-#endif
-#ifndef FWI_UMMA_STAGES
-#define FWI_UMMA_STAGES 1
-#endif
-constexpr int kUStages = FWI_UMMA_STAGES;   // accumulator stages per pipeline (its MMAs run ahead of its epilogue by stages - 1 uses)
-constexpr int kUNacc = 512 / (kUPipes * kUStages);   // time samples per accumulator use (MMA N; every stage owns that many TMEM columns)
+constexpr int kUNacc = 512 / kUPipes;   // time samples per accumulator use (MMA N; every pipeline owns that many TMEM columns)
 constexpr int kUCst = 52;               // float64 constants per resident trace in shared memory: gbar[9] | gdc[9] (CC-shift: the interpolated
                                         // cross moment) | CC-shift: dgb[9], G'[.,0][9], G'[.,T-1][9] | TraceConst (7) at 45
 constexpr int kUTilesMax = (227 * 1024 - kUPipes * 16384 - 256) / (kUN * 128 + kUCst * 8);     // resident B'' tiles (+ a trace's constants each)
@@ -166,37 +133,6 @@ __device__ __forceinline__ double rsqrt64(double x) {
     y = y * fma(-0.5 * x, y * y, 1.5);
     return y * fma(-0.5 * x, y * y, 1.5);
 }
-// packed fp32 pair arithmetic (sm_100: one instruction, two IEEE fma's): acc.{lo,hi} += {a,b}^2
-__device__ __forceinline__ void sq_acc2(uint64_t& acc, float a, float b) {
-    asm("{\n\t.reg .b64 p;\n\tmov.b64 p, {%1, %2};\n\tfma.rn.f32x2 %0, p, p, %0;\n\t}" : "+l"(acc) : "f"(a), "f"(b));
-}
-__device__ __forceinline__ float pair_sum(uint64_t acc) {
-    float lo, hi;
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(acc));
-    return lo + hi;
-}
-__device__ __forceinline__ void row_set(float (&row)[32], int idx, float v) {      // runtime index, registers only
-#pragma unroll
-    for (int q = 0; q < 32; ++q) row[q] = (q == idx) ? v : row[q];
-}
-__host__ __device__ inline float tf32_round(float x);
-// A''[n] = [M_hi | M_hi | M_lo | -1 -1 (with_d) | 0 ...]; CT = the number of components when it is known at compile time
-template <int CT>
-__device__ __forceinline__ void a_row(float (&row)[32], const float (&m)[9], int C, bool with_d) {
-#pragma unroll
-    for (int c = 0; c < 9; ++c) {
-        if (c < (CT ? CT : C)) {
-            const float x = m[c];
-            const float hi = tf32_round(x), lo = tf32_round(x - hi);
-            if (CT) { row[c] = hi; row[CT + c] = hi; row[2 * CT + c] = lo; }
-            else { row[c] = hi; row_set(row, C + c, hi); row_set(row, 2 * C + c, lo); }
-        }
-    }
-    if (with_d) {
-        if (CT) { row[3 * CT] = -1.f; row[3 * CT + 1] = -1.f; }
-        else { row_set(row, 3 * C, -1.f); row_set(row, 3 * C + 1, -1.f); }
-    }
-}
 __device__ __forceinline__ float fmax3(float a, float b, float c) {      // FMNMX3: one instruction for two comparisons
     float d;
     asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
@@ -246,14 +182,7 @@ struct UmmaEvalArgs {
 // handshake of one accumulator costs ~0.3 us per use and the epilogue's serial work (TMEM load latency, per-trace
 // combination) does not overlap with its own pipeline's MMAs, so two independent pipelines on the same resident B'' tiles
 // is what keeps the tensor core and the epilogue warps busy at the same time.
-#if FWI_UMMA_TRACE
-constexpr int kTrFirst = 84, kTrN = 48;          // accumulator uses traced (per pipeline): the CTA's 3rd and 4th sample group
-__device__ long long g_trace[2][kUPipes][kTrN][6];
-#endif
-constexpr int kULdUnroll = FWI_UMMA_LDUNROLL;
-constexpr int kUIssuers = FWI_UMMA_ISSUERS;
-static_assert(kUIssuers == 1 || kUIssuers == kUPipes, "one MMA issuer, or one per pipeline");
-constexpr int kUThreads = (4 * kUPipes + 1 + kUIssuers) * 32;        // 4 epilogue warps per pipeline + TMA producer + MMA issuer(s)
+constexpr int kUThreads = (4 * kUPipes + 2) * 32;        // 4 epilogue warps per pipeline + TMA producer + MMA issuer
 template <int MODE, bool SH>
 __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
                                                                UmmaEvalArgs a) {
@@ -264,9 +193,9 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
     uint64_t* b_full = bars;                       // 1
     uint64_t* a_full = bars + 1;                   // [pipes]
     uint64_t* a_empty = a_full + kUPipes;          // [pipes]
-    uint64_t* t_full = a_empty + kUPipes;          // [pipes][stages]
-    uint64_t* t_empty = t_full + kUPipes * kUStages;   // [pipes][stages]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + kUPipes * kUStages);
+    uint64_t* t_full = a_empty + kUPipes;          // [pipes]
+    uint64_t* t_empty = t_full + kUPipes;          // [pipes]
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t_empty + kUPipes);
     double* cst = reinterpret_cast<double*>(reinterpret_cast<uint8_t*>(bars) + 256);     // [resident traces][kUCst]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -282,7 +211,7 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
     if (threadIdx.x == 0) {
         mbar_init(b_full, 1);
         for (int s = 0; s < kUPipes; ++s) { mbar_init(&a_full[s], 1); mbar_init(&a_empty[s], 1); }
-        for (int s = 0; s < kUPipes * kUStages; ++s) { mbar_init(&t_full[s], 1); mbar_init(&t_empty[s], 4); }
+        for (int s = 0; s < kUPipes; ++s) { mbar_init(&t_full[s], 1); mbar_init(&t_empty[s], 4); }
         fence_mbar_init();
         fence_proxy_async();
     }
@@ -313,7 +242,6 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                 const int k = k0 + j / a.tiles_per_trace, tt = j % a.tiles_per_trace;
                 tma_load_2d(b_smem + (size_t)j * kUN * kUK, &tm_b, 0, (k * a.tiles_per_trace + tt) * kUN, b_full);
             }
-#if !FWI_UMMA_FUSEPACK
             int i = 0;
             for (int g = blockIdx.x; g < a.n_groups; g += ncta, ++i) {
                 const int p = i % kUPipes, use = i / kUPipes;          // pipeline, and how often its A'' stage has been used
@@ -321,53 +249,8 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                 mbar_expect_tx(&a_full[p], kUM * kUK * 4);
                 tma_load_2d(a_smem + (size_t)p * kUM * kUK, &tm_a, 0, g * kUM, &a_full[p]);
             }
-#endif
         }
-#if FWI_UMMA_FUSEPACK
-        // The A'' tile of a sample group straight from the sampler's (rows, N) layout: each lane splits the coefficients of four
-        // samples into tf32 hi / lo parts and writes the 128-byte rows in the layout a SWIZZLE_128B TMA box would have produced
-        // (16-byte chunk c of row r at chunk position c ^ (r & 7) of its 8-row group), then makes the writes visible to the
-        // async proxy the tensor core reads through.
-        // The coefficients of the NEXT group are requested right after a tile is handed over, so that only the split and the
-        // shared-memory stores follow the wait for the stage (the global loads took ~3x a TMA load's latency otherwise).
-        __syncwarp();
-        float xv[kUM / 32][9];
-        auto request = [&](int g) {
-#pragma unroll
-            for (int j = 0; j < kUM / 32; ++j) {
-                const int64_t n = (int64_t)g * kUM + lane + 32 * j;
-#pragma unroll
-                for (int c = 0; c < 9; ++c) xv[j][c] = (g < a.n_groups && n < a.N && c < a.C) ? __ldg(a.M + (size_t)c * a.ldm + n) : 0.f;
-            }
-        };
-        request(blockIdx.x);
-        int i = 0;
-        for (int g = blockIdx.x; g < a.n_groups; g += ncta, ++i) {
-            const int p = i % kUPipes, use = i / kUPipes;              // pipeline, and how often its A'' stage has been used
-            if (use >= 1) mbar_wait(&a_empty[p], (use - 1) & 1);
-            float* dst = a_smem + (size_t)p * kUM * kUK;
-#pragma unroll
-            for (int j = 0; j < kUM / 32; ++j) {
-                const int r = lane + 32 * j;
-                const bool live = (int64_t)g * kUM + r < a.N;
-                float row[kUK];
-#pragma unroll
-                for (int q = 0; q < kUK; ++q) row[q] = 0.f;
-                if (a.C == 9) a_row<9>(row, xv[j], 9, live && MODE == MODE_SSE);
-                else if (a.C == 6) a_row<6>(row, xv[j], 6, live && MODE == MODE_SSE);
-                else if (a.C == 3) a_row<3>(row, xv[j], 3, live && MODE == MODE_SSE);
-                else a_row<0>(row, xv[j], a.C, live && MODE == MODE_SSE);
-#pragma unroll
-                for (int c8 = 0; c8 < kUK / 4; ++c8)
-                    *reinterpret_cast<float4*>(dst + (size_t)r * kUK + ((c8 ^ (r & 7)) << 2)) = make_float4(row[4 * c8], row[4 * c8 + 1], row[4 * c8 + 2], row[4 * c8 + 3]);
-            }
-            fence_proxy_async();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&a_full[p]);
-            request(g + ncta);
-        }
-#endif
-    } else if (warp >= kMma) {
+    } else if (warp >= kMma) {                                      // kMma is the last warp
         // ------------------------------------------------ MMA issuer (one elected lane), round robin over the pipelines.
         // The lane's own instructions sit on every accumulator's critical path (release -> MMAs -> commit), and a lone thread
         // issues a dependent instruction every 4-10 cycles: everything the MMAs need (descriptors, instruction word, TMEM
@@ -385,7 +268,7 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
             uint64_t a_desc[kUPipes];
 #pragma unroll
             for (int p = 0; p < kUPipes; ++p) {
-                grp[p] = (kUIssuers == 1 || p == warp - kMma) ? blockIdx.x + p * ncta : a.n_groups;      // (not mine: done)
+                grp[p] = blockIdx.x + p * ncta;
                 chunk[p] = 0; ci[p] = 0; use_a[p] = 0; use_t[p] = 0; b_tr[p] = 0; b_off[p] = 0;
                 a_desc[p] = kDescHi | (uint64_t)((smem_u32(a_smem + (size_t)p * kUM * kUK) >> 4) & 0x3FFF);
             }
@@ -396,19 +279,12 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                 for (int p = 0; p < kUPipes; ++p) {
                     if (grp[p] >= a.n_groups) continue;
                     busy = true;
-                    const uint32_t ts = p * kUStages + use_t[p] % kUStages;     // accumulator stage of this use
-                    const uint32_t tm = tmem_base + ts * kUNacc;
+                    const uint32_t tm = tmem_base + p * kUNacc;                  // this pipeline's accumulator
                     const uint64_t ad = a_desc[p], bd = b_desc0 + b_off[p];
                     const uint32_t idesc = (ci[p] == cpt - 1) ? a.idesc_last : a.idesc_full;
-#if FWI_UMMA_TRACE
-                    const long long tr0 = clock64();
-#endif
                     if (chunk[p] == 0) mbar_wait(&a_full[p], use_a[p] & 1);
-                    if (use_t[p] >= kUStages) mbar_wait(&t_empty[ts], (use_t[p] / kUStages - 1) & 1);
+                    if (use_t[p] >= 1) mbar_wait(&t_empty[p], (use_t[p] - 1) & 1);
                     tc_fence_after();
-#if FWI_UMMA_TRACE
-                    const long long tr1 = clock64();
-#endif
                     const bool last_chunk = chunk[p] + 1 == nchunks;
                     if (elect_one()) {
                         if (!(a.debug & 1)) {                                   // a K-step of 8 floats advances the start address by 32 B
@@ -417,16 +293,10 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                             umma_tf32(tm, ad + 4, bd + 4, idesc, 1);
                             umma_tf32(tm, ad + 6, bd + 6, idesc, 1);
                         }
-                        umma_commit(&t_full[ts]);                   // accumulator ready for this pipeline's epilogue warps
+                        umma_commit(&t_full[p]);                    // accumulator ready for this pipeline's epilogue warps
                         if (last_chunk) umma_commit(&a_empty[p]);   // all MMAs reading this A'' tile have completed
                     }
                     __syncwarp();
-#if FWI_UMMA_TRACE
-                    if (lane == 0 && blockIdx.x == 0 && blockIdx.y == 0 && use_t[p] >= kTrFirst && use_t[p] < kTrFirst + kTrN) {
-                        long long* t = g_trace[0][p][use_t[p] - kTrFirst];
-                        t[0] = tr0; t[1] = tr1; t[2] = clock64(); t[3] = 0;
-                    }
-#endif
                     ++use_t[p];
                     if (++ci[p] == cpt) { ci[p] = 0; b_tr[p] += trace_step; b_off[p] = b_tr[p]; }
                     else b_off[p] += kUNacc * (kUK * 4 / 16);
@@ -457,7 +327,6 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
             double grp_first = 0.0, carry_s = 0.0, carry_d = 0.0;     // flattened CC-shift: boundary values (see the header)
             for (int k = k0; k < k1; ++k) {
                 float s0 = 0.f, s1 = 0.f, s2a = 0.f, s3 = 0.f, vmax = -3.0e38f, vmin = 3.0e38f;
-                uint64_t s01 = 0, s23 = 0;                            // the same four partial sums as packed pairs (FWI_UMMA_F32X2)
                 float p0 = 0.f, p1 = 0.f, prev = 0.f;                 // CC-shift: lag-one products, last column of the previous piece
                 // the trace's constants and the first-order terms (9-term dot products with float64 constants) do not need the
                 // accumulator: they are issued here, so that their loads and fp64 chains overlap the wait for this trace's first MMAs
@@ -472,38 +341,19 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                         if (SH) { dlt = fma(coef[c], ck[18 + c], dlt); f = fma(coef[c], ck[27 + c], f); l = fma(coef[c], ck[36 + c], l); }
                     }
                 }
-#if FWI_UMMA_TRACE
-                if (blockIdx.x == 0 && blockIdx.y == 0 && (warp & 3) == 0 && lane == 0 && use_t >= kTrFirst && use_t < kTrFirst + kTrN)
-                    g_trace[1][p][use_t - kTrFirst][5] = clock64();                // constants and dot products of this trace issued
-#endif
                 for (int ci = 0; ci < a.chunks_per_trace; ++ci, ++use_t) {
-                    const int ts = p * kUStages + use_t % kUStages;
-#if FWI_UMMA_TRACE
-                    const long long te0 = clock64();
-#endif
-                    mbar_wait(&t_full[ts], (use_t / kUStages) & 1);
+                    mbar_wait(&t_full[p], use_t & 1);
                     tc_fence_after();
-#if FWI_UMMA_TRACE
-                    const long long te1 = clock64();
-                    long long te2 = 0;
-#endif
-                    const uint32_t taddr = tmem_base + ts * kUNacc + ((uint32_t)(wq * 32) << 16);
+                    const uint32_t taddr = tmem_base + p * kUNacc + ((uint32_t)(wq * 32) << 16);
                     // columns the MMA of this chunk wrote (those past T hold 0: B'' is zero-padded); a multiple of 16
                     const int ncol = (ci == a.chunks_per_trace - 1) ? a.n_last : kUNacc;
                     // one 32-column piece of the accumulator (a trace's last piece may hold 16 columns: `half`)
                     auto fold = [&](const float (&v)[32], const bool half) {
-#if FWI_UMMA_EXP == 1
-                        s0 += v[0];
-                        if (false)
-#endif
 #pragma unroll
                         for (int i = 0; i < 32; i += 4) {
                             if (i < 16 || !half) {
-                                if (FWI_UMMA_F32X2) { sq_acc2(s01, v[i], v[i + 1]); sq_acc2(s23, v[i + 2], v[i + 3]); }
-                                else {
-                                    s0 = fmaf(v[i], v[i], s0); s1 = fmaf(v[i + 1], v[i + 1], s1);
-                                    s2a = fmaf(v[i + 2], v[i + 2], s2a); s3 = fmaf(v[i + 3], v[i + 3], s3);
-                                }
+                                s0 = fmaf(v[i], v[i], s0); s1 = fmaf(v[i + 1], v[i + 1], s1);
+                                s2a = fmaf(v[i + 2], v[i + 2], s2a); s3 = fmaf(v[i + 3], v[i + 3], s3);
                                 if (MODE == MODE_MOM_MAX) {
                                     vmax = fmax3(vmax, v[i], v[i + 1]); vmin = fmin3(vmin, v[i], v[i + 1]);
                                     vmax = fmax3(vmax, v[i + 2], v[i + 3]); vmin = fmin3(vmin, v[i + 2], v[i + 3]);
@@ -520,19 +370,16 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                     auto release = [&]() {                              // accumulator drained by this warp
                         tc_fence_before();
                         __syncwarp();
-                        if (lane == 0) mbar_arrive(&t_empty[ts]);
-#if FWI_UMMA_TRACE
-                        te2 = clock64();
-#endif
+                        if (lane == 0) mbar_arrive(&t_empty[p]);
                     };
                     if (a.debug & 2) {
                         release();
-                    } else if (FWI_UMMA_LDPIPE && ncol == kUNacc) {
+                    } else if (ncol == kUNacc) {
                         // full chunk, unrolled: the next piece's tcgen05.ld is in flight while the current piece is folded, and the
                         // accumulator goes back to the MMA issuer as soon as its last piece is in registers
                         float va[32], vb[32];
                         tmem_ld32(taddr, va);
-#pragma unroll kULdUnroll
+#pragma unroll 4
                         for (int i = 0; i < kUNacc / 32; i += 2) {
                             tmem_ld_wait_dep(va);
                             tmem_ld32(taddr + (i + 1) * 32, vb);
@@ -544,26 +391,15 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                     } else {
                         for (int c0 = 0; c0 < ncol; c0 += 32) {
                             float v[32];
-#if FWI_UMMA_EXP == 2
-#pragma unroll
-                            for (int i = 0; i < 32; ++i) asm volatile("" : "=f"(v[i]));
-#else
                             tmem_ld32(taddr + c0, v);
                             tmem_ld_wait_dep(v);
-#endif
                             fold(v, ncol - c0 < 32);
                         }
                         release();
                     }
-#if FWI_UMMA_TRACE
-                    if (blockIdx.x == 0 && blockIdx.y == 0 && (warp & 3) == 0 && lane == 0 && use_t >= kTrFirst && use_t < kTrFirst + kTrN) {
-                        long long* t = g_trace[1][p][use_t - kTrFirst];
-                        t[0] = te0; t[1] = te1; t[2] = te2; t[3] = clock64();
-                    }
-#endif
                 }
                 // ---- combine trace k (float64; the expressions of mc_eval_kernel's fold)
-                const double s2 = FWI_UMMA_F32X2 ? (double)(pair_sum(s01) + pair_sum(s23)) : (double)((s0 + s1) + (s2a + s3));
+                const double s2 = (double)((s0 + s1) + (s2a + s3));
                 if (MODE == MODE_SSE) {
                     const double sse = s2, dd = tc.sumd2;
                     q1 += sse; q2 += dd;
@@ -619,10 +455,6 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
                         q2 += aa * bb * (sd + Tn * tc.mean_d * mud);
                     }
                 }
-#if FWI_UMMA_TRACE
-                if (blockIdx.x == 0 && blockIdx.y == 0 && (warp & 3) == 0 && lane == 0 && use_t - 1 >= kTrFirst && use_t - 1 < kTrFirst + kTrN)
-                    g_trace[1][p][use_t - 1 - kTrFirst][4] = clock64() + (long long)(q0 * 0.0);      // trace combined (depends on its result)
-#endif
             }
             if (live) {
                 double* o = a.part + (size_t)tg * a.npart * a.N + n;
@@ -633,18 +465,6 @@ __global__ void __launch_bounds__(kUThreads, 1) mc_umma_kernel(const __grid_cons
     }
     tc_fence_before();
     __syncthreads();
-#if FWI_UMMA_TRACE
-    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
-        const long long t0 = g_trace[0][0][0][0];
-        for (int i = 0; i < kTrN; ++i)
-            for (int p = 0; p < kUPipes; ++p) {
-                const long long* I = g_trace[0][p][i];
-                const long long* E = g_trace[1][p][i];
-                printf("use %3d p%d | issuer: wait %6lld wake %6lld committed %6lld | epilogue: consts %6lld wait %6lld wake %6lld released %6lld folded %6lld combined %6lld\n",
-                       kTrFirst + i, p, I[0] - t0, I[1] - t0, I[2] - t0, E[5] ? E[5] - t0 : 0, E[0] - t0, E[1] - t0, E[2] - t0, E[3] - t0, E[4] ? E[4] - t0 : 0);
-            }
-    }
-#endif
     if (warp == kMma) tmem_dealloc(tmem_base, 512);
 }
 
@@ -903,7 +723,7 @@ int umma_eval(UmmaPath* u, const float* M_dev, int64_t ldm, int64_t N, int metri
     const bool shift = metric == FWI_METRIC_CC_SHIFT;
     const int npart = (shift && simul) ? 5 : 3;
     const int64_t ngroups = (N + kUM - 1) / kUM, Npad = ngroups * kUM;
-    if (!FWI_UMMA_FUSEPACK && u->A_rows < (size_t)Npad) {
+    if (u->A_rows < (size_t)Npad) {
         if (u->A) cudaFree(u->A);
         u->A = nullptr; u->A_rows = 0;
         FWI_CUDA(cudaMalloc(&u->A, (size_t)Npad * kUK * sizeof(float)));
@@ -916,14 +736,10 @@ int umma_eval(UmmaPath* u, const float* M_dev, int64_t ldm, int64_t N, int metri
         u->part_cap = (size_t)u->n_tgroups * npart * N;
     }
     CUtensorMap tm_a;
-    memset(&tm_a, 0, sizeof(tm_a));
-    int rc = FWI_OK;
-    if (!FWI_UMMA_FUSEPACK) {
-        rc = encode_rows32_sw128(&tm_a, u->A, (uint64_t)Npad, kUM);
-        if (rc) return rc;
-        mc_umma_pack_kernel<<<(unsigned)((Npad + 127) / 128), 128, 0, st>>>(M_dev, ldm, u->C, N, Npad, mode == MODE_SSE ? 1 : 0, u->A);
-        FWI_CUDA(cudaGetLastError());
-    }
+    int rc = encode_rows32_sw128(&tm_a, u->A, (uint64_t)Npad, kUM);
+    if (rc) return rc;
+    mc_umma_pack_kernel<<<(unsigned)((Npad + 127) / 128), 128, 0, st>>>(M_dev, ldm, u->C, N, Npad, mode == MODE_SSE ? 1 : 0, u->A);
+    FWI_CUDA(cudaGetLastError());
     // CTAs per trace group in proportion to its traces (K = 21, two resident traces: 10 groups x 14 CTAs + 1 group x 7 = 147)
     const int last_traces = u->K - (u->n_tgroups - 1) * u->traces_per_cta;
     const int ctas_full = (int)std::min<int64_t>(ngroups, std::max(1, u->sms * u->traces_per_cta / u->K));

@@ -163,11 +163,11 @@ typedef struct fwi_fd2d fwi_fd2d;
  * accumulator and the TMA descriptors. */
 int fwi_fd2d_create(int device, int nz, int nx, float h, float dt, int nabs, float alpha, fwi_fd2d** out);
 int fwi_fd2d_destroy(fwi_fd2d* plan);
-/* Select the one-tile-per-CTA step kernel with bz tile rows and nw warps per CTA: (32, 4), (64, 8), (16, 2), or 7 rows per
- * warp: (28, 4), (42, 6), (56, 8).  fwi_fd2d_create picks, for L2-resident grids, the height whose tiles
- * fill whole waves of the GPU's SMs (all shapes give bit-identical fields).  Clears the geometry. */
+/* Select the one-tile-per-CTA step kernel with bz tile rows and nw warps per CTA: (32, 4), or 7 rows per warp:
+ * (28, 4), (42, 6), (56, 8); any other pair is FWI_EINVAL.  fwi_fd2d_create picks, for L2-resident grids, the height
+ * whose tiles fill whole waves of the GPU's SMs (all shapes give bit-identical fields).  Clears the geometry. */
 int fwi_fd2d_set_tile(fwi_fd2d* plan, int bz, int nw);
-/* Select the temporally blocked kernel: two leapfrog steps per pass on 120 x cz core tiles (cz in 16, 24, 32);
+/* Select the temporally blocked kernel: two leapfrog steps per pass on 120 x cz core tiles (cz 24 or 32, else FWI_EINVAL);
  * an odd leftover step runs the one-step tile kernel.  Clears the geometry. */
 int fwi_fd2d_set_tb2(fwi_fd2d* plan, int cz);
 /* Replay the time loops as cached CUDA graphs (default on) or as individual launches (0). */

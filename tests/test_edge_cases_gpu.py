@@ -79,6 +79,10 @@ def test_monte_carlo_single_sample_and_remainders(mods):
 
 
 # ------------------------------------------------------------------------------------------------ Track B
+# the size-dependent default, the two-steps-per-pass kernel with 32 core rows and the one-step kernel with 28-row tiles
+EDGE_KERNELS = [dict(), pytest.param(dict(tb2=32), id="tb2_32"), pytest.param(dict(tile=(28, 4)), id="tile_28x4")]
+
+
 def _grid(nz=37, nx=131, seed=0):
     rng = np.random.default_rng(seed)
     v = (2000.0 + 500.0 * rng.random((nz, nx))).astype(np.float32).astype(np.float64)
@@ -86,7 +90,7 @@ def _grid(nz=37, nx=131, seed=0):
     return v, h, fo.stable_dt(v.max(), h, 2)
 
 
-@pytest.mark.parametrize("kw", [dict(), dict(tb2=16), dict(tile=(16, 2))])
+@pytest.mark.parametrize("kw", EDGE_KERNELS)
 @pytest.mark.parametrize("nt", [1, 2, 3, 37])
 def test_short_and_odd_step_counts(mods, kw, nt):
     """nt = 1 and odd nt: the two-steps-per-pass kernel must hand its leftover step to the one-step kernel, the
@@ -108,17 +112,18 @@ def test_short_and_odd_step_counts(mods, kw, nt):
     prop.close()
 
 
-@pytest.mark.parametrize("kw", [dict(), dict(tb2=16), dict(tile=(16, 2))])
+@pytest.mark.parametrize("kw", EDGE_KERNELS)
 def test_corner_duplicate_and_colocated_points(mods, kw):
     """Sources in the grid corners, two sources on the same cell, a receiver on the source cell, duplicated
-    receivers, points on tile boundaries (x = 119/120/127/128, z = 15/16/31/32)."""
+    receivers, points on tile boundaries (x = 119/120/127/128, z = 15/16/23/24/27/28/31/32)."""
     ac, _ = mods
     v, h, dt = _grid(48, 260, seed=3)
     nz, nx = v.shape
-    src = [(0, 0), (nz - 1, nx - 1), (16, 128), (16, 128), (31, 119)]
-    rec = [(0, 0), (16, 128), (16, 128), (15, 127), (32, 120), (nz - 1, 0), (0, nx - 1), (20, 200)]
+    src = [(0, 0), (nz - 1, nx - 1), (16, 128), (16, 128), (31, 119), (24, 119), (27, 128)]
+    rec = [(0, 0), (16, 128), (16, 128), (15, 127), (32, 120), (nz - 1, 0), (0, nx - 1), (20, 200),
+           (23, 120), (24, 119), (27, 127), (28, 128)]
     nt = 90
-    wav = np.stack([fo.ricker(nt, dt, 25.0) * a for a in (1.0, -0.5, 0.8, 0.3, 0.6)], 1)
+    wav = np.stack([fo.ricker(nt, dt, 25.0) * a for a in (1.0, -0.5, 0.8, 0.3, 0.6, -0.7, 0.4)], 1)
     obs = fo.Problem(v * 0.97, h, dt, src, rec, nabs=5).forward(wav)
     J_want, g_want, tr_want = fo.Problem(v, h, dt, src, rec, nabs=5).misfit_and_gradient(wav, obs)
     prop = ac.Propagator2D(v.shape, h, dt, nabs=5, **kw)

@@ -9,7 +9,7 @@ nz, nx, nt = 1000, 3000, 600
 v = torch.tensor(fo.layered_model((nz, nx), 1500.0, 4500.0, 6), dtype=torch.float32)
 dt = fo.stable_dt(4500.0, 10.0, 2)
 wav = fo.ricker(nt, dt, 12.0).astype(np.float32)
-for kw in (dict(tile=(16, 2)), dict(tile=(16, 2), graphs=False), dict(tile=(32, 4))):
+for kw in (dict(tile=(28, 4)), dict(tile=(28, 4), graphs=False), dict(tile=(32, 4))):
     prop = ac.Propagator2D((nz, nx), 10.0, dt, nabs=40, **kw)
     prop.set_model(v)
     prop.set_geometry([(40, 700)], [(50, 715), (45, 705), (300, 900)])

@@ -2,9 +2,6 @@
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
-from full_waveform_inversion_b200 import _lib
-if os.environ.get("FWI_VARIANT_LIB"):
-    _lib.LIB_PATH = os.environ["FWI_VARIANT_LIB"]
 from full_waveform_inversion_b200 import acoustic as ac
 
 def timed(fn, reps):

@@ -35,9 +35,9 @@ python tools/mc_bench.py 2000000 > $O/${TAG}_mc_bench.txt 2>&1 && ncu --set full
 ncu -i $O/prof_mc.ncu-rep --page raw --csv > /tmp/p.csv 2>/dev/null
 python tools/summarize_ncu.py raw /tmp/p.csv > $O/${TAG}_mc_eval_ncu_full.txt; rm -f $O/prof_mc.ncu-rep
 
-# 5. Track A tensor-core likelihood kernel (default path): the N = 4e6 VR per-trace evaluation of tools/umma_trace.py
-python tools/umma_trace.py 4000000 VR 0 > $O/plain_u.log 2>&1 && ncu --set full --clock-control none --import-source on -k regex:mc_umma_kernel \
-    -c 1 -o $O/prof_umma python tools/umma_trace.py 4000000 VR 0 > $O/ncu_umma.log 2>&1
+# 5. Track A tensor-core likelihood kernel (default path): the first evaluation of tools/mc_bench.py at N = 4e6
+python tools/mc_bench.py 4000000 > $O/plain_u.log 2>&1 && ncu --set full --clock-control none --import-source on -k regex:mc_umma_kernel \
+    -c 1 -o $O/prof_umma python tools/mc_bench.py 4000000 > $O/ncu_umma.log 2>&1
 ncu -i $O/prof_umma.ncu-rep --page raw --csv > /tmp/p.csv 2>/dev/null
 python tools/summarize_ncu.py raw /tmp/p.csv > $O/${TAG}_mc_umma_ncu_full.txt; rm -f $O/prof_umma.ncu-rep
 du -sh $O

@@ -3,9 +3,6 @@ variants: fits t = a + b * points to separate the fixed per-launch cost from the
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from full_waveform_inversion_b200 import _lib
-if os.environ.get("FWI_VARIANT_LIB"):
-    _lib.LIB_PATH = os.environ["FWI_VARIANT_LIB"]          # tuning builds from tools/build_variant.sh
 from full_waveform_inversion_b200 import acoustic as ac
 
 def time_forward(nz, nx, nt, **kw):
@@ -20,7 +17,7 @@ def time_forward(nz, nx, nt, **kw):
     prop.close()
     return e0.elapsed_time(e1) * 1e3 / nt     # us per step
 
-variants = [("tile", (16, 2)), ("tile", (32, 4)), ("tile", (64, 8))]
+variants = [("tile", (28, 4)), ("tile", (32, 4)), ("tile", (56, 8))]
 if len(sys.argv) > 1:
     variants = []
     for a in sys.argv[1:]:

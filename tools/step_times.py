@@ -3,9 +3,6 @@ import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import bench
-from full_waveform_inversion_b200 import _lib
-if os.environ.get("FWI_VARIANT_LIB"):
-    _lib.LIB_PATH = os.environ["FWI_VARIANT_LIB"]          # tuning builds from tools/build_variant.sh
 from full_waveform_inversion_b200 import acoustic as ac
 
 class A: grid = "1000x3000"; nt = int(sys.argv[1]) if len(sys.argv) > 1 else 5000

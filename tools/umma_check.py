@@ -1,11 +1,8 @@
 """Tensor-core likelihood path (csrc/mc_umma.cu) vs the float64 oracle and the fp32 CUDA-core kernels, every metric x mode
-it covers; then rates.   python tools/umma_check.py [N_bench] [--quick]   (FWI_VARIANT_LIB=<.so from tools/build_variant.sh>)"""
+it covers; then rates.   python tools/umma_check.py [N_bench] [--quick]"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from full_waveform_inversion_b200 import _lib
-if os.environ.get("FWI_VARIANT_LIB"):
-    _lib.LIB_PATH = os.environ["FWI_VARIANT_LIB"]          # tuning builds from tools/build_variant.sh
 from full_waveform_inversion_b200 import full_waveform_inversion as fw
 from oracle import mc_oracle as orc
 TENSOR, NO_TENSOR = 16, 32

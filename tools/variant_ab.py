@@ -1,13 +1,11 @@
-"""Tuning aid: times the bench workload's forward and gradient with the library FWI_VARIANT_LIB points at (default: the
-in-tree one) and prints SHA-256 digests of the traces and the gradient, so two builds can be compared for bit-identity.
+"""Tuning aid: times the bench workload's forward and gradient and prints SHA-256 digests of the traces and the gradient,
+so two builds (two checkouts, run one after the other) can be compared for bit-identity.
   python tools/variant_ab.py [nt]"""
 import sys, os, hashlib
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 import bench
 from full_waveform_inversion_b200 import _lib
-if os.environ.get("FWI_VARIANT_LIB"):
-    _lib.LIB_PATH = os.environ["FWI_VARIANT_LIB"]
 from full_waveform_inversion_b200 import acoustic as ac
 
 class A: grid = "1000x3000"; nt = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
