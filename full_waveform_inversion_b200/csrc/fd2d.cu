@@ -282,14 +282,57 @@ struct PointList {
         if (d_id) cudaFree(d_id);
         d_tile_ptr = d_off = d_id = nullptr; n = cap = nbins = 0;
     }
-    PointListDev dev() const { return PointListDev{d_tile_ptr, d_off, d_id}; }
+    // what a kernel reads; an absent or empty list is all null, which the kernels skip
+    static PointListDev dev(const PointList* pl) {
+        return (pl && pl->n) ? PointListDev{pl->d_tile_ptr, pl->d_off, pl->d_id} : PointListDev{nullptr, nullptr, nullptr};
+    }
 };
 
+// The step-kernel families: the one-step tile kernel, the two-steps-per-pass kernel (temporal blocking, "tb2") and the
+// 3-D kernel.  A tb2 plan also runs the tile kernel, for the odd step of a sweep and for fwi_fd_step.
+enum Family { kTile, kTb2, k3D };
+
+// One built shape of a family: tile rows (bz / cz / by), warps per CTA, dynamic shared memory per CTA, and its kernel for
+// each mode, indexed by STEP_FWD .. STEP_ADJ2 (null where the family has no such mode).  The tables below are the only
+// list of the shapes the library builds.
+template <typename Kernel> struct StepShape {
+    int rows, warps;
+    size_t smem;
+    Kernel fn[4];
+};
+using TileShape = StepShape<void (*)(CUtensorMap, Step2DArgs)>;
+using Tb2Shape = StepShape<void (*)(CUtensorMap, CUtensorMap, CUtensorMap, Tb2Args)>;
+using Fd3Shape = StepShape<void (*)(CUtensorMap, CUtensorMap, CUtensorMap, Step3DArgs)>;
+
 constexpr int kBX = 128;
+template <int BZ, int NW> TileShape tile_shape() {
+    return {BZ, NW, (size_t)(kBX + 2 * kHalo) * (BZ + 2 * kHalo) * sizeof(float),
+            {fd2d_step_kernel<BZ, NW, STEP_FWD>, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, fd2d_step_kernel<BZ, NW, STEP_ADJ>,
+             fd2d_step_kernel<BZ, NW, STEP_ADJ2>}};
+}
+constexpr int kTb2Warps = 8;          // (4 warps at 24 rows measured 8 % slower)
+template <int CZ> Tb2Shape tb2_shape() {
+    return {CZ, kTb2Warps, ((size_t)(CZ + 16) * kT2W0 + 2 * (size_t)(CZ + 8) * kT2W1) * sizeof(float),
+            {fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD>, fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD_SAVE>,
+             fd2d_tb2_kernel<CZ, kTb2Warps, STEP_ADJ>, nullptr}};
+}
+template <int BY> Fd3Shape fd3_shape() {
+    return {BY, T3<BY>::Threads / 32, T3<BY>::Smem,
+            {fd3d_step_kernel<STEP_FWD, BY>, fd3d_step_kernel<STEP_FWD_SAVE, BY>, fd3d_step_kernel<STEP_ADJ, BY>,
+             fd3d_step_kernel<STEP_ADJ2, BY>}};
+}
 // The one-step kernel is built for exactly these (rows, warps per CTA): the round-1 sweep's winner and three heights of 7 rows
 // per warp among which one has tiles that fill whole waves.  pick_tile() breaks ties by this order.
 // (5 and 7 warps per CTA measured 1.5x slower at 1000 x 3000)
-constexpr int kStepTiles[][2] = {{32, 4}, {28, 4}, {42, 6}, {56, 8}};
+static const TileShape kTileShapes[] = {tile_shape<32, 4>(), tile_shape<28, 4>(), tile_shape<42, 6>(), tile_shape<56, 8>()};
+static const Tb2Shape kTb2Shapes[] = {tb2_shape<32>(), tb2_shape<24>()};
+static const Fd3Shape kFd3Shapes[] = {fd3_shape<16>(), fd3_shape<14>()};     // the first row is the single-GPU tile height
+
+template <typename Shape, size_t N> const Shape* find_shape(const Shape (&table)[N], int rows, int warps) {
+    for (const auto& k : table)
+        if (k.rows == rows && k.warps == warps) return &k;
+    return nullptr;
+}
 
 struct GraphEntry {
     int kind, nt, nsrc, nrec, seg, nseg;
@@ -302,7 +345,8 @@ struct GraphEntry {
 struct fwi_fd2d {
     int device = 0, nz = 0, ny = 1, nx = 0, px = 0, nabs = 0;   // ny == 1: 2-D plan; rows() = nz * ny
     float h = 0, dt = 0, alpha = 0;
-    int tiles_y = 1, zchunk = 0, nzch = 1, by = 16;             // 3-D tiling: 128 x by columns (by = 16 or 14), z chunks
+    int tiles_y = 1, zchunk = 0, nzch = 1;                      // 3-D tiling: 128 x fd3->rows columns, z chunks
+    const Fd3Shape* fd3 = kFd3Shapes;
     float* gy = nullptr;
     CUtensorMap tm3[8], tm3_old[8], tm3_m;
     // slab decomposition over peer memory (3-D only)
@@ -316,12 +360,13 @@ struct fwi_fd2d {
     int last_desc = 0;                          // the last z chunk marches downwards (slab with a lower neighbour)
     long long slab_timeout_cycles = 4000000000LL;   // bounded spin on a neighbour's flag (~2 s; FWI_SLAB_TIMEOUT_MS)
     bool peers() const { return peer_arena[0] || peer_arena[1]; }
-    int bz = 32, nw = 4;              // tiled variant: tile rows / warps per CTA (tunable)
+    Family family = kTile;
+    const TileShape* tile = kTileShapes;        // the one-step tile kernel's shape (2-D plans)
     int tiles_x = 0, tiles_z = 0;
-    int variant = 0;                  // 0 = one-tile-per-CTA kernel, 2 = two-steps-per-pass kernel (temporal blocking)
     int sm_count = 148;
-    CUtensorMap tb_cur[8], tb_old[8], tb_m;     // temporally blocked kernel (variant 2)
-    int cz = 32, tb_nw = 8, tiles_x2 = 0, tiles_z2 = 0;
+    CUtensorMap tb_cur[8], tb_old[8], tb_m;     // two-steps-per-pass kernel
+    const Tb2Shape* tb2 = kTb2Shapes;
+    int tiles_x2 = 0, tiles_z2 = 0;
     float *m = nullptr, *vp = nullptr, *gx = nullptr, *gz = nullptr;
     void* arena = nullptr;
     float* fld[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // forward 0..3, adjoint 4..7 (one-step kernels use 0/1 and 4/5)
@@ -335,7 +380,7 @@ struct fwi_fd2d {
     float* wav = nullptr; size_t wav_cap = 0;
     double* d_J = nullptr;
     PointList src, rec;
-    PointList src_ext2, src_own2, rec_ext2, rec_own2;   // variant 2: binned by the 120 x cz core tiles (+-4 for *_ext2)
+    PointList src_ext2, src_own2, rec_ext2, rec_own2;   // tb2: binned by the 120 x cz core tiles (+-4 for *_ext2)
     int nsrc = 0, nrec = 0;
     size_t mem_limit = 0;             // 0 = automatic (fraction of free memory)
     bool pdl = true;                  // chain 2-D steps with programmatic dependent launch (FWI_PDL=0 turns it off)
@@ -344,7 +389,7 @@ struct fwi_fd2d {
     int fwd_c = 0, fwd_o = 1;         // fld[] indices of u_n and u_{n-1} after the last forward
     bool model_set = false;
     bool use_graphs = true;
-    bool defer_imaging = true;        // tile variant: image two adjoint steps per accumulator update
+    bool defer_imaging = true;        // tile and 3-D kernels: image two adjoint steps per accumulator update
     int64_t launches = 0;
     cudaStream_t work = nullptr;
     cudaEvent_t ev_in = nullptr, ev_out = nullptr, ev_geom = nullptr;
@@ -378,24 +423,24 @@ static int make_tmaps3(fwi_fd2d* p) {
         // at the end of the launch; the model charges that late push 3 %; 4 GPUs, 128 planes per rank: 152.4 vs 157.2 us)
         int force_by = 0;
         if (const char* e = getenv("FWI_FD3D_BY")) force_by = atoi(e);
-        int best_by = 16, best = 1;
+        const Fd3Shape* best_k = kFd3Shapes;
+        int best = 1;
         double best_cost = 1e300;
-        for (int by : {16, 14}) {
-            if (force_by ? by != force_by : (by != 16 && !p->peers())) continue;
-            const int txy = p->tiles_x * ((p->ny + by - 1) / by);
+        for (const auto& k : kFd3Shapes) {
+            if (force_by ? k.rows != force_by : (&k != kFd3Shapes && !p->peers())) continue;
+            const int txy = p->tiles_x * ((p->ny + k.rows - 1) / k.rows);
             for (int nzch = 1; nzch <= std::max(1, nzo / 8); ++nzch) {
                 const int zc = (nzo + nzch - 1) / nzch;
                 const int real = (nzo + zc - 1) / zc;
                 if (p->peers() && nzo - (real - 1) * zc < kHalo) continue;
                 const double waves = std::ceil((double)txy * real / p->sm_count);
                 const double late_push = (p->peer_arena[1] && real == 1) ? 1.03 : 1.0;
-                const double cost = waves * (zc + 2 * kHalo) * by * late_push;
-                if (cost < best_cost - 1e-9) { best_cost = cost; best = nzch; best_by = by; }
+                const double cost = waves * (zc + 2 * kHalo) * k.rows * late_push;
+                if (cost < best_cost - 1e-9) { best_cost = cost; best = nzch; best_k = &k; }
             }
         }
-        if (force_by == 14 || force_by == 16) best_by = force_by;
-        p->by = best_by;
-        p->tiles_y = (p->ny + p->by - 1) / p->by;
+        p->fd3 = best_k;
+        p->tiles_y = (p->ny + p->fd3->rows - 1) / p->fd3->rows;
         p->zchunk = (nzo + best - 1) / best;
         p->nzch = (nzo + p->zchunk - 1) / p->zchunk;
         p->last_desc = (p->peer_arena[1] && p->nzch >= 2) ? 1 : 0;
@@ -403,11 +448,11 @@ static int make_tmaps3(fwi_fd2d* p) {
     for (int i = 0; i < 8; ++i) {
         const uint64_t dims[3] = {(uint64_t)p->nx, (uint64_t)p->ny, (uint64_t)p->nz};
         const uint64_t strides[2] = {(uint64_t)p->px * sizeof(float), (uint64_t)p->px * p->ny * sizeof(float)};
-        const uint32_t box[3] = {(uint32_t)k3SX, (uint32_t)(p->by + 2 * kHalo), 1u};
+        const uint32_t box[3] = {(uint32_t)k3SX, (uint32_t)(p->fd3->rows + 2 * kHalo), 1u};
         int rc = encode_tiled_f32(&p->tm3[i], p->fld[i], 3, dims, strides, box);
         if (rc) return rc;
         const uint64_t dims_p[3] = {(uint64_t)p->px, (uint64_t)p->ny, (uint64_t)p->nz};
-        const uint32_t box_o[3] = {(uint32_t)k3BX, (uint32_t)p->by, 1u};
+        const uint32_t box_o[3] = {(uint32_t)k3BX, (uint32_t)p->fd3->rows, 1u};
         rc = encode_tiled_f32(&p->tm3_old[i], p->fld[i], 3, dims_p, strides, box_o);
         if (rc) return rc;
         if (i == 0 && (rc = encode_tiled_f32(&p->tm3_m, p->m, 3, dims_p, strides, box_o))) return rc;
@@ -416,14 +461,15 @@ static int make_tmaps3(fwi_fd2d* p) {
 }
 
 static int make_tmaps(fwi_fd2d* p) {
-    if (p->ny > 1) return make_tmaps3(p);
+    if (p->family == k3D) return make_tmaps3(p);
+    const int cz = p->tb2->rows;
     p->tiles_x2 = (p->nx + kT2CX - 1) / kT2CX;
-    p->tiles_z2 = (p->nz + p->cz - 1) / p->cz;
+    p->tiles_z2 = (p->nz + cz - 1) / cz;
     {
         const uint64_t dims[2] = {(uint64_t)p->nx, (uint64_t)p->nz};
         const uint64_t dims_p[2] = {(uint64_t)p->px, (uint64_t)p->nz};
         const uint64_t strides[1] = {(uint64_t)p->px * sizeof(float)};
-        const uint32_t box_c[2] = {(uint32_t)kT2W0, (uint32_t)(p->cz + 16)}, box_o[2] = {(uint32_t)kT2W1, (uint32_t)(p->cz + 8)};
+        const uint32_t box_c[2] = {(uint32_t)kT2W0, (uint32_t)(cz + 16)}, box_o[2] = {(uint32_t)kT2W1, (uint32_t)(cz + 8)};
         for (int i = 0; i < 8; ++i) {
             int rc = encode_tiled_f32(&p->tb_cur[i], p->fld[i], 2, dims, strides, box_c);
             if (rc) return rc;
@@ -436,17 +482,11 @@ static int make_tmaps(fwi_fd2d* p) {
     for (int i = 0; i < 8; ++i) {
         const uint64_t dims[2] = {(uint64_t)p->nx, (uint64_t)p->nz};
         const uint64_t strides[1] = {(uint64_t)p->px * sizeof(float)};
-        const uint32_t box[2] = {(uint32_t)(kBX + 2 * kHalo), (uint32_t)(p->bz + 2 * kHalo)};
+        const uint32_t box[2] = {(uint32_t)(kBX + 2 * kHalo), (uint32_t)(p->tile->rows + 2 * kHalo)};
         int rc = encode_tiled_f32(&p->tmap[i], p->fld[i], 2, dims, strides, box);
         if (rc) return rc;
     }
     return FWI_OK;
-}
-
-// bin that owns grid point (z, x): the CTA tile (tiled variant) or the warp whose row-unit range holds it
-static int owner_bin(const fwi_fd2d* p, int z, int y, int x) {
-    if (p->ny > 1) return ((std::max(0, z - p->z_own0) / p->zchunk) * p->tiles_y + y / p->by) * p->tiles_x + x / k3BX;
-    return (z / p->bz) * p->tiles_x + x / kBX;
 }
 
 // ---- pinned staging of the point lists ---------------------------------------------------------------------------
@@ -487,67 +527,62 @@ static int stage_end(fwi_fd2d* p) {
     return FWI_OK;
 }
 
-static int build_point_list(fwi_fd2d* p, PointList& pl, int n, const int* iz, const int* iy, const int* ix, const char* what) {
-    const int nbins = (p->ny > 1) ? p->tiles_x * p->tiles_y * p->nzch : p->tiles_x * p->tiles_z;
-    std::vector<int> tile_ptr(nbins + 1, 0), off(std::max(n, 1)), id(std::max(n, 1));
+// Bins points by the CTA tiles of a kernel family: (z, y, x) tile size and count, and the first plane of the z tiles (the
+// 3-D kernel's z chunks start at the slab's first owned plane).  Bin (tz, ty, tx) is the CTA (tx, ty, tz) of the launch.
+struct TileGrid { int size[3], count[3], z0; };
+
+static TileGrid tile_grid(const fwi_fd2d* p, Family f) {
+    if (f == k3D) return {{p->zchunk, p->fd3->rows, k3BX}, {p->nzch, p->tiles_y, p->tiles_x}, p->z_own0};
+    if (f == kTb2) return {{p->tb2->rows, 1, kT2CX}, {p->tiles_z2, 1, p->tiles_x2}, 0};
+    return {{p->tile->rows, 1, kBX}, {p->tiles_z, 1, p->tiles_x}, 0};
+}
+
+// Lists each point in every tile whose core widened by `reach` on each side holds it: reach 0 gives the single owning tile,
+// kHalo the tb2 kernel's extended list.  A counting sort keeps the points of a bin in input order.
+static int build_point_list(fwi_fd2d* p, PointList& pl, const TileGrid& g, int reach, int n, const int* iz, const int* iy,
+                            const int* ix, const char* what) {
+    const int nbins = g.count[0] * g.count[1] * g.count[2];
+    const int z_own1 = p->z_own1 > 0 ? p->z_own1 : p->nz;
+    std::vector<int> tile_ptr(nbins + 1, 0);
+    std::vector<std::pair<int, int>> hits;      // (bin, point) in input order
+    hits.reserve(n);
     for (int i = 0; i < n; ++i) {
         const int yy = iy ? iy[i] : 0;
         FWI_REQUIRE(iz[i] >= 0 && iz[i] < p->nz && ix[i] >= 0 && ix[i] < p->nx && yy >= 0 && yy < p->ny, "%s %d at (z=%d, y=%d, x=%d) is outside the %d x %d x %d grid", what, i, iz[i], yy, ix[i], p->nz, p->ny, p->nx);
-        tile_ptr[owner_bin(p, iz[i], yy, ix[i]) + 1]++;
+        // a slab computes only its owned planes; the neighbours overwrite the ghost planes
+        FWI_REQUIRE(iz[i] >= p->z_own0 && iz[i] < z_own1, "%s %d at z=%d is outside the planes [%d, %d) this slab owns", what, i, iz[i], p->z_own0, z_own1);
+        const int c[3] = {iz[i] - g.z0, yy, ix[i]};
+        int lo[3], hi[3];
+        for (int d = 0; d < 3; ++d) {
+            lo[d] = std::max(0, (c[d] - reach) / g.size[d]);
+            hi[d] = std::min(g.count[d] - 1, (c[d] + reach) / g.size[d]);
+        }
+        for (int tz = lo[0]; tz <= hi[0]; ++tz)
+            for (int ty = lo[1]; ty <= hi[1]; ++ty)
+                for (int tx = lo[2]; tx <= hi[2]; ++tx) {
+                    const int b = (tz * g.count[1] + ty) * g.count[2] + tx;
+                    hits.push_back({b, i});
+                    tile_ptr[b + 1]++;
+                }
     }
     for (int t = 0; t < nbins; ++t) tile_ptr[t + 1] += tile_ptr[t];
-    std::vector<int> fill(tile_ptr.begin(), tile_ptr.end() - 1);
-    for (int i = 0; i < n; ++i) {
-        const int yy = iy ? iy[i] : 0;
-        const int e = fill[owner_bin(p, iz[i], yy, ix[i])]++;
-        off[e] = (iz[i] * p->ny + yy) * p->px + ix[i];
+    const int tot = std::max(1, tile_ptr[nbins]);
+    std::vector<int> fill(tile_ptr.begin(), tile_ptr.end() - 1), off(tot), id(tot);
+    for (const auto& h : hits) {
+        const int i = h.second, e = fill[h.first]++;
+        off[e] = (iz[i] * p->ny + (iy ? iy[i] : 0)) * p->px + ix[i];
         id[e] = i;
     }
-    if (pl.nbins != nbins || pl.cap < std::max(n, 1)) {     // allocations change -> cached graphs hold stale pointers
+    if (pl.nbins != nbins || pl.cap < tot) {     // allocations change -> cached graphs hold stale pointers
         pl.release();
         drop_graphs(p);
-        const int cap = std::max(n, 1);
+        const int cap = tot + tot / 2 + 16;      // slack: the tb2 extended lists vary a little from shot to shot
         FWI_CUDA(cudaMalloc(&pl.d_tile_ptr, (nbins + 1) * sizeof(int)));
         FWI_CUDA(cudaMalloc(&pl.d_off, cap * sizeof(int)));
         FWI_CUDA(cudaMalloc(&pl.d_id, cap * sizeof(int)));
         pl.cap = cap; pl.nbins = nbins;
     }
     // contents are rewritten in place on the work stream, ordered after the previous shot's graph
-    int rc = stage_upload(p, pl.d_tile_ptr, tile_ptr.data(), nbins + 1);
-    if (!rc) rc = stage_upload(p, pl.d_off, off.data(), std::max(n, 1));
-    if (!rc) rc = stage_upload(p, pl.d_id, id.data(), std::max(n, 1));
-    if (rc) return rc;
-    pl.n = n;
-    return FWI_OK;
-}
-
-// variant 2: bin points by the 120 x cz core tiles; with `ext` a point is listed in every tile whose core +- 4 holds it
-static int build_point_list_tb2(fwi_fd2d* p, PointList& pl, int n, const int* iz, const int* ix, bool ext) {
-    const int nbins = p->tiles_x2 * p->tiles_z2;
-    std::vector<std::vector<std::pair<int, int>>> bins(nbins);
-    const int h = ext ? kHalo : 0;
-    for (int i = 0; i < n; ++i) {
-        const int tz0 = std::max(0, (iz[i] - h) / p->cz), tz1 = std::min(p->tiles_z2 - 1, (iz[i] + h) / p->cz);
-        const int tx0 = std::max(0, (ix[i] - h) / kT2CX), tx1 = std::min(p->tiles_x2 - 1, (ix[i] + h) / kT2CX);
-        for (int tz = tz0; tz <= tz1; ++tz)
-            for (int tx = tx0; tx <= tx1; ++tx) bins[tz * p->tiles_x2 + tx].push_back({iz[i] * p->px + ix[i], i});
-    }
-    std::vector<int> tile_ptr(nbins + 1, 0), off, id;
-    for (int t = 0; t < nbins; ++t) {
-        tile_ptr[t + 1] = tile_ptr[t] + (int)bins[t].size();
-        for (auto& e : bins[t]) { off.push_back(e.first); id.push_back(e.second); }
-    }
-    const int tot = std::max<int>(1, (int)off.size());
-    off.resize(tot); id.resize(tot);
-    if (pl.nbins != nbins || pl.cap < tot) {
-        pl.release();
-        drop_graphs(p);
-        const int cap = tot + tot / 2 + 16;          // extended lists vary a little from shot to shot
-        FWI_CUDA(cudaMalloc(&pl.d_tile_ptr, (nbins + 1) * sizeof(int)));
-        FWI_CUDA(cudaMalloc(&pl.d_off, cap * sizeof(int)));
-        FWI_CUDA(cudaMalloc(&pl.d_id, cap * sizeof(int)));
-        pl.cap = cap; pl.nbins = nbins;
-    }
     int rc = stage_upload(p, pl.d_tile_ptr, tile_ptr.data(), nbins + 1);
     if (!rc) rc = stage_upload(p, pl.d_off, off.data(), tot);
     if (!rc) rc = stage_upload(p, pl.d_id, id.data(), tot);
@@ -556,42 +591,42 @@ static int build_point_list_tb2(fwi_fd2d* p, PointList& pl, int n, const int* iz
     return FWI_OK;
 }
 
-template <int BZ, int NW>
-static int launch_step_cfg(fwi_fd2d* p, int mode, int cur, float* oldnew, const PointList* inj, const float* inj_vals,
-                           const PointList* rec, float* rec_out, float* snap, cudaStream_t st, const float* snap_prev = nullptr) {
-    Step2DArgs a{};
-    a.oldnew = oldnew; a.m = p->m; a.gx = p->gx; a.gz = p->gz; a.snap = snap; a.acc = p->acc; a.snap_prev = snap_prev;
-    a.nx = p->nx; a.nz = p->nz; a.px = p->px;
-    a.inj = (inj && inj->n) ? inj->dev() : PointListDev{nullptr, nullptr, nullptr};
-    a.inj_vals = inj_vals;
-    a.rec = (rec && rec->n) ? rec->dev() : PointListDev{nullptr, nullptr, nullptr};
-    a.rec_out = rec_out;
-    const dim3 grid(p->tiles_x, p->tiles_z), block(NW * 32);
-    const size_t smem = (size_t)(kBX + 2 * kHalo) * (BZ + 2 * kHalo) * sizeof(float);
-    // Programmatic dependent launch: consecutive steps are chained with a programmatic edge (also inside captured graphs),
-    // the kernel orders itself behind its predecessor with griddepcontrol.wait.
+// Launches the kernel of `mode` of a step-kernel shape.  With `pdl` it is chained to the previous kernel on the stream by a
+// programmatic edge (also inside captured graphs) and orders itself behind its predecessor with griddepcontrol.wait.
+template <typename Kernel, typename... Args>
+static int launch_shape(const StepShape<Kernel>& k, int mode, dim3 grid, bool pdl, cudaStream_t st, const Args&... args) {
+    FWI_REQUIRE(k.fn[mode], "fd2d: the %d-row kernel has no step mode %d", k.rows, mode);
     cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cfg.gridDim = grid; cfg.blockDim = dim3(k.warps * 32); cfg.dynamicSmemBytes = k.smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = (p->pdl && p->pdl_chain) ? 1 : 0;
-    p->pdl_chain = true;
-    if (mode == STEP_FWD) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_FWD>, p->tmap[cur], a));
-    else if (mode == STEP_FWD_SAVE) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, p->tmap[cur], a));
-    else if (mode == STEP_ADJ2) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_ADJ2>, p->tmap[cur], a));
-    else FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_step_kernel<BZ, NW, STEP_ADJ>, p->tmap[cur], a));
+    cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
+    FWI_CUDA(cudaLaunchKernelEx(&cfg, k.fn[mode], args...));
     return FWI_OK;
 }
 
-static int launch_step3(fwi_fd2d* p, int mode, int cur, float* oldnew, const PointList* inj, const float* inj_vals,
-                        const PointList* rec, float* rec_out, float* snap, cudaStream_t st, const float* snap_prev) {
+static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const PointList* inj, const float* inj_vals,
+                       const PointList* rec, float* rec_out, float* snap, cudaStream_t st, const float* snap_prev = nullptr) {
+    p->launches++;
+    if (p->family != k3D) {
+        Step2DArgs a{};
+        a.oldnew = oldnew; a.m = p->m; a.gx = p->gx; a.gz = p->gz; a.snap = snap; a.acc = p->acc; a.snap_prev = snap_prev;
+        a.nx = p->nx; a.nz = p->nz; a.px = p->px;
+        a.inj = PointList::dev(inj);
+        a.inj_vals = inj_vals;
+        a.rec = PointList::dev(rec);
+        a.rec_out = rec_out;
+        const bool pdl = p->pdl && p->pdl_chain;
+        p->pdl_chain = true;
+        return launch_shape(*p->tile, mode, dim3(p->tiles_x, p->tiles_z), pdl, st, p->tmap[cur], a);
+    }
     Step3DArgs a{};
     a.oldnew = oldnew; a.m = p->m; a.gx = p->gx; a.gy = p->gy; a.gz = p->gz; a.snap = snap; a.acc = p->acc; a.snap_prev = snap_prev;
     a.nx = p->nx; a.ny = p->ny; a.nz = p->nz; a.px = p->px; a.zchunk = p->zchunk;
-    a.inj = (inj && inj->n) ? inj->dev() : PointListDev{nullptr, nullptr, nullptr};
+    a.inj = PointList::dev(inj);
     a.inj_vals = inj_vals;
-    a.rec = (rec && rec->n) ? rec->dev() : PointListDev{nullptr, nullptr, nullptr};
+    a.rec = PointList::dev(rec);
     a.rec_out = rec_out;
     a.z_own0 = p->z_own0; a.z_own1 = p->z_own1 > 0 ? p->z_own1 : p->nz;
     int oi = -1;
@@ -605,31 +640,8 @@ static int launch_step3(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poi
     a.flag_peer_up = p->peer_arena[0] ? (int*)((char*)p->peer_arena[0] + p->peer_flags_off[0]) + kSyncFlagDn : nullptr;   // I am its lower neighbour
     a.flag_peer_dn = p->peer_arena[1] ? (int*)((char*)p->peer_arena[1] + p->peer_flags_off[1]) + kSyncFlagUp : nullptr;   // I am its upper neighbour
     a.timeout_cycles = p->slab_timeout_cycles;
-    const dim3 grid(p->tiles_x, p->tiles_y, p->nzch);
     // (programmatic dependent launch was measured on this kernel too: 2 % at 128^3, nothing from 256^3 up - not used)
-#define LAUNCH3(BYV)                                                                                                         \
-    do {                                                                                                                        \
-        const dim3 block(T3<BYV>::Threads);                                                                                     \
-        const size_t smem = T3<BYV>::Smem;                                                                                      \
-        if (mode == STEP_FWD) fd3d_step_kernel<STEP_FWD, BYV><<<grid, block, smem, st>>>(p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);               \
-        else if (mode == STEP_FWD_SAVE) fd3d_step_kernel<STEP_FWD_SAVE, BYV><<<grid, block, smem, st>>>(p->tm3[cur], p->tm3_old[oi], p->tm3_m, a); \
-        else if (mode == STEP_ADJ2) fd3d_step_kernel<STEP_ADJ2, BYV><<<grid, block, smem, st>>>(p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);        \
-        else fd3d_step_kernel<STEP_ADJ, BYV><<<grid, block, smem, st>>>(p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);                               \
-    } while (0)
-    if (p->by == 14) LAUNCH3(14); else LAUNCH3(16);
-#undef LAUNCH3
-    return FWI_OK;
-}
-
-static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const PointList* inj, const float* inj_vals,
-                       const PointList* rec, float* rec_out, float* snap, cudaStream_t st, const float* snap_prev = nullptr) {
-    p->launches++;
-    if (p->ny > 1) return launch_step3(p, mode, cur, oldnew, inj, inj_vals, rec, rec_out, snap, st, snap_prev);
-#define CFG(BZV, NWV) if (p->bz == BZV && p->nw == NWV) return launch_step_cfg<BZV, NWV>(p, mode, cur, oldnew, inj, inj_vals, rec, rec_out, snap, st, snap_prev)
-    CFG(32, 4); CFG(28, 4); CFG(42, 6); CFG(56, 8);      // every entry of kStepTiles
-#undef CFG
-    set_error("fd2d: unsupported tile configuration bz=%d nw=%d", p->bz, p->nw);
-    return FWI_EINVAL;
+    return launch_shape(*p->fd3, mode, dim3(p->tiles_x, p->tiles_y, p->nzch), false, st, p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);
 }
 
 static int ensure_floats(fwi_fd2d* p, float** ptr, size_t* cap, size_t need_floats) {
@@ -650,7 +662,7 @@ static void other_two(const State& s, int base, int& a, int& b) {
     a = f[0]; b = f[1];
 }
 static State advance_state(const fwi_fd2d* p, State s, int base, int nsteps) {
-    if (p->variant == 2 && p->ny == 1) {
+    if (p->family == kTb2) {
         for (int k = 0; k + 1 < nsteps; k += 2) { int a, b; other_two(s, base, a, b); s = State{a, b}; }
         if (nsteps & 1) s = State{s.o, s.c};
         return s;
@@ -659,50 +671,21 @@ static State advance_state(const fwi_fd2d* p, State s, int base, int nsteps) {
     return s;
 }
 
-template <int CZ, int NW>
-static int launch_tb2_cfg(fwi_fd2d* p, int mode, const State& s, int jc, int jd, const PointList* inj_ext, const PointList* inj_own,
-                          const float* inj1, const float* inj2, const PointList* rec, float* rec1, float* rec2, float* snap1,
-                          float* snap2, cudaStream_t st) {
-    Tb2Args a{};
-    a.out_new = p->fld[jc]; a.out_mid = p->fld[jd]; a.gx = p->gx; a.gz = p->gz; a.m = p->m; a.snap1 = snap1; a.snap2 = snap2; a.acc = p->acc;
-    a.nx = p->nx; a.nz = p->nz; a.px = p->px;
-    const PointListDev none{nullptr, nullptr, nullptr};
-    a.inj_ext = (inj_ext && inj_ext->n) ? inj_ext->dev() : none;
-    a.inj_own = (inj_own && inj_own->n) ? inj_own->dev() : none;
-    a.inj1 = inj1; a.inj2 = inj2;
-    a.rec = (rec && rec->n) ? rec->dev() : none;
-    a.rec1 = rec1; a.rec2 = rec2;
-    const dim3 grid(p->tiles_x2, p->tiles_z2), block(NW * 32);
-    const size_t smem = ((size_t)(CZ + 16) * kT2W0 + 2 * (size_t)(CZ + 8) * kT2W1) * sizeof(float);
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = (p->pdl && p->pdl_chain) ? 1 : 0;      // the pass loads m before its dependency wait
-    p->pdl_chain = true;
-    if (mode == STEP_FWD) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_tb2_kernel<CZ, NW, STEP_FWD>, p->tb_cur[s.c], p->tb_old[s.o], p->tb_m, a));
-    else if (mode == STEP_FWD_SAVE) FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_tb2_kernel<CZ, NW, STEP_FWD_SAVE>, p->tb_cur[s.c], p->tb_old[s.o], p->tb_m, a));
-    else FWI_CUDA(cudaLaunchKernelEx(&cfg, fd2d_tb2_kernel<CZ, NW, STEP_ADJ>, p->tb_cur[s.c], p->tb_old[s.o], p->tb_m, a));
-    return FWI_OK;
-}
-template <int CZ, int NW>
-static int tb2_attrs() {
-    const int smem = (int)(((size_t)(CZ + 16) * kT2W0 + 2 * (size_t)(CZ + 8) * kT2W1) * sizeof(float));
-    FWI_CUDA(cudaFuncSetAttribute(fd2d_tb2_kernel<CZ, NW, STEP_FWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    FWI_CUDA(cudaFuncSetAttribute(fd2d_tb2_kernel<CZ, NW, STEP_FWD_SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    FWI_CUDA(cudaFuncSetAttribute(fd2d_tb2_kernel<CZ, NW, STEP_ADJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    return FWI_OK;
-}
 static int launch_tb2(fwi_fd2d* p, int mode, const State& s, int jc, int jd, const PointList* inj_ext, const PointList* inj_own,
                       const float* inj1, const float* inj2, const PointList* rec, float* rec1, float* rec2, float* snap1, float* snap2,
                       cudaStream_t st) {
     p->launches++;
-#define TB(CZV, NWV) if (p->cz == CZV && p->tb_nw == NWV) return launch_tb2_cfg<CZV, NWV>(p, mode, s, jc, jd, inj_ext, inj_own, inj1, inj2, rec, rec1, rec2, snap1, snap2, st)
-    TB(32, 8); TB(24, 8);
-#undef TB
-    set_error("fd2d: unsupported temporal-blocking tile cz=%d", p->cz);
-    return FWI_EINVAL;
+    Tb2Args a{};
+    a.out_new = p->fld[jc]; a.out_mid = p->fld[jd]; a.gx = p->gx; a.gz = p->gz; a.m = p->m; a.snap1 = snap1; a.snap2 = snap2; a.acc = p->acc;
+    a.nx = p->nx; a.nz = p->nz; a.px = p->px;
+    a.inj_ext = PointList::dev(inj_ext);
+    a.inj_own = PointList::dev(inj_own);
+    a.inj1 = inj1; a.inj2 = inj2;
+    a.rec = PointList::dev(rec);
+    a.rec1 = rec1; a.rec2 = rec2;
+    const bool pdl = p->pdl && p->pdl_chain;      // the pass loads m before its dependency wait
+    p->pdl_chain = true;
+    return launch_shape(*p->tb2, mode, dim3(p->tiles_x2, p->tiles_z2), pdl, st, p->tb_cur[s.c], p->tb_old[s.o], p->tb_m, a);
 }
 
 // forward time loop over steps [n0, n1); `s` holds the fld[] indices of (u_n, u_{n-1}) on entry and on return
@@ -711,7 +694,7 @@ static int run_forward(fwi_fd2d* p, const float* wavelet, int n0, int n1, float*
     const size_t pl = p->plane();
     p->pdl_chain = false;             // (segment of) a sweep starts behind memsets / checkpoint copies: full dependency
     int n = n0;
-    if (p->variant == 2 && p->ny == 1) {
+    if (p->family == kTb2) {
         for (; n + 1 < n1; n += 2) {
             int jc, jd;
             other_two(s, 0, jc, jd);
@@ -725,7 +708,7 @@ static int run_forward(fwi_fd2d* p, const float* wavelet, int n0, int n1, float*
         }
     }
     // a leftover single step behind a two-steps-per-pass launch reads u_{n-1} written by that very pass: no chaining
-    if (p->variant == 2 && p->ny == 1) p->pdl_chain = false;
+    if (p->family == kTb2) p->pdl_chain = false;
     for (; n < n1; ++n) {
         float* snap = save ? p->snap + (size_t)(n - snap_base) * pl : nullptr;
         int rc = launch_step(p, save ? STEP_FWD_SAVE : STEP_FWD, s.c, p->fld[s.o], &p->src, wavelet + (size_t)n * p->nsrc,
@@ -742,7 +725,7 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
     const size_t pl = p->plane();
     p->pdl_chain = false;             // first adjoint step follows the residual kernel and the field memsets
     int n = n1 - 1;
-    if (p->variant == 2 && p->ny == 1) {
+    if (p->family == kTb2) {
         for (; n - 1 >= n0; n -= 2) {
             int jc, jd;
             other_two(s, 4, jc, jd);
@@ -752,7 +735,7 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
             s = State{jc, jd};
         }
     }
-    if ((p->ny > 1 || p->variant == 0) && p->defer_imaging) {
+    if (p->family != kTb2 && p->defer_imaging) {
         // deferred imaging: the first step of a pair only propagates (17 B/pt of traffic instead of 29), the second one
         // images both fields, touching the accumulator once per two steps
         for (; n - 1 >= n0; n -= 2) {
@@ -765,7 +748,7 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
             s = State{s.o, s.c};
         }
     }
-    if (p->variant == 2 && p->ny == 1) p->pdl_chain = false;          // see run_forward: leftover step behind a two-step pass
+    if (p->family == kTb2) p->pdl_chain = false;          // see run_forward: leftover step behind a two-step pass
     for (; n >= n0; --n) {
         int rc = launch_step(p, STEP_ADJ, s.c, p->fld[s.o], &p->rec, resid + (size_t)n * p->nrec, nullptr, nullptr,
                              p->snap + (size_t)(n - snap_base) * pl, st);
@@ -915,6 +898,13 @@ static int leave(fwi_fd2d* p, cudaStream_t user) {       // ... and the caller's
     return FWI_OK;
 }
 
+template <typename Shape, size_t N> static int allow_smem(const Shape (&table)[N]) {
+    for (const auto& k : table)
+        for (auto fn : k.fn)
+            if (fn) FWI_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
+    return FWI_OK;
+}
+
 extern "C" {
 
 static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, float dt, int nabs, float alpha);
@@ -931,6 +921,7 @@ static int create_plan(int device, int nz, int ny, int nx, float h, float dt, in
     FWI_REQUIRE(device >= 0 && device < ndev, "fwi_fd2d_create: device %d out of range (%d visible)", device, ndev);
     DeviceGuard g(device);
     auto* p = new fwi_fd2d();
+    p->family = ny > 1 ? k3D : kTile;
     const int rc = init_plan(p, device, nz, ny, nx, h, dt, nabs, alpha);
     if (rc) { fwi_fd2d_destroy(p); return rc; }          // nothing half-built leaks
     *out = p;
@@ -941,7 +932,7 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
     p->device = device; p->nz = nz; p->ny = ny; p->nx = nx; p->h = h; p->dt = dt; p->nabs = nabs; p->alpha = alpha;
     p->px = (nx + 31) & ~31;
     p->tiles_x = (nx + kBX - 1) / kBX;
-    p->tiles_z = (nz + p->bz - 1) / p->bz;
+    p->tiles_z = (nz + p->tile->rows - 1) / p->tile->rows;
     const size_t pl = p->plane();
     FWI_CUDA(cudaStreamCreateWithFlags(&p->work, cudaStreamNonBlocking));
     FWI_CUDA(cudaEventCreateWithFlags(&p->ev_in, cudaEventDisableTiming));
@@ -984,14 +975,8 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
     cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, device);
     int rc = make_tmaps(p);
     if (rc) return rc;
-    if ((rc = tb2_attrs<32, 8>()) || (rc = tb2_attrs<24, 8>())) return rc;
-#define ATTR3(BYV)                                                                                                                        \
-    FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_FWD, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem));        \
-    FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_FWD_SAVE, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem));   \
-    FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_ADJ, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem));        \
-    FWI_CUDA(cudaFuncSetAttribute(fd3d_step_kernel<STEP_ADJ2, BYV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)T3<BYV>::Smem))
-    ATTR3(16); ATTR3(14);
-#undef ATTR3
+    // the tb2 and 3-D kernels take more than the default 48 KB of dynamic shared memory (the tile kernel stays below it)
+    if ((rc = allow_smem(kTb2Shapes)) || (rc = allow_smem(kFd3Shapes))) return rc;
     return FWI_OK;
 }
 
@@ -1001,14 +986,16 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
 // Model cost: ceil(tiles / SMs) x (rows + 4) - the 8 halo rows are loaded but not computed.  Measured at 1000 x 3000, us per
 // forward+adjoint step pair: 32 rows 16.67, 28: 15.34, 42: 15.50, 56: 15.56 (forward step 6.77 / 5.83 / 5.94 / 5.85); at
 // 1500 x 3000: 27.9 / 25.9 / 26.1 / 26.8.  The kernels are bit-identical, only the decomposition differs.
-static void pick_tile(int nz, int nx, int sms, int* bz, int* nw) {
+static const TileShape* pick_tile(int nz, int nx, int sms) {
     const long tx = (nx + kBX - 1) / kBX;
+    const TileShape* pick = kTileShapes;
     double best = 1e300;
-    for (const auto& c : kStepTiles) {
-        const long tiles = tx * ((nz + c[0] - 1) / c[0]);
-        const double cost = (double)((tiles + sms - 1) / sms) * (c[0] + 4);
-        if (cost < best - 1e-9) { best = cost; *bz = c[0]; *nw = c[1]; }
+    for (const auto& k : kTileShapes) {
+        const long tiles = tx * ((nz + k.rows - 1) / k.rows);
+        const double cost = (double)((tiles + sms - 1) / sms) * (k.rows + 4);
+        if (cost < best - 1e-9) { best = cost; pick = &k; }
     }
+    return pick;
 }
 
 int fwi_fd2d_create(int device, int nz, int nx, float h, float dt, int nabs, float alpha, fwi_fd2d** out) {
@@ -1027,10 +1014,9 @@ int fwi_fd2d_create(int device, int nz, int nx, float h, float dt, int nabs, flo
         else if (pts > 7.5e6) rc = fwi_fd2d_set_tb2(*out, 32);
         if (rc) { fwi_fd2d_destroy(*out); *out = nullptr; return rc; }
     }
-    if ((*out)->variant == 0 && nz >= 32) {
-        int bz = 32, nw = 4;
-        pick_tile(nz, nx, (*out)->sm_count, &bz, &nw);
-        rc = fwi_fd2d_set_tile(*out, bz, nw);
+    if ((*out)->family == kTile && nz >= 32) {
+        const TileShape* t = pick_tile(nz, nx, (*out)->sm_count);
+        rc = fwi_fd2d_set_tile(*out, t->rows, t->warps);
         if (rc) { fwi_fd2d_destroy(*out); *out = nullptr; }
     }
     return rc;
@@ -1067,14 +1053,13 @@ int fwi_fd2d_destroy(fwi_fd2d* p) {
 
 int fwi_fd2d_set_tile(fwi_fd2d* p, int bz, int nw) {
     FWI_REQUIRE(p, "fwi_fd2d_set_tile: NULL plan");
-    bool ok = false;
-    for (const auto& c : kStepTiles) ok = ok || (bz == c[0] && nw == c[1]);
-    FWI_REQUIRE(ok, "fwi_fd2d_set_tile: unsupported (bz=%d, nw=%d)", bz, nw);
-    FWI_REQUIRE(p->ny == 1, "fwi_fd2d_set_tile: 2-D plans only");
+    const TileShape* t = find_shape(kTileShapes, bz, nw);
+    FWI_REQUIRE(t, "fwi_fd2d_set_tile: unsupported (bz=%d, nw=%d)", bz, nw);
+    FWI_REQUIRE(p->family != k3D, "fwi_fd2d_set_tile: 2-D plans only");
     DeviceGuard g(p->device);
     FWI_CUDA(cudaStreamSynchronize(p->work));
     drop_graphs(p);
-    p->variant = 0; p->bz = bz; p->nw = nw;
+    p->family = kTile; p->tile = t;
     p->tiles_z = (p->nz + bz - 1) / bz;
     p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;      // tile binning changed
     return make_tmaps(p);
@@ -1082,13 +1067,13 @@ int fwi_fd2d_set_tile(fwi_fd2d* p, int bz, int nw) {
 
 int fwi_fd2d_set_tb2(fwi_fd2d* p, int cz) {
     FWI_REQUIRE(p, "fwi_fd2d_set_tb2: NULL plan");
-    FWI_REQUIRE(cz == 24 || cz == 32, "fwi_fd2d_set_tb2: unsupported core rows %d (24, 32)", cz);
-    FWI_REQUIRE(p->ny == 1, "fwi_fd2d_set_tb2: 2-D plans only");
+    const Tb2Shape* t = find_shape(kTb2Shapes, cz, kTb2Warps);
+    FWI_REQUIRE(t, "fwi_fd2d_set_tb2: unsupported core rows %d", cz);
+    FWI_REQUIRE(p->family != k3D, "fwi_fd2d_set_tb2: 2-D plans only");
     DeviceGuard g(p->device);
     FWI_CUDA(cudaStreamSynchronize(p->work));
     drop_graphs(p);
-    p->variant = 2; p->cz = cz;
-    p->tb_nw = 8;                                                      // warps per CTA (4 warps at 24 rows measured 8 % slower)
+    p->family = kTb2; p->tb2 = t;
     p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;
     p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
     return make_tmaps(p);
@@ -1129,15 +1114,17 @@ static int set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_
     const size_t bins = (size_t)std::max({p->tiles_x * p->tiles_y * p->nzch, p->tiles_x * p->tiles_z, p->tiles_x2 * p->tiles_z2}) + 1;
     int rc = stage_begin(p, 6 * bins + 2 * 10 * ((size_t)nsrc + nrec + 16));      // 2 + 4 lists; a tb2 point sits in <= 4 tiles
     if (rc) return rc;
-    rc = build_point_list(p, p->src, nsrc, src_z, src_y, src_x, "source");
+    const TileGrid step = tile_grid(p, p->family == k3D ? k3D : kTile);     // tb2 plans run the tile kernel for single steps
+    rc = build_point_list(p, p->src, step, 0, nsrc, src_z, src_y, src_x, "source");
     if (rc) return rc;
-    rc = build_point_list(p, p->rec, nrec, rec_z, rec_y, rec_x, "receiver");
+    rc = build_point_list(p, p->rec, step, 0, nrec, rec_z, rec_y, rec_x, "receiver");
     if (rc) return rc;
-    if (p->variant == 2 && p->ny == 1) {
-        if ((rc = build_point_list_tb2(p, p->src_ext2, nsrc, src_z, src_x, true))) return rc;
-        if ((rc = build_point_list_tb2(p, p->src_own2, nsrc, src_z, src_x, false))) return rc;
-        if ((rc = build_point_list_tb2(p, p->rec_ext2, nrec, rec_z, rec_x, true))) return rc;
-        if ((rc = build_point_list_tb2(p, p->rec_own2, nrec, rec_z, rec_x, false))) return rc;
+    if (p->family == kTb2) {
+        const TileGrid pass = tile_grid(p, kTb2);
+        if ((rc = build_point_list(p, p->src_ext2, pass, kHalo, nsrc, src_z, src_y, src_x, "source"))) return rc;
+        if ((rc = build_point_list(p, p->src_own2, pass, 0, nsrc, src_z, src_y, src_x, "source"))) return rc;
+        if ((rc = build_point_list(p, p->rec_ext2, pass, kHalo, nrec, rec_z, rec_y, rec_x, "receiver"))) return rc;
+        if ((rc = build_point_list(p, p->rec_own2, pass, 0, nrec, rec_z, rec_y, rec_x, "receiver"))) return rc;
     }
     p->nsrc = nsrc; p->nrec = nrec;
     return stage_end(p);

@@ -24,7 +24,7 @@ from . import fd_oracle as fo
 
 EPS32 = float(np.finfo(np.float32).eps)
 HALO = 4
-STEP_TILES = ((32, 4), (28, 4), (42, 6), (56, 8))        # the one-step kernel's built (rows, warps); csrc/fd2d.cu kStepTiles
+STEP_TILES = ((32, 4), (28, 4), (42, 6), (56, 8))        # the one-step kernel's built (rows, warps); csrc/fd2d.cu kTileShapes
 TB2_CORE_X = 120                                         # two-steps-per-pass kernel: 120-column core tiles (fd2d_tb2.cuh)
 TILE_X = 128                                             # one-step 2-D and 3-D kernels: 128-column tiles
 

@@ -133,6 +133,31 @@ def test_slab_owned_range_logic_on_one_gpu(ac):
         p.close()
 
 
+def test_slab_rejects_points_in_ghost_planes(ac):
+    """A slab computes only its owned planes and its neighbours overwrite the ghost planes, so a source or receiver there
+    would be injected into a plane that is overwritten, or binned past the last z chunk.  The two plans of
+    test_slab_owned_range_logic_on_one_gpu: set_geometry accepts points in the first and last owned planes and raises
+    ValueError, naming the owned range, for a source or a receiver in either ghost zone."""
+    from full_waveform_inversion_b200 import _lib
+    shape = (48, 20, 140)
+    H, half = 4, shape[0] // 2
+    lib = _lib.load()
+    for r in range(2):
+        up, down = (H if r else 0), (0 if r else H)
+        p = ac.Propagator((half + up + down,) + shape[1:], 10.0, 1e-3, nabs=6, graphs=False)
+        _lib.check(lib.fwi_fd_slab_connect(p._h, up, up + half, None, None, 0, None, None))
+        owned = [(up, 10, 40), (up + half - 1, 3, 139)]
+        p.set_geometry(owned, owned)
+        ghosts = range(half, half + H) if down else range(0, H)
+        for z in (ghosts[0], ghosts[-1]):
+            bad = [(z, 10, 40)]
+            with pytest.raises(ValueError, match=r"\[%d, %d\)" % (up, up + half)):
+                p.set_geometry(bad, owned)
+            with pytest.raises(ValueError, match=r"\[%d, %d\)" % (up, up + half)):
+                p.set_geometry(owned, owned + bad)
+        p.close()
+
+
 def _local_slabs(ac, shape, h, dt, nabs, nslab, v, src, rec, **kw):
     """What SlabPropagator builds per rank, for `nslab` plans living on ONE GPU and connected with
     fwi_fd_slab_connect_local (the peer-memory protocol without IPC)."""
