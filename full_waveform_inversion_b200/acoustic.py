@@ -9,7 +9,7 @@ over shots.
 
 Conventions: velocity grids are (nz, nx) [2-D] or (nz, ny, nx) [3-D] float32, x contiguous;
 a shot is ``(src, rec)`` with integer index arrays of shape (n, ndim) in (z[, y], x) order;
-wavelets are (nt,) or (nt, nsrc); traces are (nt, nrec), time-major.
+wavelets are (nt,) or (nt, nsrc); traces are (nt, nrec), time-major; a velocity perturbation dv is grid-shaped.
 """
 from __future__ import annotations
 
@@ -35,6 +35,8 @@ _lib.register({
     "fwi_fd2d_forward": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "fwi_fd2d_wavefield": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "fwi_fd2d_gradient": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, POINTER(c_double), c_void_p]),
+    "fwi_fd2d_born": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "fwi_fd2d_gauss_newton": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "fwi_fd2d_launch_count": (c_int64, [c_void_p]),
     "fwi_fd3d_create": (c_int, [c_int, c_int, c_int, c_int, c_float, c_float, c_int, c_float, POINTER(c_void_p)]),
     "fwi_fd3d_set_geometry": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
@@ -184,6 +186,44 @@ class Propagator:
             check(self._lib.fwi_fd2d_gradient(self._h, ptr(w), ptr(obs), nt, ptr(grad), ptr(traces),
                                               ctypes.byref(J) if want_misfit else None, current_stream()))
         return (J.value if want_misfit else None), grad, traces
+
+    def _grid_arg(self, x, name):
+        t = _dev_f32(x, self.torch_device)
+        if tuple(t.shape) != self.shape:
+            raise ValueError("%s has shape %s, expected the grid shape %s" % (name, tuple(t.shape), self.shape))
+        return t
+
+    def _out_arg(self, t, shape, name):
+        if not (isinstance(t, torch.Tensor) and tuple(t.shape) == tuple(shape) and t.dtype == torch.float32
+                and t.is_contiguous() and t.device == self.torch_device):
+            raise ValueError("%s must be a contiguous float32 tensor of shape %s on %s" % (name, tuple(shape), self.torch_device))
+        return t
+
+    def born(self, wavelet, dv, out=None, want_traces=False):
+        """Born (linearised) traces J dv for the velocity perturbation `dv` (grid-shaped) -> (dtraces (nt, nrec), background
+        traces | None)  (spec B5, tests/born_reference.py born).  `out`: caller-owned (nt, nrec) float32 buffer for J dv."""
+        w = self._wavelet(wavelet)
+        nt = w.shape[0]
+        dv = self._grid_arg(dv, "dv")
+        dtr = torch.empty((nt, self.nrec), dtype=torch.float32, device=self.torch_device) if out is None else \
+            self._out_arg(out, (nt, self.nrec), "out")
+        traces = torch.empty((nt, self.nrec), dtype=torch.float32, device=self.torch_device) if want_traces else None
+        with torch.cuda.device(self.device):
+            check(self._lib.fwi_fd2d_born(self._h, ptr(w), ptr(dv), nt, ptr(dtr), ptr(traces), current_stream()))
+        return dtr, traces
+
+    def gauss_newton(self, wavelet, dv, hv=None, want_dtraces=False):
+        """Gauss-Newton Hessian-vector product: hv (grid-shaped, accumulated into `hv`) += J^T J dv -> (hv, J dv | None)
+        (spec B5, tests/born_reference.py gauss_newton).  Snapshots are stored or checkpointed as in `gradient`."""
+        w = self._wavelet(wavelet)
+        nt = w.shape[0]
+        dv = self._grid_arg(dv, "dv")
+        hv = torch.zeros(self.shape, dtype=torch.float32, device=self.torch_device) if hv is None else \
+            self._out_arg(hv, self.shape, "hv")
+        dtr = torch.empty((nt, self.nrec), dtype=torch.float32, device=self.torch_device) if want_dtraces else None
+        with torch.cuda.device(self.device):
+            check(self._lib.fwi_fd2d_gauss_newton(self._h, ptr(w), ptr(dv), nt, ptr(hv), ptr(dtr), current_stream()))
+        return hv, dtr
 
     # ---- low-level stepping (the caller drives the time loop; used by SlabPropagator) --------------------------
     def set_profiles(self, gz=None, gy=None, gx=None):
@@ -534,6 +574,50 @@ def forward_model(v, h, dt, shots, wavelet, nabs=20, alpha=0.3, device=None, pro
             prop.set_geometry(src, rec)
             out.append(prop.forward(wavelet))
         return out
+    finally:
+        if propagator is None:
+            prop.close()
+
+
+def born_model(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None):
+    """Born traces J dv of every shot -> list of (nt, nrec) device tensors (spec B5 per shot, tests/born_reference.py)."""
+    device = torch.cuda.current_device() if device is None else device
+    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    try:
+        prop.set_model(v)
+        out = []
+        for src, rec in shots:
+            prop.set_geometry(src, rec)
+            out.append(prop.born(wavelet, dv)[0])
+        return out
+    finally:
+        if propagator is None:
+            prop.close()
+
+
+def gauss_newton_product(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None, allreduce=True,
+                         shot_ids=None):
+    """Gauss-Newton Hessian-vector product summed over shots, sum_s J_s^T J_s dv -> grid-shaped device tensor.
+
+    Under torch.distributed the shots are sharded round-robin over the ranks and the product is summed with ONE
+    all-reduce, as in `gradient`; with `shot_ids`, `shots` holds just this rank's shots."""
+    device = torch.cuda.current_device() if device is None else device
+    dist = _dist() if allreduce else None
+    if shot_ids is None:
+        ids = shard_shots(len(shots), dist.get_world_size(), dist.get_rank()) if dist else range(len(shots))
+        mine = [shots[i] for i in ids]
+    else:
+        mine = list(shots)
+    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    try:
+        prop.set_model(v)
+        hv = torch.zeros(tuple(v.shape), dtype=torch.float32, device=prop.torch_device)
+        for src, rec in mine:
+            prop.set_geometry(src, rec)
+            prop.gauss_newton(wavelet, dv, hv=hv)
+        if dist:
+            dist.all_reduce(hv)
+        return hv
     finally:
         if propagator is None:
             prop.close()

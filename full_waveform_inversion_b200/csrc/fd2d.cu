@@ -13,7 +13,8 @@
 // ~4 x 16 B per float4 of output.  u_{n-1} and m are touched once per point straight from global
 // (coalesced float4) and u_{n+1} overwrites u_{n-1} in place: 16 B of algorithmic traffic per update.
 // The forward pass can stream w_n to an HBM snapshot (evict-first stores); the adjoint pass reads it
-// back and accumulates the zero-lag cross-correlation in the same kernel.
+// back and accumulates the zero-lag cross-correlation in the same kernel.  The Born (linearised) step reads it back as the
+// source term of the scattered field: du_{n+1} = g (2 du_n - g du_{n-1} + m lap(du_n) + dm w_n)  (spec B5).
 #include "fd_common.cuh"
 #include <vector>
 #include <algorithm>
@@ -22,7 +23,9 @@
 
 namespace fwi {
 
-enum { STEP_FWD = 0, STEP_FWD_SAVE = 1, STEP_ADJ = 2, STEP_ADJ2 = 3 };   // ADJ2: image this step AND the previous one (deferred)
+// ADJ2: image this step AND the previous one (deferred).  BORN: a scattered (linearised) step whose source term is
+// dm * w_n, w_n read from the background sweep's snapshot (spec B5, tests/born_reference.py)
+enum { STEP_FWD = 0, STEP_FWD_SAVE = 1, STEP_ADJ = 2, STEP_ADJ2 = 3, STEP_BORN = 4 };
 }  // namespace fwi
 #include "fd3d.cuh"
 #include "fd2d_tb2.cuh"
@@ -41,6 +44,7 @@ struct Step2DArgs {
     const float* inj_vals;
     PointListDev rec;     // receivers to sample (forward only; tile_ptr == nullptr otherwise)
     float* rec_out;
+    const float* dm;      // BORN: model perturbation dm = (2 m / v) dv, pitched like m
 };
 
 // rows of u_{n-1} / m requested before the dependency wait.  ms per 1000-step gradient at 1000x3000: 0 rows 17.0, 1 row
@@ -119,6 +123,9 @@ __global__ void __launch_bounds__(NW * 32) fd2d_step_kernel(const __grid_constan
                 const size_t off = (size_t)z * a.px + x;
                 const float4 o4 = (r < kPrefetchRows) ? o4p[r < kPrefetchRows ? r : 0] : ld4(a.oldnew + off);
                 const float4 m4 = (r < kPrefetchRows) ? m4p[r < kPrefetchRows ? r : 0] : ld4(a.m + off);
+                float4 w4 = make_float4(0.f, 0.f, 0.f, 0.f), d4 = w4;
+                if (MODE == STEP_BORN) { w4 = ld4_stream(a.snap + off); d4 = ld4(a.dm + off); }
+                const float bw[4] = {w4.x, w4.y, w4.z, w4.w}, bd[4] = {d4.x, d4.y, d4.z, d4.w};
                 const float gzv = __ldg(a.gz + z);
                 const float ov[4] = {o4.x, o4.y, o4.z, o4.w}, mv[4] = {m4.x, m4.y, m4.z, m4.w};
                 const float gv[4] = {gx4.x * gzv, gx4.y * gzv, gx4.z * gzv, gx4.w * gzv};
@@ -132,7 +139,10 @@ __global__ void __launch_bounds__(NW * 32) fd2d_step_kernel(const __grid_constan
                     lap = fmaf(kC3, (ax[1 + j] + ax[7 + j]) + (zc[1][j] + zc[7][j]), lap);
                     lap = fmaf(kC4, (ax[0 + j] + ax[8 + j]) + (zc[0][j] + zc[8][j]), lap);
                     wv[j] = lap;
-                    nv[j] = gv[j] * fmaf(mv[j], lap, fmaf(-gv[j], ov[j], 2.0f * c));
+                    // BORN: nv = g * fma(m, lap, fma(dm, w, fma(-g, o, 2 c))) - the forward update with dm * w_n added last
+                    float rest = fmaf(-gv[j], ov[j], 2.0f * c);
+                    if (MODE == STEP_BORN) rest = fmaf(bd[j], bw[j], rest);
+                    nv[j] = gv[j] * fmaf(mv[j], lap, rest);
                 }
                 st4(a.oldnew + off, make_float4(nv[0], nv[1], nv[2], nv[3]));
                 if (MODE == STEP_FWD_SAVE) st4_stream(a.snap + off, make_float4(wv[0], wv[1], wv[2], wv[3]));
@@ -186,6 +196,15 @@ __global__ void fd_model_kernel(const float* __restrict__ v, int nz, int nx, int
     if (x < nx) { vv = v[(size_t)z * nx + x]; const float c = vv * dt_over_h; val = c * c; }
     m[(size_t)z * px + x] = val;
     vp[(size_t)z * px + x] = vv;
+}
+
+// Born: dm = (2 m / v) dv in the owned columns (dm/dv of m = (v dt / h)^2, spec B5), 0 in the pad columns
+__global__ void fd_dm_kernel(const float* __restrict__ dv, const float* __restrict__ m, const float* __restrict__ vp, int nz,
+                             int nx, int px, float* __restrict__ dm) {
+    const int x = blockIdx.y * blockDim.x + threadIdx.x, z = blockIdx.x;   // rows on grid.x (no 65535 limit)
+    if (x >= px || z >= nz) return;
+    const size_t o = (size_t)z * px + x;
+    dm[o] = (x < nx) ? 2.0f * m[o] * dv[(size_t)z * nx + x] / vp[o] : 0.f;
 }
 
 __global__ void fd_grad_finalize_kernel(const float* __restrict__ acc, const float* __restrict__ vp, int nz, int nx,
@@ -293,12 +312,12 @@ struct PointList {
 enum Family { kTile, kTb2, k3D };
 
 // One built shape of a family: tile rows (bz / cz / by), warps per CTA, dynamic shared memory per CTA, and its kernel for
-// each mode, indexed by STEP_FWD .. STEP_ADJ2 (null where the family has no such mode).  The tables below are the only
+// each mode, indexed by STEP_FWD .. STEP_BORN (null where the family has no such mode).  The tables below are the only
 // list of the shapes the library builds.
 template <typename Kernel> struct StepShape {
     int rows, warps;
     size_t smem;
-    Kernel fn[4];
+    Kernel fn[5];
 };
 using TileShape = StepShape<void (*)(CUtensorMap, Step2DArgs)>;
 using Tb2Shape = StepShape<void (*)(CUtensorMap, CUtensorMap, CUtensorMap, Tb2Args)>;
@@ -308,18 +327,18 @@ constexpr int kBX = 128;
 template <int BZ, int NW> TileShape tile_shape() {
     return {BZ, NW, (size_t)(kBX + 2 * kHalo) * (BZ + 2 * kHalo) * sizeof(float),
             {fd2d_step_kernel<BZ, NW, STEP_FWD>, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, fd2d_step_kernel<BZ, NW, STEP_ADJ>,
-             fd2d_step_kernel<BZ, NW, STEP_ADJ2>}};
+             fd2d_step_kernel<BZ, NW, STEP_ADJ2>, fd2d_step_kernel<BZ, NW, STEP_BORN>}};
 }
 constexpr int kTb2Warps = 8;          // (4 warps at 24 rows measured 8 % slower)
 template <int CZ> Tb2Shape tb2_shape() {
     return {CZ, kTb2Warps, ((size_t)(CZ + 16) * kT2W0 + 2 * (size_t)(CZ + 8) * kT2W1) * sizeof(float),
             {fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD>, fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD_SAVE>,
-             fd2d_tb2_kernel<CZ, kTb2Warps, STEP_ADJ>, nullptr}};
+             fd2d_tb2_kernel<CZ, kTb2Warps, STEP_ADJ>, nullptr, nullptr}};
 }
 template <int BY> Fd3Shape fd3_shape() {
     return {BY, T3<BY>::Threads / 32, T3<BY>::Smem,
             {fd3d_step_kernel<STEP_FWD, BY>, fd3d_step_kernel<STEP_FWD_SAVE, BY>, fd3d_step_kernel<STEP_ADJ, BY>,
-             fd3d_step_kernel<STEP_ADJ2, BY>}};
+             fd3d_step_kernel<STEP_ADJ2, BY>, fd3d_step_kernel<STEP_BORN, BY>}};
 }
 // The one-step kernel is built for exactly these (rows, warps per CTA): the round-1 sweep's winner and three heights of 7 rows
 // per warp among which one has tiles that fill whole waves.  pick_tile() breaks ties by this order.
@@ -378,6 +397,7 @@ struct fwi_fd2d {
     float* syn = nullptr; size_t syn_cap = 0;
     float* obs = nullptr; size_t obs_cap = 0;
     float* wav = nullptr; size_t wav_cap = 0;
+    float* dm = nullptr; size_t dm_cap = 0;   // Born: pitched dm = (2 m / v) dv
     double* d_J = nullptr;
     PointList src, rec;
     PointList src_ext2, src_own2, rec_ext2, rec_own2;   // tb2: binned by the 120 x cz core tiles (+-4 for *_ext2)
@@ -617,6 +637,7 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
         a.inj_vals = inj_vals;
         a.rec = PointList::dev(rec);
         a.rec_out = rec_out;
+        a.dm = p->dm;
         const bool pdl = p->pdl && p->pdl_chain;
         p->pdl_chain = true;
         return launch_shape(*p->tile, mode, dim3(p->tiles_x, p->tiles_z), pdl, st, p->tmap[cur], a);
@@ -640,6 +661,7 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
     a.flag_peer_up = p->peer_arena[0] ? (int*)((char*)p->peer_arena[0] + p->peer_flags_off[0]) + kSyncFlagDn : nullptr;   // I am its lower neighbour
     a.flag_peer_dn = p->peer_arena[1] ? (int*)((char*)p->peer_arena[1] + p->peer_flags_off[1]) + kSyncFlagUp : nullptr;   // I am its upper neighbour
     a.timeout_cycles = p->slab_timeout_cycles;
+    a.dm = p->dm;
     // (programmatic dependent launch was measured on this kernel too: 2 % at 128^3, nothing from 256^3 up - not used)
     return launch_shape(*p->fd3, mode, dim3(p->tiles_x, p->tiles_y, p->nzch), false, st, p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);
 }
@@ -759,6 +781,22 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
     return FWI_OK;
 }
 
+// scattered (Born) steps [n0, n1) on fld[4..5], one-step kernel in every 2-D family: dm * w_n is the source term, w_n the
+// snapshot the background sweep of the same steps saved at n - snap_base; no injection, receivers sample du_{n+1}.
+// The first launch may be chained to the background sweep: before its dependency wait a Born step reads only du_{n-1} and
+// m, which that sweep does not write.
+static int run_born(fwi_fd2d* p, int n0, int n1, size_t snap_base, State& s, float* traces, cudaStream_t st) {
+    const size_t pl = p->plane();
+    for (int n = n0; n < n1; ++n) {
+        int rc = launch_step(p, STEP_BORN, s.c, p->fld[s.o], nullptr, nullptr, &p->rec, traces + (size_t)n * p->nrec,
+                             p->snap + (size_t)(n - snap_base) * pl, st);
+        if (rc) return rc;
+        s = State{s.o, s.c};
+    }
+    FWI_CUDA(cudaGetLastError());
+    return FWI_OK;
+}
+
 // ---- peer-memory slabs: what may be overwritten when ---------------------------------------------------------------
 // A neighbour stores its boundary planes of launch k into THIS GPU's ghost planes of the buffer launch k writes.  Before a
 // run (or a checkpointed segment) rewrites wavefields, a one-thread kernel waits until the neighbours have pushed
@@ -802,30 +840,51 @@ static int record_forward(fwi_fd2d* p, int nt, cudaStream_t st) {
     return run_forward(p, p->wav, 0, nt, p->nrec ? p->syn : nullptr, false, 0, s, st);
 }
 
+// Born modelling of one shot: per segment of S steps the background forward saves its S snapshots (traces -> p->syn)
+// and the scattered sweep over the same steps consumes them (traces -> p->resid).  Both states carry over from one
+// segment to the next, so no checkpoints are needed and S changes no result.
+static int record_born(fwi_fd2d* p, int nt, int S, cudaStream_t st) {
+    int rc = zero_state(p, 0, 1, st);
+    if (rc || (rc = zero_state(p, 4, 5, st))) return rc;
+    State fs{0, 1}, bs{4, 5};
+    for (int n0 = 0; n0 < nt; n0 += S) {
+        const int n1 = std::min(nt, n0 + S);
+        if ((rc = run_forward(p, p->wav, n0, n1, p->syn, true, n0, fs, st))) return rc;
+        if ((rc = run_born(p, n0, n1, n0, bs, p->resid, st))) return rc;
+    }
+    return FWI_OK;
+}
+
 // The gradient of one shot as a sequence of stream operations on `st`: forward (+ snapshots or checkpoints),
 // residual, adjoint with imaging.  Reads p->wav / p->obs, leaves synthetics in p->syn, I in p->acc, J in p->d_J.
-static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t st) {
+// gauss_newton: every forward segment (or the single full forward) saves its snapshots and is followed by the Born
+// sweep over it, which writes J dv into p->resid in place of the residual; the adjoint then images J^T J dv.
+static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t st, bool gauss_newton = false) {
     const size_t pl = p->plane();
     const size_t ntr = (size_t)nt * p->nrec;
     int rc = zero_state(p, 0, 1, st);
     if (rc) return rc;
-    State fs{0, 1};
+    State fs{0, 1}, bs{4, 5};
     std::vector<State> seg_state(nseg, fs);
+    if (gauss_newton && (rc = zero_state(p, 4, 5, st))) return rc;
     if (nseg == 1) {
         rc = run_forward(p, p->wav, 0, nt, p->nrec ? p->syn : nullptr, true, 0, fs, st);
         if (rc) return rc;
+        if (gauss_newton && (rc = run_born(p, 0, nt, 0, bs, p->resid, st))) return rc;
     } else {
         for (int s = 0; s < nseg; ++s) {
             if ((rc = slab_fence(p, st))) return rc;       // the ghost planes of u_n must have arrived before they are saved
             FWI_CUDA(cudaMemcpyAsync(p->ckpt + (size_t)(2 * s) * pl, p->fld[fs.c], pl * sizeof(float), cudaMemcpyDeviceToDevice, st));
             FWI_CUDA(cudaMemcpyAsync(p->ckpt + (size_t)(2 * s + 1) * pl, p->fld[fs.o], pl * sizeof(float), cudaMemcpyDeviceToDevice, st));
             seg_state[s] = fs;
-            rc = run_forward(p, p->wav, s * seg, std::min(nt, (s + 1) * seg), p->nrec ? p->syn : nullptr, false, 0, fs, st);
+            const int n0 = s * seg, n1 = std::min(nt, (s + 1) * seg);
+            rc = run_forward(p, p->wav, n0, n1, p->nrec ? p->syn : nullptr, gauss_newton, n0, fs, st);
             if (rc) return rc;
+            if (gauss_newton && (rc = run_born(p, n0, n1, n0, bs, p->resid, st))) return rc;
         }
     }
     FWI_CUDA(cudaMemsetAsync(p->d_J, 0, sizeof(double), st));
-    if (ntr) {
+    if (ntr && !gauss_newton) {
         fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntr + 255) / 256), 256, 0, st>>>(p->syn, p->obs, (int64_t)ntr, p->resid, p->d_J);
         FWI_CUDA(cudaGetLastError());
         p->launches += 1;
@@ -1039,6 +1098,7 @@ int fwi_fd2d_destroy(fwi_fd2d* p) {
     if (p->syn) cudaFree(p->syn);
     if (p->obs) cudaFree(p->obs);
     if (p->wav) cudaFree(p->wav);
+    if (p->dm) cudaFree(p->dm);
     p->src.release(); p->rec.release();
     p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
     for (int s = 0; s < 2; ++s) if (p->peer_arena[s] && p->peer_ipc[s]) cudaIpcCloseMemHandle(p->peer_arena[s]);
@@ -1259,6 +1319,101 @@ int fwi_fd2d_gradient(fwi_fd2d* p, const float* wavelet_dev, const float* obs_de
     if ((rc = leave(p, user))) return rc;
     if (misfit_host) FWI_CUDA(cudaStreamSynchronize(p->work));
     return FWI_OK;
+}
+
+// ---- Born modelling and Gauss-Newton Hessian-vector products (spec B5) ------------------------------------------
+// Steps per Born segment: the background sweep saves this many snapshots, then the scattered sweep reads them back.
+// (profiles/r3_born_bench.txt, ms per Born shot at 1000 x 3000, nt = 5000: see DESIGN.md)
+constexpr int kBornSeg = 128;
+
+static int check_linearised(fwi_fd2d* p, const char* fn, const float* wavelet_dev, const float* dv_dev, const float* out_dev, int nt) {
+    FWI_REQUIRE(p && p->model_set, "%s: set the model first", fn);
+    FWI_REQUIRE(wavelet_dev && dv_dev && out_dev && nt >= 1, "%s: NULL argument or nt < 1", fn);
+    FWI_REQUIRE(p->nsrc >= 1 && p->nrec >= 1, "%s: geometry needs at least one source and one receiver", fn);
+    // the slab step-id protocol assumes the same launch sequence on every rank
+    FWI_REQUIRE(!p->peers(), "%s: not available on a plan connected as a peer-memory slab", fn);
+    return FWI_OK;
+}
+
+// dm = (2 m / v) dv into the plan-owned pitched buffer, on the work stream ahead of the time loop (captured graphs keep
+// the buffer's address)
+static int stage_dm(fwi_fd2d* p, const float* dv_dev) {
+    dim3 grid(p->rows(), (p->px + 127) / 128);
+    fd_dm_kernel<<<grid, 128, 0, p->work>>>(dv_dev, p->m, p->vp, p->rows(), p->nx, p->px, p->dm);
+    FWI_CUDA(cudaGetLastError());
+    return FWI_OK;
+}
+
+// Segment length S of a Born run and its buffers: S = min(nt, kBornSeg, snapshot planes the memory limit / free memory
+// allows).  Free memory is only queried when the snapshot buffer cannot already hold min(nt, kBornSeg) planes.
+static int prepare_born(fwi_fd2d* p, int nt, int& S) {
+    const size_t pl = p->plane();
+    S = std::min(nt, kBornSeg);
+    size_t max_planes = 0;
+    if (p->mem_limit) max_planes = p->mem_limit / (pl * sizeof(float));
+    else if (p->snap_steps >= (size_t)S * pl) max_planes = (size_t)S;
+    else {
+        size_t fr = 0, tot = 0;
+        FWI_CUDA(cudaMemGetInfo(&fr, &tot));
+        max_planes = (size_t)((fr + p->snap_steps * sizeof(float)) * 0.85) / (pl * sizeof(float));
+    }
+    FWI_REQUIRE(max_planes >= 1, "fwi_fd2d_born: the memory limit holds no snapshot plane of %zu bytes", pl * sizeof(float));
+    S = (int)std::min<size_t>((size_t)S, max_planes);
+    const size_t ntr = (size_t)nt * p->nrec;
+    int rc;
+    if ((rc = ensure_floats(p, &p->snap, &p->snap_steps, (size_t)S * pl))) return rc;
+    if ((rc = ensure_floats(p, &p->resid, &p->resid_cap, ntr))) return rc;
+    if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, ntr))) return rc;
+    if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
+    return ensure_floats(p, &p->dm, &p->dm_cap, pl);
+}
+
+int fwi_fd2d_born(fwi_fd2d* p, const float* wavelet_dev, const float* dv_dev, int nt, float* dtraces_dev, float* traces_dev,
+                  void* stream) {
+    int rc = check_linearised(p, "fwi_fd2d_born", wavelet_dev, dv_dev, dtraces_dev, nt);
+    if (rc) return rc;
+    DeviceGuard g(p->device);
+    cudaStream_t user = (cudaStream_t)stream;
+    int S = 1;
+    if ((rc = prepare_born(p, nt, S))) return rc;
+    const size_t ntr = (size_t)nt * p->nrec;
+    if ((rc = enter(p, user))) return rc;
+    FWI_CUDA(cudaMemcpyAsync(p->wav, wavelet_dev, (size_t)nt * p->nsrc * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if ((rc = stage_dm(p, dv_dev))) return rc;
+    rc = run_cached(p, 2, nt, S, 0, [&](cudaStream_t st) { return record_born(p, nt, S, st); });
+    if (rc) return rc;
+    FWI_CUDA(cudaMemcpyAsync(dtraces_dev, p->resid, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (traces_dev) FWI_CUDA(cudaMemcpyAsync(traces_dev, p->syn, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    {   // the background ran in segments: a tb2 plan pairs its steps per segment
+        State fs{0, 1};
+        for (int n0 = 0; n0 < nt; n0 += S) fs = advance_state(p, fs, 0, std::min(nt, n0 + S) - n0);
+        p->fwd_c = fs.c; p->fwd_o = fs.o;
+    }
+    return leave(p, user);
+}
+
+int fwi_fd2d_gauss_newton(fwi_fd2d* p, const float* wavelet_dev, const float* dv_dev, int nt, float* hv_dev, float* dtraces_dev,
+                          void* stream) {
+    int rc = check_linearised(p, "fwi_fd2d_gauss_newton", wavelet_dev, dv_dev, hv_dev, nt);
+    if (rc) return rc;
+    DeviceGuard g(p->device);
+    cudaStream_t user = (cudaStream_t)stream;
+    int seg = nt, nseg = 1;
+    if ((rc = prepare_gradient(p, nt, seg, nseg))) return rc;
+    if ((rc = ensure_floats(p, &p->dm, &p->dm_cap, p->plane()))) return rc;
+    const size_t ntr = (size_t)nt * p->nrec;
+    if ((rc = enter(p, user))) return rc;
+    FWI_CUDA(cudaMemcpyAsync(p->wav, wavelet_dev, (size_t)nt * p->nsrc * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if ((rc = stage_dm(p, dv_dev))) return rc;
+    rc = run_cached(p, 3, nt, seg, nseg, [&](cudaStream_t st) { return record_gradient(p, nt, seg, nseg, st, true); });
+    if (rc) return rc;
+    { State fs = advance_state(p, State{0, 1}, 0, nt); p->fwd_c = fs.c; p->fwd_o = fs.o; }
+    dim3 grid(p->rows(), (p->nx + 127) / 128);
+    fd_grad_finalize_kernel<<<grid, 128, 0, p->work>>>(p->acc, p->vp, p->rows(), p->nx, p->px, hv_dev);   // H dv = (2 / v) I
+    FWI_CUDA(cudaGetLastError());
+    p->launches += 1;
+    if (dtraces_dev) FWI_CUDA(cudaMemcpyAsync(dtraces_dev, p->resid, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    return leave(p, user);
 }
 
 int64_t fwi_fd2d_launch_count(fwi_fd2d* p) { return p ? p->launches : 0; }

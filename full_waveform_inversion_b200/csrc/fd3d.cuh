@@ -12,7 +12,8 @@
 //     come from the centre plane, which is still in the ring four planes behind the newest one;
 //   * u_{n+1} overwrites u_{n-1} in place (plain per-warp global loads of u_{n-1} / m instead of the second ring cost
 //     40 % of the step); snapshot write / snapshot read + imaging are fused exactly as in 2-D; the CTA applies its own
-//     source / receiver points at the end.
+//     source / receiver points at the end; the Born step reads w_n and dm from global memory beside the adjoint's
+//     operands (not through the u_{n-1} / m ring) and adds dm * w_n inside the update.
 // Algorithmic traffic: 16 B per point update (+ halo re-reads that hit L2).
 #pragma once
 #include "fd_common.cuh"
@@ -61,6 +62,7 @@ struct Step3DArgs {
     int* flag_peer_up;         // where I announce "boundary planes of launch k pushed" to the upper / lower neighbour
     int* flag_peer_dn;
     long long timeout_cycles;  // bounded spin on a neighbour's flag
+    const float* dm;           // BORN: model perturbation dm = (2 m / v) dv, pitched like m
 };
 
 // sync words of one plan (ints inside its arena; the neighbours write [0] / [1] through their peer mapping)
@@ -230,7 +232,7 @@ __global__ void __launch_bounds__(T3<BY>::Threads, 1) fd3d_step_kernel(const __g
             const int z = zbeg + zstep * iz;
             const int ptop = iz + 2 * kHalo, pmid = iz + kHalo;
             // global operands first: their latency overlaps the barrier wait and the shared-memory reads
-            float4 o4[k3RPW], m4[k3RPW], s4[k3RPW], c4[k3RPW], sp4[k3RPW];
+            float4 o4[k3RPW], m4[k3RPW], s4[k3RPW], c4[k3RPW], sp4[k3RPW], d4[k3RPW];
             size_t off[k3RPW];
             bool ok[k3RPW];
 #pragma unroll
@@ -241,6 +243,7 @@ __global__ void __launch_bounds__(T3<BY>::Threads, 1) fd3d_step_kernel(const __g
                 if (ok[r]) {
                     if (MODE == STEP_ADJ || MODE == STEP_ADJ2) { s4[r] = ld4_stream(a.snap + off[r]); c4[r] = ld4(a.acc + off[r]); }
                     if (MODE == STEP_ADJ2) sp4[r] = ld4_stream(a.snap_prev + off[r]);
+                    if (MODE == STEP_BORN) { s4[r] = ld4_stream(a.snap + off[r]); d4[r] = ld4(a.dm + off[r]); }
                 }
             }
             const float gzv = __ldg(a.gz + z);
@@ -283,7 +286,10 @@ __global__ void __launch_bounds__(T3<BY>::Threads, 1) fd3d_step_kernel(const __g
                     lap = fmaf(kC3, ((ax[1 + q] + ax[7 + q]) + (comp(yc[r + 1]) + comp(yc[r + 7]))) + (comp(win[r][1]) + comp(win[r][7])), lap);
                     lap = fmaf(kC4, ((ax[0 + q] + ax[8 + q]) + (comp(yc[r + 0]) + comp(yc[r + 8]))) + (comp(win[r][0]) + comp(win[r][8])), lap);
                     wv[q] = lap;
-                    nv[q] = gv[q] * fmaf(mv[q], lap, fmaf(-gv[q], ov[q], 2.0f * c));
+                    // BORN: nv = g * fma(m, lap, fma(dm, w, fma(-g, o, 2 c))), the same order as the 2-D kernel
+                    float rest = fmaf(-gv[q], ov[q], 2.0f * c);
+                    if (MODE == STEP_BORN) rest = fmaf(comp(d4[r]), comp(s4[r]), rest);
+                    nv[q] = gv[q] * fmaf(mv[q], lap, rest);
                 }
                 if (ok[r]) {
                     const float4 n4 = make_float4(nv[0], nv[1], nv[2], nv[3]);

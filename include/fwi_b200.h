@@ -173,7 +173,9 @@ int fwi_fd2d_set_tb2(fwi_fd2d* plan, int cz);
 /* Replay the time loops as cached CUDA graphs (default on) or as individual launches (0). */
 int fwi_fd2d_set_graphs(fwi_fd2d* plan, int enable);
 /* Cap (bytes) on the forward-field storage used by fwi_fd2d_gradient; 0 = 85 % of free HBM.  When all nt
- * snapshots do not fit, the gradient switches to two-level checkpointing (recompute per segment). */
+ * snapshots do not fit, the gradient switches to two-level checkpointing (recompute per segment).
+ * fwi_fd2d_gauss_newton follows the same rule; fwi_fd2d_born keeps at most min(nt, 128) snapshots and takes fewer
+ * when the cap holds fewer planes (same results); a cap below one plane is FWI_EINVAL. */
 int fwi_fd2d_set_memory_limit(fwi_fd2d* plan, uint64_t bytes);
 /* v_dev: (nz, nx) fp32 velocities, dense.  Builds m = (v dt / h)^2 in the pitched layout (fd_oracle B1). */
 int fwi_fd2d_set_model(fwi_fd2d* plan, const float* v_dev, void* stream);
@@ -193,6 +195,15 @@ int fwi_fd2d_wavefield(fwi_fd2d* plan, int which, float* out_dev, void* stream);
  * (requesting it synchronises the stream). */
 int fwi_fd2d_gradient(fwi_fd2d* plan, const float* wavelet_dev, const float* obs_dev, int nt, float* grad_dev,
                       float* traces_dev, double* misfit_host, void* stream);
+/* Born (linearised) modelling: dtraces_dev (nt, nrec) = J dv for the velocity perturbation dv_dev (dense, grid-shaped);
+ * traces_dev (nullable) receives the background synthetics, bit-identical to fwi_fd2d_forward.  (spec B5, tests/born_reference.py) */
+int fwi_fd2d_born(fwi_fd2d* plan, const float* wavelet_dev, const float* dv_dev, int nt, float* dtraces_dev,
+                  float* traces_dev, void* stream);
+/* Gauss-Newton Hessian-vector product: hv_dev (grid-shaped) += J^T J dv; dtraces_dev (nullable) receives J dv.
+ * Same snapshot storage / checkpointing rule as fwi_fd2d_gradient.  (spec B5, tests/born_reference.py)
+ * Both return FWI_EINVAL on a plan connected as a peer-memory slab. */
+int fwi_fd2d_gauss_newton(fwi_fd2d* plan, const float* wavelet_dev, const float* dv_dev, int nt, float* hv_dev,
+                          float* dtraces_dev, void* stream);
 int64_t fwi_fd2d_launch_count(fwi_fd2d* plan);
 /* Allocate what fwi_fd2d_forward (gradient = 0) or fwi_fd2d_gradient (1) over nt steps will need with the current
  * geometry, without launching anything (allocations synchronise the device: keep them out of timed regions). */
