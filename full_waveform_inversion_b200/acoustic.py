@@ -10,6 +10,8 @@ over shots.
 Conventions: velocity grids are (nz, nx) [2-D] or (nz, ny, nx) [3-D] float32, x contiguous;
 a shot is ``(src, rec)`` with integer index arrays of shape (n, ndim) in (z[, y], x) order;
 wavelets are (nt,) or (nt, nsrc); traces are (nt, nrec), time-major; a velocity perturbation dv is grid-shaped.
+`free_surface=True` makes grid row (plane) z = 0 a pressure-free surface (spec B6, tests/free_surface_reference.py):
+the field is mirrored oddly above it, the sponge leaves that face undamped, and sources and receivers need z >= 1.
 """
 from __future__ import annotations
 
@@ -29,6 +31,7 @@ _lib.register({
     "fwi_fd2d_set_tile": (c_int, [c_void_p, c_int, c_int]),
     "fwi_fd2d_set_graphs": (c_int, [c_void_p, c_int]),
     "fwi_fd2d_set_tb2": (c_int, [c_void_p, c_int]),
+    "fwi_fd2d_set_free_surface": (c_int, [c_void_p, c_int]),
     "fwi_fd2d_set_memory_limit": (c_int, [c_void_p, c_uint64]),
     "fwi_fd2d_set_model": (c_int, [c_void_p, c_void_p, c_void_p]),
     "fwi_fd2d_set_geometry": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
@@ -88,9 +91,10 @@ def _points(pts, ndim):
 
 class Propagator:
     """One GPU's propagator plan (wraps ``fwi_fd2d``; 2-D or 3-D by the length of `shape`): model, sponge,
-    wavefields, TMA descriptors, cached CUDA graphs."""
+    wavefields, TMA descriptors, cached CUDA graphs.  `free_surface`: z = 0 is a free surface (spec B6)."""
 
-    def __init__(self, shape, h, dt, nabs=20, alpha=0.3, device=None, tile=None, memory_limit=0, graphs=True, tb2=None):
+    def __init__(self, shape, h, dt, nabs=20, alpha=0.3, device=None, tile=None, memory_limit=0, graphs=True, tb2=None,
+                 free_surface=False):
         self._lib = _lib.require_gpu()
         self.shape = tuple(int(n) for n in shape)
         self.ndim = len(self.shape)
@@ -114,6 +118,9 @@ class Propagator:
             check(self._lib.fwi_fd2d_set_memory_limit(self._h, int(memory_limit)))
         if not graphs:
             check(self._lib.fwi_fd2d_set_graphs(self._h, 0))
+        self.free_surface = bool(free_surface)
+        if self.free_surface:
+            check(self._lib.fwi_fd2d_set_free_surface(self._h, 1))
         self.nsrc = self.nrec = 0
 
     @property
@@ -275,12 +282,13 @@ def _make_propagator(shape, h, dt, nabs, alpha, device, **kw):
     return Propagator(shape, h, dt, nabs, alpha, device, **kw)
 
 
-def sponge_profile(n, nabs, alpha):
-    """1-D Cerjan profile (fd_oracle.sponge_profile)."""
+def sponge_profile(n, nabs, alpha, free_surface=False):
+    """1-D Cerjan profile (fd_oracle.sponge_profile); `free_surface` leaves index 0's face undamped (spec B6)."""
     prof = np.ones(n, dtype=np.float64)
     for i in range(min(nabs, n)):
         val = math.exp(-((alpha * (nabs - i) / nabs) ** 2))
-        prof[i] = min(prof[i], val)
+        if not free_surface:
+            prof[i] = min(prof[i], val)
         prof[n - 1 - i] = min(prof[n - 1 - i], val)
     return prof.astype(np.float32)
 
@@ -297,11 +305,13 @@ class SlabPropagator:
     `forward` / `gradient` (same checkpointing when the snapshots do not fit, per rank); no collective per step.
     Fallback / 2-D (`p2p=False`): the ordinary step kernel runs on the local grid and the boundary planes are exchanged
     with NCCL send/recv, the loop captured as a CUDA graph (every w_n held in HBM).
-    Either way the owned planes are bit-identical to a single-GPU run."""
+    Either way the owned planes are bit-identical to a single-GPU run.  With `free_surface`, global z = 0 is a free
+    surface (spec B6): every rank slices the global profile, and only rank 0's plan mirrors the field above z = 0."""
 
     HALO = 4
 
-    def __init__(self, shape, h, dt, nabs=20, alpha=0.3, device=None, use_graphs=True, p2p=None, memory_limit=0):
+    def __init__(self, shape, h, dt, nabs=20, alpha=0.3, device=None, use_graphs=True, p2p=None, memory_limit=0,
+                 free_surface=False):
         import torch.distributed as dist
         if not (dist.is_available() and dist.is_initialized()):
             raise RuntimeError("SlabPropagator needs an initialised torch.distributed process group")
@@ -323,8 +333,8 @@ class SlabPropagator:
         # itself); p2p=False forces the NCCL send/recv exchange, which is also the fallback if IPC mapping fails.
         self.p2p = (p2p is None or bool(p2p)) and len(self.shape) == 3 and self.world > 1
         self.prop = Propagator(self.local_shape, h, dt, nabs, alpha, device, graphs=bool(use_graphs and self.p2p),
-                               memory_limit=memory_limit)
-        gz = sponge_profile(nz, nabs, alpha)[self.z0 - self.up: self.z0 + self.n_own + self.down]
+                               memory_limit=memory_limit, free_surface=bool(free_surface) and self.rank == 0)
+        gz = sponge_profile(nz, nabs, alpha, free_surface)[self.z0 - self.up: self.z0 + self.n_own + self.down]
         self.prop.set_profiles(gz=gz)
         self.fields = [self.prop.field_view(i) for i in range(8)]
         self.nsrc = self.nrec = 0
@@ -563,10 +573,10 @@ def shard_shots(n_shots, world, rank):
     return list(range(rank, n_shots, world))
 
 
-def forward_model(v, h, dt, shots, wavelet, nabs=20, alpha=0.3, device=None, propagator=None):
+def forward_model(v, h, dt, shots, wavelet, nabs=20, alpha=0.3, device=None, propagator=None, free_surface=False):
     """Forward model every shot -> list of (nt, nrec) device tensors (fd_oracle.Problem.forward per shot)."""
     device = torch.cuda.current_device() if device is None else device
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
     try:
         prop.set_model(v)
         out = []
@@ -579,10 +589,10 @@ def forward_model(v, h, dt, shots, wavelet, nabs=20, alpha=0.3, device=None, pro
             prop.close()
 
 
-def born_model(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None):
+def born_model(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None, free_surface=False):
     """Born traces J dv of every shot -> list of (nt, nrec) device tensors (spec B5 per shot, tests/born_reference.py)."""
     device = torch.cuda.current_device() if device is None else device
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
     try:
         prop.set_model(v)
         out = []
@@ -596,7 +606,7 @@ def born_model(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, pr
 
 
 def gauss_newton_product(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None, allreduce=True,
-                         shot_ids=None):
+                         shot_ids=None, free_surface=False):
     """Gauss-Newton Hessian-vector product summed over shots, sum_s J_s^T J_s dv -> grid-shaped device tensor.
 
     Under torch.distributed the shots are sharded round-robin over the ranks and the product is summed with ONE
@@ -608,7 +618,7 @@ def gauss_newton_product(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, devic
         mine = [shots[i] for i in ids]
     else:
         mine = list(shots)
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
     try:
         prop.set_model(v)
         hv = torch.zeros(tuple(v.shape), dtype=torch.float32, device=prop.torch_device)
@@ -641,7 +651,7 @@ def misfit(traces, observed):
 
 
 def gradient(v, h, dt, shots, wavelet, observed, nabs=20, alpha=0.3, device=None, propagator=None, allreduce=True,
-             shot_ids=None):
+             shot_ids=None, free_surface=False):
     """Misfit and dJ/dv summed over shots -> (J, grad (grid-shaped device tensor)).
 
     Under torch.distributed the shots are sharded round-robin over the ranks (one GPU each) and the gradient and
@@ -655,7 +665,7 @@ def gradient(v, h, dt, shots, wavelet, observed, nabs=20, alpha=0.3, device=None
         mine = [(shots[i], observed[i]) for i in ids]
     else:
         mine = list(zip(shots, observed))
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
     try:
         prop.set_model(v)
         grad = torch.zeros(tuple(v.shape), dtype=torch.float32, device=prop.torch_device)
@@ -695,7 +705,7 @@ def absmax(x):
 
 
 def fwi(v0, h, dt, shots, wavelet, observed, niter, vmin, vmax, step_frac=0.02, max_backtrack=4, nabs=20, alpha=0.3,
-        device=None, callback=None):
+        device=None, callback=None, free_surface=False):
     """Steepest-descent full-waveform inversion (fd_oracle.fwi, B4) -> (v, misfit history).
 
     Each iteration: gradient over all shots (sharded + all-reduced when distributed), step = step_frac * max|v| /
@@ -704,7 +714,7 @@ def fwi(v0, h, dt, shots, wavelet, observed, niter, vmin, vmax, step_frac=0.02, 
     dev = torch.device("cuda", device)
     v = _dev_f32(v0, dev).clone()
     dist = _dist()
-    prop = _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device)
+    prop = _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
     ids = shard_shots(len(shots), dist.get_world_size(), dist.get_rank()) if dist else list(range(len(shots)))
     my_shots = [shots[i] for i in ids]
     my_obs = [_dev_f32(observed[i], dev) for i in ids]

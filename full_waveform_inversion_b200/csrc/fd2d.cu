@@ -15,6 +15,8 @@
 // The forward pass can stream w_n to an HBM snapshot (evict-first stores); the adjoint pass reads it
 // back and accumulates the zero-lag cross-correlation in the same kernel.  The Born (linearised) step reads it back as the
 // source term of the scattered field: du_{n+1} = g (2 du_n - g du_{n-1} + m lap(du_n) + dm w_n)  (spec B5).
+// A plan may make row z = 0 a free surface (spec B6, fwi_fd2d_set_free_surface): every step kernel has an FS instance in which
+// the CTAs at z = 0 replace the zero halo above the grid by the odd mirror u[-k] = -u[k]; all other CTAs run unchanged code.
 #include "fd_common.cuh"
 #include <vector>
 #include <algorithm>
@@ -55,7 +57,9 @@ constexpr int kPrefetchRows = 2;
 // store phases and costs L2 bandwidth (ms per 5000-step gradient: no PDL 85.5, implicit 84.5, after the dense part 88.6,
 // at the top 101).
 // No minimum-blocks bound: ptxas settles at 80 registers (3 CTAs of 256 threads per SM); with an explicit minimum of 1 it takes 110.
-template <int BZ, int NW, int MODE>
+// FS: free surface at z = 0 (spec B6, tests/free_surface_reference.py): the top row of CTAs replaces the zero-filled rows
+// above the grid by the odd mirror u[-k] = -u[k] before computing; every other CTA runs the FS = false code.
+template <int BZ, int NW, int MODE, bool FS>
 __global__ void __launch_bounds__(NW * 32) fd2d_step_kernel(const __grid_constant__ CUtensorMap tm_cur, Step2DArgs a) {
     constexpr int BX = 128, SX = BX + 2 * kHalo, SZ = BZ + 2 * kHalo, RPW = BZ / NW;
     static_assert(BZ % NW == 0, "rows must split evenly over warps");
@@ -99,6 +103,10 @@ __global__ void __launch_bounds__(NW * 32) fd2d_step_kernel(const __grid_constan
     __syncthreads();        // barrier init visible to every waiter
 
     mbar_wait(&bar, 0);
+    if (FS && tz0 == 0) {           // uniform per CTA
+        mirror_rows(tile, SX, kHalo, SX);       // tile row kHalo is z = 0; the x halo columns are mirrored too
+        __syncthreads();
+    }
 
     if (col_ok && zw < a.nz) {
         // register window over z: win[k] holds row (z - 4 + k) of this lane's float4 column
@@ -312,12 +320,12 @@ struct PointList {
 enum Family { kTile, kTb2, k3D };
 
 // One built shape of a family: tile rows (bz / cz / by), warps per CTA, dynamic shared memory per CTA, and its kernel for
-// each mode, indexed by STEP_FWD .. STEP_BORN (null where the family has no such mode).  The tables below are the only
-// list of the shapes the library builds.
+// each free-surface setting (0 off, 1 on: spec B6) and mode, indexed by STEP_FWD .. STEP_BORN (null where the family has no
+// such mode).  The tables below are the only list of the shapes the library builds.
 template <typename Kernel> struct StepShape {
     int rows, warps;
     size_t smem;
-    Kernel fn[5];
+    Kernel fn[2][5];
 };
 using TileShape = StepShape<void (*)(CUtensorMap, Step2DArgs)>;
 using Tb2Shape = StepShape<void (*)(CUtensorMap, CUtensorMap, CUtensorMap, Tb2Args)>;
@@ -326,19 +334,29 @@ using Fd3Shape = StepShape<void (*)(CUtensorMap, CUtensorMap, CUtensorMap, Step3
 constexpr int kBX = 128;
 template <int BZ, int NW> TileShape tile_shape() {
     return {BZ, NW, (size_t)(kBX + 2 * kHalo) * (BZ + 2 * kHalo) * sizeof(float),
-            {fd2d_step_kernel<BZ, NW, STEP_FWD>, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE>, fd2d_step_kernel<BZ, NW, STEP_ADJ>,
-             fd2d_step_kernel<BZ, NW, STEP_ADJ2>, fd2d_step_kernel<BZ, NW, STEP_BORN>}};
+            {{fd2d_step_kernel<BZ, NW, STEP_FWD, false>, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE, false>,
+              fd2d_step_kernel<BZ, NW, STEP_ADJ, false>, fd2d_step_kernel<BZ, NW, STEP_ADJ2, false>,
+              fd2d_step_kernel<BZ, NW, STEP_BORN, false>},
+             {fd2d_step_kernel<BZ, NW, STEP_FWD, true>, fd2d_step_kernel<BZ, NW, STEP_FWD_SAVE, true>,
+              fd2d_step_kernel<BZ, NW, STEP_ADJ, true>, fd2d_step_kernel<BZ, NW, STEP_ADJ2, true>,
+              fd2d_step_kernel<BZ, NW, STEP_BORN, true>}}};
 }
 constexpr int kTb2Warps = 8;          // (4 warps at 24 rows measured 8 % slower)
 template <int CZ> Tb2Shape tb2_shape() {
     return {CZ, kTb2Warps, ((size_t)(CZ + 16) * kT2W0 + 2 * (size_t)(CZ + 8) * kT2W1) * sizeof(float),
-            {fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD>, fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD_SAVE>,
-             fd2d_tb2_kernel<CZ, kTb2Warps, STEP_ADJ>, nullptr, nullptr}};
+            {{fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD, false>, fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD_SAVE, false>,
+              fd2d_tb2_kernel<CZ, kTb2Warps, STEP_ADJ, false>, nullptr, nullptr},
+             {fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD, true>, fd2d_tb2_kernel<CZ, kTb2Warps, STEP_FWD_SAVE, true>,
+              fd2d_tb2_kernel<CZ, kTb2Warps, STEP_ADJ, true>, nullptr, nullptr}}};
 }
 template <int BY> Fd3Shape fd3_shape() {
     return {BY, T3<BY>::Threads / 32, T3<BY>::Smem,
-            {fd3d_step_kernel<STEP_FWD, BY>, fd3d_step_kernel<STEP_FWD_SAVE, BY>, fd3d_step_kernel<STEP_ADJ, BY>,
-             fd3d_step_kernel<STEP_ADJ2, BY>, fd3d_step_kernel<STEP_BORN, BY>}};
+            {{fd3d_step_kernel<STEP_FWD, BY, false>, fd3d_step_kernel<STEP_FWD_SAVE, BY, false>,
+              fd3d_step_kernel<STEP_ADJ, BY, false>, fd3d_step_kernel<STEP_ADJ2, BY, false>,
+              fd3d_step_kernel<STEP_BORN, BY, false>},
+             {fd3d_step_kernel<STEP_FWD, BY, true>, fd3d_step_kernel<STEP_FWD_SAVE, BY, true>,
+              fd3d_step_kernel<STEP_ADJ, BY, true>, fd3d_step_kernel<STEP_ADJ2, BY, true>,
+              fd3d_step_kernel<STEP_BORN, BY, true>}}};
 }
 // The one-step kernel is built for exactly these (rows, warps per CTA): the round-1 sweep's winner and three heights of 7 rows
 // per warp among which one has tiles that fill whole waves.  pick_tile() breaks ties by this order.
@@ -408,6 +426,7 @@ struct fwi_fd2d {
     int split_nt = -1, split_seg = 0, split_nseg = 0; size_t split_limit = 0;   // cached storage decision of the last gradient
     int fwd_c = 0, fwd_o = 1;         // fld[] indices of u_n and u_{n-1} after the last forward
     bool model_set = false;
+    bool free_surface = false;        // spec B6: odd mirror above z = 0, no sponge on the top face (fwi_fd2d_set_free_surface)
     bool use_graphs = true;
     bool defer_imaging = true;        // tile and 3-D kernels: image two adjoint steps per accumulator update
     int64_t launches = 0;
@@ -422,6 +441,19 @@ struct fwi_fd2d {
     int rows() const { return nz * ny; }
     size_t plane() const { return (size_t)nz * ny * px; }
 };
+
+// Sponge profile (oracle/fd_oracle.py sponge_profile), float64 on the host then rounded once, padded with 1.  `free_top`
+// drops the strip at index 0: a free surface is not damped (spec B6).
+static std::vector<float> sponge_profile(int n, int padded, int nabs, float alpha, bool free_top) {
+    std::vector<float> prof(padded, 1.0f);
+    for (int i = 0; i < std::min(nabs, n); ++i) {
+        const double t = (double)alpha * (nabs - i) / nabs;
+        const float val = (float)std::exp(-t * t);
+        if (!free_top) prof[i] = std::min(prof[i], val);
+        prof[n - 1 - i] = std::min(prof[n - 1 - i], val);
+    }
+    return prof;
+}
 
 static void drop_graphs(fwi_fd2d* p) {
     for (auto& g : p->graphs) cudaGraphExecDestroy(g.exec);
@@ -463,7 +495,7 @@ static int make_tmaps3(fwi_fd2d* p) {
         p->tiles_y = (p->ny + p->fd3->rows - 1) / p->fd3->rows;
         p->zchunk = (nzo + best - 1) / best;
         p->nzch = (nzo + p->zchunk - 1) / p->zchunk;
-        p->last_desc = (p->peer_arena[1] && p->nzch >= 2) ? 1 : 0;
+        p->last_desc = (p->peer_arena[1] && p->nzch >= 2) ? 1 : 0;   // (never the chunk at z = 0, see fd3d_step_kernel FS)
     }
     for (int i = 0; i < 8; ++i) {
         const uint64_t dims[3] = {(uint64_t)p->nx, (uint64_t)p->ny, (uint64_t)p->nz};
@@ -571,6 +603,8 @@ static int build_point_list(fwi_fd2d* p, PointList& pl, const TileGrid& g, int r
         FWI_REQUIRE(iz[i] >= 0 && iz[i] < p->nz && ix[i] >= 0 && ix[i] < p->nx && yy >= 0 && yy < p->ny, "%s %d at (z=%d, y=%d, x=%d) is outside the %d x %d x %d grid", what, i, iz[i], yy, ix[i], p->nz, p->ny, p->nx);
         // a slab computes only its owned planes; the neighbours overwrite the ghost planes
         FWI_REQUIRE(iz[i] >= p->z_own0 && iz[i] < z_own1, "%s %d at z=%d is outside the planes [%d, %d) this slab owns", what, i, iz[i], p->z_own0, z_own1);
+        // the free surface holds p = 0: a point on it would inject into, or record, a row that stays 0
+        FWI_REQUIRE(!p->free_surface || iz[i] >= 1, "%s %d at (z=%d, y=%d, x=%d) lies on the free surface; sources and receivers need z >= 1", what, i, iz[i], yy, ix[i]);
         const int c[3] = {iz[i] - g.z0, yy, ix[i]};
         int lo[3], hi[3];
         for (int d = 0; d < 3; ++d) {
@@ -611,18 +645,19 @@ static int build_point_list(fwi_fd2d* p, PointList& pl, const TileGrid& g, int r
     return FWI_OK;
 }
 
-// Launches the kernel of `mode` of a step-kernel shape.  With `pdl` it is chained to the previous kernel on the stream by a
-// programmatic edge (also inside captured graphs) and orders itself behind its predecessor with griddepcontrol.wait.
+// Launches the kernel of `mode` of a step-kernel shape, its free-surface instance when `fs`.  With `pdl` it is chained to
+// the previous kernel on the stream by a programmatic edge (also inside captured graphs) and orders itself behind its
+// predecessor with griddepcontrol.wait.
 template <typename Kernel, typename... Args>
-static int launch_shape(const StepShape<Kernel>& k, int mode, dim3 grid, bool pdl, cudaStream_t st, const Args&... args) {
-    FWI_REQUIRE(k.fn[mode], "fd2d: the %d-row kernel has no step mode %d", k.rows, mode);
+static int launch_shape(const StepShape<Kernel>& k, int mode, bool fs, dim3 grid, bool pdl, cudaStream_t st, const Args&... args) {
+    FWI_REQUIRE(k.fn[fs][mode], "fd2d: the %d-row kernel has no step mode %d", k.rows, mode);
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = grid; cfg.blockDim = dim3(k.warps * 32); cfg.dynamicSmemBytes = k.smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = pdl ? 1 : 0;
-    FWI_CUDA(cudaLaunchKernelEx(&cfg, k.fn[mode], args...));
+    FWI_CUDA(cudaLaunchKernelEx(&cfg, k.fn[fs][mode], args...));
     return FWI_OK;
 }
 
@@ -640,7 +675,7 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
         a.dm = p->dm;
         const bool pdl = p->pdl && p->pdl_chain;
         p->pdl_chain = true;
-        return launch_shape(*p->tile, mode, dim3(p->tiles_x, p->tiles_z), pdl, st, p->tmap[cur], a);
+        return launch_shape(*p->tile, mode, p->free_surface, dim3(p->tiles_x, p->tiles_z), pdl, st, p->tmap[cur], a);
     }
     Step3DArgs a{};
     a.oldnew = oldnew; a.m = p->m; a.gx = p->gx; a.gy = p->gy; a.gz = p->gz; a.snap = snap; a.acc = p->acc; a.snap_prev = snap_prev;
@@ -663,7 +698,7 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
     a.timeout_cycles = p->slab_timeout_cycles;
     a.dm = p->dm;
     // (programmatic dependent launch was measured on this kernel too: 2 % at 128^3, nothing from 256^3 up - not used)
-    return launch_shape(*p->fd3, mode, dim3(p->tiles_x, p->tiles_y, p->nzch), false, st, p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);
+    return launch_shape(*p->fd3, mode, p->free_surface, dim3(p->tiles_x, p->tiles_y, p->nzch), false, st, p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);
 }
 
 static int ensure_floats(fwi_fd2d* p, float** ptr, size_t* cap, size_t need_floats) {
@@ -707,7 +742,7 @@ static int launch_tb2(fwi_fd2d* p, int mode, const State& s, int jc, int jd, con
     a.rec1 = rec1; a.rec2 = rec2;
     const bool pdl = p->pdl && p->pdl_chain;      // the pass loads m before its dependency wait
     p->pdl_chain = true;
-    return launch_shape(*p->tb2, mode, dim3(p->tiles_x2, p->tiles_z2), pdl, st, p->tb_cur[s.c], p->tb_old[s.o], p->tb_m, a);
+    return launch_shape(*p->tb2, mode, p->free_surface, dim3(p->tiles_x2, p->tiles_z2), pdl, st, p->tb_cur[s.c], p->tb_old[s.o], p->tb_m, a);
 }
 
 // forward time loop over steps [n0, n1); `s` holds the fld[] indices of (u_n, u_{n-1}) on entry and on return
@@ -959,8 +994,9 @@ static int leave(fwi_fd2d* p, cudaStream_t user) {       // ... and the caller's
 
 template <typename Shape, size_t N> static int allow_smem(const Shape (&table)[N]) {
     for (const auto& k : table)
-        for (auto fn : k.fn)
-            if (fn) FWI_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
+        for (const auto& row : k.fn)
+            for (auto fn : row)
+                if (fn) FWI_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
     return FWI_OK;
 }
 
@@ -1016,18 +1052,8 @@ static int init_plan(fwi_fd2d* p, int device, int nz, int ny, int nx, float h, f
     FWI_CUDA(cudaMalloc(&p->gz, nz * sizeof(float)));
     FWI_CUDA(cudaMalloc(&p->gy, ny * sizeof(float)));
     FWI_CUDA(cudaMalloc(&p->d_J, sizeof(double)));
-    // sponge profiles (oracle/fd_oracle.py sponge_profile), float64 on the host then rounded once
-    auto profile = [&](int n, int padded) {
-        std::vector<float> prof(padded, 1.0f);
-        for (int i = 0; i < std::min(nabs, n); ++i) {
-            const double t = (double)alpha * (nabs - i) / nabs;
-            const float val = (float)std::exp(-t * t);
-            prof[i] = std::min(prof[i], val);
-            prof[n - 1 - i] = std::min(prof[n - 1 - i], val);
-        }
-        return prof;
-    };
-    std::vector<float> gxh = profile(nx, p->px), gzh = profile(nz, nz), gyh = (ny > 1) ? profile(ny, ny) : std::vector<float>(1, 1.0f);
+    std::vector<float> gxh = sponge_profile(nx, p->px, nabs, alpha, false), gzh = sponge_profile(nz, nz, nabs, alpha, false),
+                       gyh = (ny > 1) ? sponge_profile(ny, ny, nabs, alpha, false) : std::vector<float>(1, 1.0f);
     FWI_CUDA(cudaMemcpy(p->gy, gyh.data(), ny * sizeof(float), cudaMemcpyHostToDevice));
     FWI_CUDA(cudaMemcpy(p->gx, gxh.data(), p->px * sizeof(float), cudaMemcpyHostToDevice));
     FWI_CUDA(cudaMemcpy(p->gz, gzh.data(), nz * sizeof(float), cudaMemcpyHostToDevice));
@@ -1137,6 +1163,21 @@ int fwi_fd2d_set_tb2(fwi_fd2d* p, int cz) {
     p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;
     p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
     return make_tmaps(p);
+}
+
+int fwi_fd2d_set_free_surface(fwi_fd2d* p, int enable) {
+    FWI_REQUIRE(p, "fwi_fd2d_set_free_surface: NULL plan");
+    FWI_REQUIRE(!enable || !p->peer_arena[0], "fwi_fd2d_set_free_surface: this slab has an upper neighbour; only the slab that owns z = 0 has the surface");
+    DeviceGuard g(p->device);
+    FWI_CUDA(cudaStreamSynchronize(p->work));
+    drop_graphs(p);
+    p->free_surface = enable != 0;
+    const std::vector<float> gzh = sponge_profile(p->nz, p->nz, p->nabs, p->alpha, p->free_surface);
+    FWI_CUDA(cudaMemcpy(p->gz, gzh.data(), p->nz * sizeof(float), cudaMemcpyHostToDevice));
+    // the geometry is checked against the surface when it is set
+    p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;
+    p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
+    return FWI_OK;
 }
 
 int fwi_fd2d_set_graphs(fwi_fd2d* p, int enable) {
@@ -1505,6 +1546,7 @@ int fwi_fd_slab_connect(fwi_fd2d* p, int z_own0, int z_own1, const void* up_hand
                         const void* dn_handle, const uint64_t* dn_offsets) {
     FWI_REQUIRE(p && p->ny > 1, "fwi_fd_slab_connect: needs a 3-D plan");
     FWI_REQUIRE(z_own0 >= 0 && z_own1 <= p->nz && z_own1 - z_own0 >= 2 * kHalo, "fwi_fd_slab_connect: owned range [%d, %d) invalid for nz=%d", z_own0, z_own1, p->nz);
+    FWI_REQUIRE(!p->free_surface || !up_handle, "fwi_fd_slab_connect: a free-surface plan cannot have an upper neighbour; only the slab that owns z = 0 has the surface");
     DeviceGuard g(p->device);
     FWI_CUDA(cudaStreamSynchronize(p->work));
     drop_graphs(p);
@@ -1528,6 +1570,7 @@ int fwi_fd_slab_connect(fwi_fd2d* p, int z_own0, int z_own1, const void* up_hand
 int fwi_fd_slab_connect_local(fwi_fd2d* p, int z_own0, int z_own1, fwi_fd2d* up, int up_ghost_z, fwi_fd2d* dn) {
     FWI_REQUIRE(p && p->ny > 1, "fwi_fd_slab_connect_local: needs a 3-D plan");
     FWI_REQUIRE(z_own0 >= 0 && z_own1 <= p->nz && z_own1 - z_own0 >= 2 * kHalo, "fwi_fd_slab_connect_local: owned range [%d, %d) invalid for nz=%d", z_own0, z_own1, p->nz);
+    FWI_REQUIRE(!p->free_surface || !up, "fwi_fd_slab_connect_local: a free-surface plan cannot have an upper neighbour; only the slab that owns z = 0 has the surface");
     DeviceGuard g(p->device);
     FWI_CUDA(cudaStreamSynchronize(p->work));
     drop_graphs(p);

@@ -41,7 +41,9 @@ struct Tb2Args {
     float* rec2;
 };
 
-template <int CZ, int NW, int MODE>
+// FS: free surface at z = 0 (spec B6).  The top row of CTAs mirrors the u_n rows above the surface after the TMA arrives,
+// and the u_{n+1} rows above it again after step 1 and its injection; step 1's own values above the surface are discarded.
+template <int CZ, int NW, int MODE, bool FS>
 __global__ void __launch_bounds__(NW * 32) fd2d_tb2_kernel(const __grid_constant__ CUtensorMap tm_cur,
                                                             const __grid_constant__ CUtensorMap tm_old,
                                                             const __grid_constant__ CUtensorMap tm_m, Tb2Args a) {
@@ -78,6 +80,10 @@ __global__ void __launch_bounds__(NW * 32) fd2d_tb2_kernel(const __grid_constant
     __syncthreads();
 
     mbar_wait(&bar, 0);
+    if (FS && z0 == 0) {                                     // uniform per CTA; sCur row 8 is z = 0
+        mirror_rows(sCur, kT2W0, 8, kT2W0);
+        __syncthreads();
+    }
 
     // ------------------------------------------------------------------ step 1 on the core +- 4
     {
@@ -137,6 +143,10 @@ __global__ void __launch_bounds__(NW * 32) fd2d_tb2_kernel(const __grid_constant
             }
             __syncthreads();
         }
+    }
+    if (FS && z0 == 0) {                                     // sOld row 4 is z = 0; the injected u_{n+1} is mirrored
+        mirror_rows(sOld, kT2W1, 4, kT2W1);
+        __syncthreads();
     }
 
     // ------------------------------------------------------------------ step 2 on the core

@@ -112,7 +112,13 @@ __global__ void fd3d_slab_sync_kernel(int* sync, int has_up, int has_dn, long lo
     }
 }
 
-template <int MODE, int BY>
+// FS: free surface at z = 0 (spec B6).  For a plane z < 0 the producer loads plane -z and the consumers negate it as it enters
+// their register windows (u[-k] = -u[k]); centre planes never lie above the surface, so the x / y neighbours are unchanged.
+// The planes above the surface are the first four of the chunk that starts at z = 0, which marches upwards: a chunk marches
+// downwards only when it is the last of two or more, and chunks hold at least 8 planes (make_tmaps3), so a downward march
+// ends at z >= 4.  The producer handles both directions; the consumers test only while priming (testing every plane of the
+// march as well raised the ADJ2 instance's spills from 24 to 92 bytes at BY = 16).
+template <int MODE, int BY, bool FS>
 __global__ void __launch_bounds__(T3<BY>::Threads, 1) fd3d_step_kernel(const __grid_constant__ CUtensorMap tm_cur,
                                                                        const __grid_constant__ CUtensorMap tm_old,
                                                                        const __grid_constant__ CUtensorMap tm_m, Step3DArgs a) {
@@ -186,7 +192,8 @@ __global__ void __launch_bounds__(T3<BY>::Threads, 1) fd3d_step_kernel(const __g
                     const int slot = t % k3NP;
                     if (t >= k3NP) mbar_wait(&empty_bar[slot], ((t / k3NP) - 1) & 1);
                     mbar_expect_tx(&full_bar[slot], k3PlaneFloats * (uint32_t)sizeof(float));
-                    tma_load_3d(ring + (size_t)slot * k3PlaneStride, &tm_cur, x0 - kHalo, y0 - kHalo, zbeg + zstep * (t - kHalo), &full_bar[slot]);
+                    const int zp = zbeg + zstep * (t - kHalo);
+                    tma_load_3d(ring + (size_t)slot * k3PlaneStride, &tm_cur, x0 - kHalo, y0 - kHalo, (FS && zp < 0) ? -zp : zp, &full_bar[slot]);
                 }
                 const int j = t - k3OmLead;
                 if (do_om && j >= 0 && j < nout) {
@@ -214,12 +221,16 @@ __global__ void __launch_bounds__(T3<BY>::Threads, 1) fd3d_step_kernel(const __g
         auto own = [&](int p, int r) {                 // this lane's element of row r in ring plane p
             return ld4(ring + (size_t)(p % k3NP) * k3PlaneStride + (yl + r + kHalo) * k3SX + kHalo + 4 * lane);
         };
+        auto neg = [](float4 v) { return make_float4(-v.x, -v.y, -v.z, -v.w); };
         // prime with planes 0..7 (the four behind the first output plane and the first four); planes 0..3 are never
         // centre planes -> release them
         for (int p = 0; p < 2 * kHalo; ++p) {
             mbar_wait(&full_bar[p % k3NP], (p / k3NP) & 1);
 #pragma unroll
-            for (int r = 0; r < k3RPW; ++r) win[r][p + 1] = own(p, r);
+            for (int r = 0; r < k3RPW; ++r) {
+                win[r][p + 1] = own(p, r);
+                if (FS && zbeg + zstep * (p - kHalo) < 0) win[r][p + 1] = neg(win[r][p + 1]);     // mirrored plane -z
+            }
             if (p < kHalo) {
                 __syncwarp();
                 if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&empty_bar[p % k3NP])) : "memory");

@@ -63,6 +63,16 @@ __device__ __forceinline__ void st4(float* p, const float4& v) { *reinterpret_ca
 __device__ __forceinline__ void st4_stream(float* p, const float4& v) { __stcs(reinterpret_cast<float4*>(p), v); }
 __device__ __forceinline__ float4 ld4_stream(const float* p) { return __ldcs(reinterpret_cast<const float4*>(p)); }
 
+// Free surface at z = 0 (spec B6): the 4 shared-memory rows above the surface become the odd mirror of the rows below it,
+// u[-k] = -u[k] for k = 1..4, over `width` floats of rows `stride` apart; row `row0` holds z = 0.  The whole CTA takes part;
+// the caller synchronises before the rows are read.
+__device__ __forceinline__ void mirror_rows(float* s, int stride, int row0, int width) {
+    for (int i = threadIdx.x; i < kHalo * width; i += blockDim.x) {
+        const int k = 1 + i / width, c = i - (k - 1) * width;
+        s[(row0 - k) * stride + c] = -s[(row0 + k) * stride + c];
+    }
+}
+
 // sparse point lists (sources / receivers) binned by the CTA tile that owns the point
 struct PointListDev {
     const int* tile_ptr;   // [ntiles + 1]

@@ -170,6 +170,12 @@ int fwi_fd2d_set_tile(fwi_fd2d* plan, int bz, int nw);
 /* Select the temporally blocked kernel: two leapfrog steps per pass on 120 x cz core tiles (cz 24 or 32, else FWI_EINVAL);
  * an odd leftover step runs the one-step tile kernel.  Clears the geometry. */
 int fwi_fd2d_set_tb2(fwi_fd2d* plan, int cz);
+/* Free surface at z = 0 (spec B6, off by default; 2-D and 3-D plans): the values above the grid's first row (plane) are
+ * the odd mirror u[-k] = -u[k] instead of 0, and the sponge does not damp that face.  Rebuilds the z sponge profile (a
+ * later fwi_fd_set_profiles still overrides it), clears the geometry and drops the cached graphs.  While it is on,
+ * fwi_fd*_set_geometry rejects sources and receivers at z = 0 (FWI_EINVAL), and the plan cannot be connected as a slab
+ * with an upper neighbour, nor enabled on one: only the slab that owns global z = 0 has the surface. */
+int fwi_fd2d_set_free_surface(fwi_fd2d* plan, int enable);
 /* Replay the time loops as cached CUDA graphs (default on) or as individual launches (0). */
 int fwi_fd2d_set_graphs(fwi_fd2d* plan, int enable);
 /* Cap (bytes) on the forward-field storage used by fwi_fd2d_gradient; 0 = 85 % of free HBM.  When all nt
