@@ -15,6 +15,7 @@ the field is mirrored oddly above it, the sponge leaves that face undamped, and 
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import math
 from ctypes import POINTER, c_double, c_float, c_int, c_int64, c_uint64, c_void_p
@@ -276,10 +277,6 @@ class Propagator:
 
 Propagator2D = Propagator
 Propagator3D = Propagator
-
-
-def _make_propagator(shape, h, dt, nabs, alpha, device, **kw):
-    return Propagator(shape, h, dt, nabs, alpha, device, **kw)
 
 
 def sponge_profile(n, nabs, alpha, free_surface=False):
@@ -573,36 +570,45 @@ def shard_shots(n_shots, world, rank):
     return list(range(rank, n_shots, world))
 
 
-def forward_model(v, h, dt, shots, wavelet, nabs=20, alpha=0.3, device=None, propagator=None, free_surface=False):
-    """Forward model every shot -> list of (nt, nrec) device tensors (fd_oracle.Problem.forward per shot)."""
-    device = torch.cuda.current_device() if device is None else device
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
+def _shard(n_shots, allreduce, shot_ids):
+    """(process group to sum over or None, indices of the shots this rank runs).  With `shot_ids` the caller passed
+    just this rank's shots, so it runs all of them."""
+    dist = _dist() if allreduce else None
+    if shot_ids is not None or not dist:
+        return dist, range(n_shots)
+    return dist, shard_shots(n_shots, dist.get_world_size(), dist.get_rank())
+
+
+@contextlib.contextmanager
+def _plan(v, h, dt, nabs, alpha, device, propagator, free_surface):
+    """The caller's `propagator`, or a new plan that is closed on exit; either way with the model v set."""
+    prop = propagator or Propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
     try:
         prop.set_model(v)
+        yield prop
+    finally:
+        if propagator is None:
+            prop.close()
+
+
+def forward_model(v, h, dt, shots, wavelet, nabs=20, alpha=0.3, device=None, propagator=None, free_surface=False):
+    """Forward model every shot -> list of (nt, nrec) device tensors (fd_oracle.Problem.forward per shot)."""
+    with _plan(v, h, dt, nabs, alpha, device, propagator, free_surface) as prop:
         out = []
         for src, rec in shots:
             prop.set_geometry(src, rec)
             out.append(prop.forward(wavelet))
         return out
-    finally:
-        if propagator is None:
-            prop.close()
 
 
 def born_model(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None, free_surface=False):
     """Born traces J dv of every shot -> list of (nt, nrec) device tensors (spec B5 per shot, tests/born_reference.py)."""
-    device = torch.cuda.current_device() if device is None else device
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
-    try:
-        prop.set_model(v)
+    with _plan(v, h, dt, nabs, alpha, device, propagator, free_surface) as prop:
         out = []
         for src, rec in shots:
             prop.set_geometry(src, rec)
             out.append(prop.born(wavelet, dv)[0])
         return out
-    finally:
-        if propagator is None:
-            prop.close()
 
 
 def gauss_newton_product(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, device=None, propagator=None, allreduce=True,
@@ -611,26 +617,15 @@ def gauss_newton_product(v, h, dt, shots, wavelet, dv, nabs=20, alpha=0.3, devic
 
     Under torch.distributed the shots are sharded round-robin over the ranks and the product is summed with ONE
     all-reduce, as in `gradient`; with `shot_ids`, `shots` holds just this rank's shots."""
-    device = torch.cuda.current_device() if device is None else device
-    dist = _dist() if allreduce else None
-    if shot_ids is None:
-        ids = shard_shots(len(shots), dist.get_world_size(), dist.get_rank()) if dist else range(len(shots))
-        mine = [shots[i] for i in ids]
-    else:
-        mine = list(shots)
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
-    try:
-        prop.set_model(v)
+    dist, ids = _shard(len(shots), allreduce, shot_ids)
+    with _plan(v, h, dt, nabs, alpha, device, propagator, free_surface) as prop:
         hv = torch.zeros(tuple(v.shape), dtype=torch.float32, device=prop.torch_device)
-        for src, rec in mine:
-            prop.set_geometry(src, rec)
+        for i in ids:
+            prop.set_geometry(*shots[i])
             prop.gauss_newton(wavelet, dv, hv=hv)
         if dist:
             dist.all_reduce(hv)
         return hv
-    finally:
-        if propagator is None:
-            prop.close()
 
 
 def misfit(traces, observed):
@@ -657,22 +652,13 @@ def gradient(v, h, dt, shots, wavelet, observed, nabs=20, alpha=0.3, device=None
     Under torch.distributed the shots are sharded round-robin over the ranks (one GPU each) and the gradient and
     the misfit are summed with ONE all-reduce over NCCL (BASELINE config 3); `shots`/`observed` hold all shots on
     every rank, or - with `shot_ids` - just this rank's."""
-    device = torch.cuda.current_device() if device is None else device
-    dist = _dist() if allreduce else None
-    ids = shot_ids
-    if ids is None:
-        ids = shard_shots(len(shots), dist.get_world_size(), dist.get_rank()) if dist else range(len(shots))
-        mine = [(shots[i], observed[i]) for i in ids]
-    else:
-        mine = list(zip(shots, observed))
-    prop = propagator or _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
-    try:
-        prop.set_model(v)
+    dist, ids = _shard(len(shots), allreduce, shot_ids)
+    with _plan(v, h, dt, nabs, alpha, device, propagator, free_surface) as prop:
         grad = torch.zeros(tuple(v.shape), dtype=torch.float32, device=prop.torch_device)
         J = 0.0
-        for (src, rec), obs in mine:
-            prop.set_geometry(src, rec)
-            j, _, _ = prop.gradient(wavelet, obs, grad=grad)
+        for i in ids:
+            prop.set_geometry(*shots[i])
+            j, _, _ = prop.gradient(wavelet, observed[i], grad=grad)
             J += j
         if dist:
             dist.all_reduce(grad)                       # the one collective of an FWI gradient: fp32, in place over NCCL
@@ -680,9 +666,6 @@ def gradient(v, h, dt, shots, wavelet, observed, nabs=20, alpha=0.3, device=None
             dist.all_reduce(Jt)                         # + the misfit (one float64 scalar)
             J = float(Jt.item())
         return J, grad
-    finally:
-        if propagator is None:
-            prop.close()
 
 
 def model_update(v, grad, step, vmin, vmax):
@@ -713,9 +696,7 @@ def fwi(v0, h, dt, shots, wavelet, observed, niter, vmin, vmax, step_frac=0.02, 
     device = torch.cuda.current_device() if device is None else device
     dev = torch.device("cuda", device)
     v = _dev_f32(v0, dev).clone()
-    dist = _dist()
-    prop = _make_propagator(tuple(v.shape), h, dt, nabs, alpha, device, free_surface=free_surface)
-    ids = shard_shots(len(shots), dist.get_world_size(), dist.get_rank()) if dist else list(range(len(shots)))
+    dist, ids = _shard(len(shots), True, None)
     my_shots = [shots[i] for i in ids]
     my_obs = [_dev_f32(observed[i], dev) for i in ids]
 
@@ -732,7 +713,7 @@ def fwi(v0, h, dt, shots, wavelet, observed, niter, vmin, vmax, step_frac=0.02, 
         return J
 
     history = []
-    try:
+    with _plan(v, h, dt, nabs, alpha, device, None, free_surface) as prop:
         for it in range(niter):
             J, g = gradient(v, h, dt, my_shots, wavelet, my_obs, propagator=prop, shot_ids=ids)
             history.append(J)
@@ -751,5 +732,3 @@ def fwi(v0, h, dt, shots, wavelet, observed, niter, vmin, vmax, step_frac=0.02, 
                 callback(it, J, v)
         history.append(total_misfit(v))
         return v, history
-    finally:
-        prop.close()

@@ -371,10 +371,22 @@ template <typename Shape, size_t N> const Shape* find_shape(const Shape (&table)
     return nullptr;
 }
 
+// The plan's shot-level operations (fwi_fd2d_forward, _gradient, _born, _gauss_newton).
+enum Op { kForward, kGradient, kBorn, kGaussNewton };
+
+// How an operation divides its nt steps: nseg segments of seg steps, the last one possibly shorter.  Gradient and
+// Gauss-Newton: checkpoint segments (nseg = 1: every snapshot is stored); Born: segments of S steps; forward: one segment.
+struct Split { int seg, nseg; };
+
+struct State { int c, o; };      // fld[] indices of u_n and u_{n-1}
+
 struct GraphEntry {
-    int kind, nt, nsrc, nrec, seg, nseg;
+    Op op;
+    int nt, nsrc, nrec;
+    Split split;
     cudaGraphExec_t exec;
     int64_t kernels;
+    State end;                   // the forward state the graph's last forward sweep leaves behind
 };
 
 }  // namespace
@@ -423,7 +435,7 @@ struct fwi_fd2d {
     size_t mem_limit = 0;             // 0 = automatic (fraction of free memory)
     bool pdl = true;                  // chain 2-D steps with programmatic dependent launch (FWI_PDL=0 turns it off)
     bool pdl_chain = false;           // false right after a kernel that rewrites what a step reads BEFORE its dependency wait (m)
-    int split_nt = -1, split_seg = 0, split_nseg = 0; size_t split_limit = 0;   // cached storage decision of the last gradient
+    int split_nt = -1; Split split{0, 0}; size_t split_limit = 0;   // cached storage decision of the last gradient
     int fwd_c = 0, fwd_o = 1;         // fld[] indices of u_n and u_{n-1} after the last forward
     bool model_set = false;
     bool free_surface = false;        // spec B6: odd mirror above z = 0, no sponge on the top face (fwi_fd2d_set_free_surface)
@@ -458,6 +470,12 @@ static std::vector<float> sponge_profile(int n, int padded, int nabs, float alph
 static void drop_graphs(fwi_fd2d* p) {
     for (auto& g : p->graphs) cudaGraphExecDestroy(g.exec);
     p->graphs.clear();
+}
+
+static void clear_geometry(fwi_fd2d* p) {
+    p->src.release(); p->rec.release();
+    p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
+    p->nsrc = p->nrec = 0;
 }
 
 static int make_tmaps3(fwi_fd2d* p) {
@@ -711,21 +729,10 @@ static int ensure_floats(fwi_fd2d* p, float** ptr, size_t* cap, size_t need_floa
     return FWI_OK;
 }
 
-struct State { int c, o; };      // fld[] indices of u_n and u_{n-1}
-
 static void other_two(const State& s, int base, int& a, int& b) {
     int f[2], k = 0;
     for (int i = base; i < base + 4 && k < 2; ++i) if (i != s.c && i != s.o) f[k++] = i;
     a = f[0]; b = f[1];
-}
-static State advance_state(const fwi_fd2d* p, State s, int base, int nsteps) {
-    if (p->family == kTb2) {
-        for (int k = 0; k + 1 < nsteps; k += 2) { int a, b; other_two(s, base, a, b); s = State{a, b}; }
-        if (nsteps & 1) s = State{s.o, s.c};
-        return s;
-    }
-    if (nsteps & 1) s = State{s.o, s.c};
-    return s;
 }
 
 static int launch_tb2(fwi_fd2d* p, int mode, const State& s, int jc, int jd, const PointList* inj_ext, const PointList* inj_own,
@@ -867,21 +874,23 @@ static int restore_state(fwi_fd2d* p, const State& c, const float* ck_cur, const
     return FWI_OK;
 }
 
-// The forward pass as a sequence of stream operations on `st` (captured into a graph or run directly).
-static int record_forward(fwi_fd2d* p, int nt, cudaStream_t st) {
+// The forward pass as a sequence of stream operations on `st` (captured into a graph or run directly).  Each record_*
+// leaves in `fs` the forward state after the last forward sweep it records.
+static int record_forward(fwi_fd2d* p, int nt, cudaStream_t st, State& fs) {
     int rc = zero_state(p, 0, 1, st);
     if (rc) return rc;
-    State s{0, 1};
-    return run_forward(p, p->wav, 0, nt, p->nrec ? p->syn : nullptr, false, 0, s, st);
+    fs = State{0, 1};
+    return run_forward(p, p->wav, 0, nt, p->nrec ? p->syn : nullptr, false, 0, fs, st);
 }
 
 // Born modelling of one shot: per segment of S steps the background forward saves its S snapshots (traces -> p->syn)
 // and the scattered sweep over the same steps consumes them (traces -> p->resid).  Both states carry over from one
 // segment to the next, so no checkpoints are needed and S changes no result.
-static int record_born(fwi_fd2d* p, int nt, int S, cudaStream_t st) {
+static int record_born(fwi_fd2d* p, int nt, int S, cudaStream_t st, State& fs) {
     int rc = zero_state(p, 0, 1, st);
     if (rc || (rc = zero_state(p, 4, 5, st))) return rc;
-    State fs{0, 1}, bs{4, 5};
+    fs = State{0, 1};
+    State bs{4, 5};
     for (int n0 = 0; n0 < nt; n0 += S) {
         const int n1 = std::min(nt, n0 + S);
         if ((rc = run_forward(p, p->wav, n0, n1, p->syn, true, n0, fs, st))) return rc;
@@ -894,12 +903,14 @@ static int record_born(fwi_fd2d* p, int nt, int S, cudaStream_t st) {
 // residual, adjoint with imaging.  Reads p->wav / p->obs, leaves synthetics in p->syn, I in p->acc, J in p->d_J.
 // gauss_newton: every forward segment (or the single full forward) saves its snapshots and is followed by the Born
 // sweep over it, which writes J dv into p->resid in place of the residual; the adjoint then images J^T J dv.
-static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t st, bool gauss_newton = false) {
+// With checkpoints, the last forward sweep is the recompute of the first segment.
+static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t st, State& fs, bool gauss_newton) {
     const size_t pl = p->plane();
     const size_t ntr = (size_t)nt * p->nrec;
     int rc = zero_state(p, 0, 1, st);
     if (rc) return rc;
-    State fs{0, 1}, bs{4, 5};
+    fs = State{0, 1};
+    State bs{4, 5};
     std::vector<State> seg_state(nseg, fs);
     if (gauss_newton && (rc = zero_state(p, 4, 5, st))) return rc;
     if (nseg == 1) {
@@ -933,9 +944,9 @@ static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t 
     } else {
         for (int s = nseg - 1; s >= 0; --s) {
             const int n0 = s * seg, n1 = std::min(nt, (s + 1) * seg);
-            State c = seg_state[s];
-            if ((rc = restore_state(p, c, p->ckpt + (size_t)(2 * s) * pl, p->ckpt + (size_t)(2 * s + 1) * pl, st))) return rc;
-            rc = run_forward(p, p->wav, n0, n1, nullptr, true, n0, c, st);     // recompute w_n for this segment
+            fs = seg_state[s];
+            if ((rc = restore_state(p, fs, p->ckpt + (size_t)(2 * s) * pl, p->ckpt + (size_t)(2 * s + 1) * pl, st))) return rc;
+            rc = run_forward(p, p->wav, n0, n1, nullptr, true, n0, fs, st);     // recompute w_n for this segment
             if (rc) return rc;
             rc = run_adjoint(p, p->resid, n0, n1, n0, as, st);
             if (rc) return rc;
@@ -944,15 +955,21 @@ static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t 
     return FWI_OK;
 }
 
-// Cached graph of a time loop, keyed by (kind, nt, nsrc, nrec, seg, nseg); captured and instantiated on first use.
-template <typename F>
-static int get_graph(fwi_fd2d* p, int kind, int nt, int seg, int nseg, F&& record, GraphEntry** out) {
+static int record(fwi_fd2d* p, Op op, int nt, const Split& split, cudaStream_t st, State& fs) {
+    if (op == kForward) return record_forward(p, nt, st, fs);
+    if (op == kBorn) return record_born(p, nt, split.seg, st, fs);
+    return record_gradient(p, nt, split.seg, split.nseg, st, fs, op == kGaussNewton);
+}
+
+// Cached graph of a time loop, keyed by (op, nt, nsrc, nrec, split); captured and instantiated on first use.
+static int get_graph(fwi_fd2d* p, Op op, int nt, const Split& split, GraphEntry** out) {
     for (auto& g : p->graphs)
-        if (g.kind == kind && g.nt == nt && g.nsrc == p->nsrc && g.nrec == p->nrec && g.seg == seg && g.nseg == nseg) { *out = &g; return FWI_OK; }
+        if (g.op == op && g.nt == nt && g.nsrc == p->nsrc && g.nrec == p->nrec && g.split.seg == split.seg && g.split.nseg == split.nseg) { *out = &g; return FWI_OK; }
     cudaGraph_t graph = nullptr;
     FWI_CUDA(cudaStreamBeginCapture(p->work, cudaStreamCaptureModeThreadLocal));
     const int64_t l0 = p->launches;
-    int rc = record(p->work);
+    State end{0, 1};
+    int rc = record(p, op, nt, split, p->work, end);
     cudaError_t e = cudaStreamEndCapture(p->work, &graph);
     const int64_t kernels = p->launches - l0;
     p->launches = l0;
@@ -963,21 +980,27 @@ static int get_graph(fwi_fd2d* p, int kind, int nt, int seg, int nseg, F&& recor
     cudaGraphDestroy(graph);
     if (e != cudaSuccess) { set_error("cudaGraphInstantiate failed: %s", cudaGetErrorString(e)); return FWI_ECUDA; }
     if (p->graphs.size() >= 6) { cudaGraphExecDestroy(p->graphs.front().exec); p->graphs.erase(p->graphs.begin()); }
-    p->graphs.push_back(GraphEntry{kind, nt, p->nsrc, p->nrec, seg, nseg, exec, kernels});
+    p->graphs.push_back(GraphEntry{op, nt, p->nsrc, p->nrec, split, exec, kernels, end});
     *out = &p->graphs.back();
     return FWI_OK;
 }
 
-// Run `record` either directly on the work stream or as a cached graph.
-template <typename F>
-static int run_cached(fwi_fd2d* p, int kind, int nt, int seg, int nseg, F&& record) {
+// Run an operation's time loop either directly on the work stream or as a cached graph, and note which buffers then
+// hold u_n and u_{n-1} of its last forward sweep.
+static int run_cached(fwi_fd2d* p, Op op, int nt, const Split& split) {
     p->pdl_chain = false;             // the first step of a sweep follows memsets / copies / foreign kernels: full dependency
-    if (!p->use_graphs) return record(p->work);
-    GraphEntry* g = nullptr;
-    int rc = get_graph(p, kind, nt, seg, nseg, record, &g);
-    if (rc) return rc;
-    FWI_CUDA(cudaGraphLaunch(g->exec, p->work));
-    p->launches += g->kernels;
+    State end{0, 1};
+    int rc;
+    if (!p->use_graphs) {
+        if ((rc = record(p, op, nt, split, p->work, end))) return rc;
+    } else {
+        GraphEntry* g = nullptr;
+        if ((rc = get_graph(p, op, nt, split, &g))) return rc;
+        FWI_CUDA(cudaGraphLaunch(g->exec, p->work));
+        p->launches += g->kernels;
+        end = g->end;
+    }
+    p->fwd_c = end.c; p->fwd_o = end.o;
     return FWI_OK;
 }
 
@@ -1125,8 +1148,7 @@ int fwi_fd2d_destroy(fwi_fd2d* p) {
     if (p->obs) cudaFree(p->obs);
     if (p->wav) cudaFree(p->wav);
     if (p->dm) cudaFree(p->dm);
-    p->src.release(); p->rec.release();
-    p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
+    clear_geometry(p);
     for (int s = 0; s < 2; ++s) if (p->peer_arena[s] && p->peer_ipc[s]) cudaIpcCloseMemHandle(p->peer_arena[s]);
     if (p->ev_in) cudaEventDestroy(p->ev_in);
     if (p->ev_out) cudaEventDestroy(p->ev_out);
@@ -1147,7 +1169,7 @@ int fwi_fd2d_set_tile(fwi_fd2d* p, int bz, int nw) {
     drop_graphs(p);
     p->family = kTile; p->tile = t;
     p->tiles_z = (p->nz + bz - 1) / bz;
-    p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;      // tile binning changed
+    clear_geometry(p);                // tile binning changed
     return make_tmaps(p);
 }
 
@@ -1160,8 +1182,7 @@ int fwi_fd2d_set_tb2(fwi_fd2d* p, int cz) {
     FWI_CUDA(cudaStreamSynchronize(p->work));
     drop_graphs(p);
     p->family = kTb2; p->tb2 = t;
-    p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;
-    p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
+    clear_geometry(p);
     return make_tmaps(p);
 }
 
@@ -1174,9 +1195,7 @@ int fwi_fd2d_set_free_surface(fwi_fd2d* p, int enable) {
     p->free_surface = enable != 0;
     const std::vector<float> gzh = sponge_profile(p->nz, p->nz, p->nabs, p->alpha, p->free_surface);
     FWI_CUDA(cudaMemcpy(p->gz, gzh.data(), p->nz * sizeof(float), cudaMemcpyHostToDevice));
-    // the geometry is checked against the surface when it is set
-    p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;
-    p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
+    clear_geometry(p);                // the geometry is checked against the surface when it is set
     return FWI_OK;
 }
 
@@ -1244,22 +1263,124 @@ int fwi_fd3d_set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* sr
     return set_geometry(p, nsrc, src_z, src_y, src_x, nrec, rec_z, rec_y, rec_x);
 }
 
+// ---- the shot-level operations -------------------------------------------------------------------------------------
+// Steps per Born segment: the background sweep saves this many snapshots, then the scattered sweep reads them back.
+// (profiles/r3_born_bench.txt, ms per Born shot at 1000 x 3000, nt = 5000: see DESIGN.md)
+constexpr int kBornSeg = 128;
+
+// Forward-field storage in planes: the memory limit, or 85 % of the free memory plus the floats the plan holds in
+// buffers it may reallocate (`reclaim`).
+static int storage_budget(fwi_fd2d* p, size_t reclaim, size_t& budget, size_t& planes) {
+    budget = p->mem_limit;
+    if (!budget) {
+        size_t fr = 0, tot = 0;
+        FWI_CUDA(cudaMemGetInfo(&fr, &tot));
+        budget = (size_t)((fr + reclaim * sizeof(float)) * 0.85);
+    }
+    planes = budget / (p->plane() * sizeof(float));
+    return FWI_OK;
+}
+
+// Storage decision and buffers of an operation over nt steps (no launches).
+// Gradient and Gauss-Newton hold every w_n in HBM if it fits, else checkpoint.  The decision is cached per (nt, limit):
+// cudaMemGetInfo takes a driver-wide lock and was measured stalling the host for 5 - 90 ms every few calls, which showed
+// up as sporadic slow shots.  Born runs in segments of S = min(nt, kBornSeg, planes the budget allows) steps; it only
+// queries free memory when the snapshot buffer cannot already hold min(nt, kBornSeg) planes.
+static int prepare(fwi_fd2d* p, Op op, int nt, Split& split) {
+    const size_t pl = p->plane(), ntr = (size_t)nt * p->nrec;
+    const bool adjoint = op == kGradient || op == kGaussNewton;
+    split = Split{nt, 1};
+    int rc;
+    if (adjoint && p->split_nt == nt && p->split_limit == p->mem_limit) {
+        split = p->split;
+    } else if (adjoint) {
+        size_t budget = 0, planes = 0;
+        if ((rc = storage_budget(p, p->snap_steps + p->ckpt_slots, budget, planes))) return rc;     // both in floats
+        if ((size_t)nt > planes) {
+            // segment length S with S + 2*ceil(nt/S) planes minimal-ish: start from sqrt(2 nt)
+            split.seg = std::max(1, (int)std::ceil(std::sqrt(2.0 * nt)));
+            split.nseg = (nt + split.seg - 1) / split.seg;
+            FWI_REQUIRE((size_t)split.seg + 2 * (size_t)split.nseg <= planes, "fwi_fd2d_gradient: %zu bytes are not enough even with checkpointing (need %zu planes of %zu bytes)", budget, (size_t)split.seg + 2 * (size_t)split.nseg, pl * sizeof(float));
+        }
+    } else if (op == kBorn) {
+        const int S = std::min(nt, kBornSeg);
+        size_t budget = 0, planes = (size_t)S;
+        if ((p->mem_limit || p->snap_steps < (size_t)S * pl) && (rc = storage_budget(p, p->snap_steps, budget, planes))) return rc;
+        FWI_REQUIRE(planes >= 1, "fwi_fd2d_born: the memory limit holds no snapshot plane of %zu bytes", pl * sizeof(float));
+        split.seg = (int)std::min<size_t>((size_t)S, planes);
+        split.nseg = (nt + split.seg - 1) / split.seg;
+    }
+    if (op != kForward && (rc = ensure_floats(p, &p->snap, &p->snap_steps, (size_t)split.seg * pl))) return rc;   // snap_steps counts floats
+    if (adjoint && split.nseg > 1 && (rc = ensure_floats(p, &p->ckpt, &p->ckpt_slots, (size_t)split.nseg * 2 * pl))) return rc;
+    if (op != kForward && (rc = ensure_floats(p, &p->resid, &p->resid_cap, ntr))) return rc;
+    if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, ntr))) return rc;
+    if (adjoint && (rc = ensure_floats(p, &p->obs, &p->obs_cap, ntr))) return rc;
+    if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
+    if (adjoint) { p->split_nt = nt; p->split_limit = p->mem_limit; p->split = split; }      // buffers exist now
+    if ((op == kBorn || op == kGaussNewton) && (rc = ensure_floats(p, &p->dm, &p->dm_cap, pl))) return rc;
+    return FWI_OK;
+}
+
+// grad (dense grid) += (2 / v) * imaging accumulator
+static int launch_finalize(fwi_fd2d* p, float* grad, cudaStream_t st) {
+    dim3 grid(p->rows(), (p->nx + 127) / 128);
+    fd_grad_finalize_kernel<<<grid, 128, 0, st>>>(p->acc, p->vp, p->rows(), p->nx, p->px, grad);
+    FWI_CUDA(cudaGetLastError());
+    return FWI_OK;
+}
+
+// dm = (2 m / v) dv into the plan-owned pitched buffer, on the work stream ahead of the time loop (captured graphs keep
+// the buffer's address)
+static int stage_dm(fwi_fd2d* p, const float* dv_dev) {
+    dim3 grid(p->rows(), (p->px + 127) / 128);
+    fd_dm_kernel<<<grid, 128, 0, p->work>>>(dv_dev, p->m, p->vp, p->rows(), p->nx, p->px, p->dm);
+    FWI_CUDA(cudaGetLastError());
+    return FWI_OK;
+}
+
+// One shot's device arrays (misfit: host).  A null pointer is an input the operation does not read or an output the
+// caller does not want.
+struct ShotIO {
+    const float* wavelet = nullptr;
+    const float* obs = nullptr;
+    const float* dv = nullptr;
+    float* image = nullptr;           // dense grid += (2 / v) I: the gradient, or J^T J dv
+    float* traces = nullptr;          // synthetics
+    float* dtraces = nullptr;         // Born traces J dv
+    double* misfit = nullptr;         // J = 1/2 sum r^2; waits for the shot
+};
+
+// One shot of `op` on the plan's work stream, ordered after everything queued on `stream` and before what follows on it.
+static int run_shot(fwi_fd2d* p, Op op, int nt, void* stream, const ShotIO& io) {
+    DeviceGuard g(p->device);
+    cudaStream_t user = (cudaStream_t)stream;
+    Split split;
+    int rc;
+    if ((rc = prepare(p, op, nt, split)) || (rc = enter(p, user))) return rc;
+    const size_t nw = (size_t)nt * p->nsrc, ntr = (size_t)nt * p->nrec;
+    if (nw) FWI_CUDA(cudaMemcpyAsync(p->wav, io.wavelet, nw * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (io.obs && ntr) FWI_CUDA(cudaMemcpyAsync(p->obs, io.obs, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (io.dv && (rc = stage_dm(p, io.dv))) return rc;
+    if ((rc = run_cached(p, op, nt, split))) return rc;
+    if (io.image) {
+        if ((rc = launch_finalize(p, io.image, p->work))) return rc;
+        p->launches += 1;
+    }
+    if (io.dtraces && ntr) FWI_CUDA(cudaMemcpyAsync(io.dtraces, p->resid, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (io.traces && ntr) FWI_CUDA(cudaMemcpyAsync(io.traces, p->syn, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (io.misfit) FWI_CUDA(cudaMemcpyAsync(io.misfit, p->d_J, sizeof(double), cudaMemcpyDeviceToHost, p->work));
+    if ((rc = leave(p, user))) return rc;
+    if (io.misfit) FWI_CUDA(cudaStreamSynchronize(p->work));
+    return FWI_OK;
+}
+
 int fwi_fd2d_forward(fwi_fd2d* p, const float* wavelet_dev, int nt, float* traces_dev, void* stream) {
     FWI_REQUIRE(p && p->model_set, "fwi_fd2d_forward: set the model first");
     FWI_REQUIRE(nt >= 0 && (p->nsrc == 0 || wavelet_dev), "fwi_fd2d_forward: bad wavelet / nt");
     FWI_REQUIRE(p->nrec == 0 || traces_dev, "fwi_fd2d_forward: traces_dev is NULL but receivers are set");
-    DeviceGuard g(p->device);
-    cudaStream_t user = (cudaStream_t)stream;
-    int rc;
-    if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
-    if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, (size_t)nt * p->nrec))) return rc;
-    if ((rc = enter(p, user))) return rc;
-    if (nt * p->nsrc) FWI_CUDA(cudaMemcpyAsync(p->wav, wavelet_dev, (size_t)nt * p->nsrc * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    rc = run_cached(p, 0, nt, 0, 0, [&](cudaStream_t st) { return record_forward(p, nt, st); });
-    if (rc) return rc;
-    if (nt * p->nrec) FWI_CUDA(cudaMemcpyAsync(traces_dev, p->syn, (size_t)nt * p->nrec * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    { State fs = advance_state(p, State{0, 1}, 0, nt); p->fwd_c = fs.c; p->fwd_o = fs.o; }
-    return leave(p, user);
+    ShotIO io;
+    io.wavelet = wavelet_dev; io.traces = traces_dev;
+    return run_shot(p, kForward, nt, stream, io);
 }
 
 int fwi_fd2d_wavefield(fwi_fd2d* p, int which, float* out_dev, void* stream) {
@@ -1275,60 +1396,21 @@ int fwi_fd2d_wavefield(fwi_fd2d* p, int which, float* out_dev, void* stream) {
     return leave(p, user);
 }
 
-// Storage decision and buffers of a gradient over nt steps (no launches).  Every w_n in HBM if it fits, else two-level
-// checkpointing.  The decision is cached per (nt, limit): cudaMemGetInfo takes a driver-wide lock and was measured
-// stalling the host for 5 - 90 ms every few calls, which showed up as sporadic slow shots.
-static int prepare_gradient(fwi_fd2d* p, int nt, int& seg, int& nseg) {
-    const size_t pl = p->plane();
-    seg = nt; nseg = 1;
-    if (p->split_nt == nt && p->split_limit == p->mem_limit) {
-        seg = p->split_seg; nseg = p->split_nseg;
-    } else {
-        size_t budget = p->mem_limit;
-        if (!budget) {
-            size_t fr = 0, tot = 0;
-            FWI_CUDA(cudaMemGetInfo(&fr, &tot));
-            budget = (size_t)((fr + (p->snap_steps + p->ckpt_slots) * sizeof(float)) * 0.85);   // both capacities are in floats
-        }
-        const size_t max_planes = budget / (pl * sizeof(float));
-        if ((size_t)nt > max_planes) {
-            // segment length S with S + 2*ceil(nt/S) planes minimal-ish: start from sqrt(2 nt)
-            seg = std::max(1, (int)std::ceil(std::sqrt(2.0 * nt)));
-            nseg = (nt + seg - 1) / seg;
-            FWI_REQUIRE((size_t)seg + 2 * (size_t)nseg <= max_planes, "fwi_fd2d_gradient: %zu bytes are not enough even with checkpointing (need %zu planes of %zu bytes)", budget, (size_t)seg + 2 * (size_t)nseg, pl * sizeof(float));
-        }
-    }
-    int rc;
-    if ((rc = ensure_floats(p, &p->snap, &p->snap_steps, (size_t)seg * pl))) return rc;     // snap_steps counts floats here
-    if (nseg > 1 && (rc = ensure_floats(p, &p->ckpt, &p->ckpt_slots, (size_t)nseg * 2 * pl))) return rc;
-    const size_t ntr = (size_t)nt * p->nrec;
-    if ((rc = ensure_floats(p, &p->resid, &p->resid_cap, ntr))) return rc;
-    if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, ntr))) return rc;
-    if ((rc = ensure_floats(p, &p->obs, &p->obs_cap, ntr))) return rc;
-    if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
-    p->split_nt = nt; p->split_limit = p->mem_limit; p->split_seg = seg; p->split_nseg = nseg;      // buffers exist now
-    return FWI_OK;
-}
-
 // Allocate everything fwi_fd2d_forward (gradient = 0) or fwi_fd2d_gradient (1) over nt steps with the current geometry
 // will need, without launching anything: keeps allocations (which synchronise the device) out of timed regions and out
 // of the way of kernels that wait for another plan.
 int fwi_fd_reserve(fwi_fd2d* p, int nt, int gradient) {
     FWI_REQUIRE(p && nt >= 1, "fwi_fd_reserve: bad arguments");
     DeviceGuard g(p->device);
-    int rc, seg = 0, nseg = 0;
-    if (gradient) { if ((rc = prepare_gradient(p, nt, seg, nseg))) return rc; }
-    else {
-        if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
-        if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, (size_t)nt * p->nrec))) return rc;
-    }
+    const Op op = gradient ? kGradient : kForward;
+    Split split;
+    int rc = prepare(p, op, nt, split);
+    if (rc) return rc;
     if (p->use_graphs && p->model_set) {          // capture, instantiate and upload the time loop now as well
-        GraphEntry* g = nullptr;
+        GraphEntry* e = nullptr;
         p->pdl_chain = false;
-        if (gradient) rc = get_graph(p, 1, nt, seg, nseg, [&](cudaStream_t st) { return record_gradient(p, nt, seg, nseg, st); }, &g);
-        else rc = get_graph(p, 0, nt, 0, 0, [&](cudaStream_t st) { return record_forward(p, nt, st); }, &g);
-        if (rc) return rc;
-        FWI_CUDA(cudaGraphUpload(g->exec, p->work));
+        if ((rc = get_graph(p, op, nt, split, &e))) return rc;
+        FWI_CUDA(cudaGraphUpload(e->exec, p->work));
         FWI_CUDA(cudaStreamSynchronize(p->work));
     }
     return FWI_OK;
@@ -1339,34 +1421,12 @@ int fwi_fd2d_gradient(fwi_fd2d* p, const float* wavelet_dev, const float* obs_de
     FWI_REQUIRE(p && p->model_set, "fwi_fd2d_gradient: set the model first");
     FWI_REQUIRE((wavelet_dev || p->nsrc == 0) && (obs_dev || p->nrec == 0) && grad_dev && nt >= 1, "fwi_fd2d_gradient: NULL argument or nt < 1");
     FWI_REQUIRE((p->nsrc >= 1 && p->nrec >= 1) || p->z_own1 > 0, "fwi_fd2d_gradient: geometry needs at least one source and one receiver");
-    DeviceGuard g(p->device);
-    cudaStream_t user = (cudaStream_t)stream;
-    int seg = nt, nseg = 1, rc;
-    if ((rc = prepare_gradient(p, nt, seg, nseg))) return rc;
-    const size_t ntr = (size_t)nt * p->nrec;
-
-    if ((rc = enter(p, user))) return rc;
-    if (nt * p->nsrc) FWI_CUDA(cudaMemcpyAsync(p->wav, wavelet_dev, (size_t)nt * p->nsrc * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if (ntr) FWI_CUDA(cudaMemcpyAsync(p->obs, obs_dev, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    rc = run_cached(p, 1, nt, seg, nseg, [&](cudaStream_t st) { return record_gradient(p, nt, seg, nseg, st); });
-    if (rc) return rc;
-    { State fs = advance_state(p, State{0, 1}, 0, nt); p->fwd_c = fs.c; p->fwd_o = fs.o; }
-    dim3 grid(p->rows(), (p->nx + 127) / 128);
-    fd_grad_finalize_kernel<<<grid, 128, 0, p->work>>>(p->acc, p->vp, p->rows(), p->nx, p->px, grad_dev);
-    FWI_CUDA(cudaGetLastError());
-    p->launches += 1;
-    if (traces_dev && ntr) FWI_CUDA(cudaMemcpyAsync(traces_dev, p->syn, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if (misfit_host) FWI_CUDA(cudaMemcpyAsync(misfit_host, p->d_J, sizeof(double), cudaMemcpyDeviceToHost, p->work));
-    if ((rc = leave(p, user))) return rc;
-    if (misfit_host) FWI_CUDA(cudaStreamSynchronize(p->work));
-    return FWI_OK;
+    ShotIO io;
+    io.wavelet = wavelet_dev; io.obs = obs_dev; io.image = grad_dev; io.traces = traces_dev; io.misfit = misfit_host;
+    return run_shot(p, kGradient, nt, stream, io);
 }
 
 // ---- Born modelling and Gauss-Newton Hessian-vector products (spec B5) ------------------------------------------
-// Steps per Born segment: the background sweep saves this many snapshots, then the scattered sweep reads them back.
-// (profiles/r3_born_bench.txt, ms per Born shot at 1000 x 3000, nt = 5000: see DESIGN.md)
-constexpr int kBornSeg = 128;
-
 static int check_linearised(fwi_fd2d* p, const char* fn, const float* wavelet_dev, const float* dv_dev, const float* out_dev, int nt) {
     FWI_REQUIRE(p && p->model_set, "%s: set the model first", fn);
     FWI_REQUIRE(wavelet_dev && dv_dev && out_dev && nt >= 1, "%s: NULL argument or nt < 1", fn);
@@ -1376,85 +1436,22 @@ static int check_linearised(fwi_fd2d* p, const char* fn, const float* wavelet_de
     return FWI_OK;
 }
 
-// dm = (2 m / v) dv into the plan-owned pitched buffer, on the work stream ahead of the time loop (captured graphs keep
-// the buffer's address)
-static int stage_dm(fwi_fd2d* p, const float* dv_dev) {
-    dim3 grid(p->rows(), (p->px + 127) / 128);
-    fd_dm_kernel<<<grid, 128, 0, p->work>>>(dv_dev, p->m, p->vp, p->rows(), p->nx, p->px, p->dm);
-    FWI_CUDA(cudaGetLastError());
-    return FWI_OK;
-}
-
-// Segment length S of a Born run and its buffers: S = min(nt, kBornSeg, snapshot planes the memory limit / free memory
-// allows).  Free memory is only queried when the snapshot buffer cannot already hold min(nt, kBornSeg) planes.
-static int prepare_born(fwi_fd2d* p, int nt, int& S) {
-    const size_t pl = p->plane();
-    S = std::min(nt, kBornSeg);
-    size_t max_planes = 0;
-    if (p->mem_limit) max_planes = p->mem_limit / (pl * sizeof(float));
-    else if (p->snap_steps >= (size_t)S * pl) max_planes = (size_t)S;
-    else {
-        size_t fr = 0, tot = 0;
-        FWI_CUDA(cudaMemGetInfo(&fr, &tot));
-        max_planes = (size_t)((fr + p->snap_steps * sizeof(float)) * 0.85) / (pl * sizeof(float));
-    }
-    FWI_REQUIRE(max_planes >= 1, "fwi_fd2d_born: the memory limit holds no snapshot plane of %zu bytes", pl * sizeof(float));
-    S = (int)std::min<size_t>((size_t)S, max_planes);
-    const size_t ntr = (size_t)nt * p->nrec;
-    int rc;
-    if ((rc = ensure_floats(p, &p->snap, &p->snap_steps, (size_t)S * pl))) return rc;
-    if ((rc = ensure_floats(p, &p->resid, &p->resid_cap, ntr))) return rc;
-    if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, ntr))) return rc;
-    if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
-    return ensure_floats(p, &p->dm, &p->dm_cap, pl);
-}
-
 int fwi_fd2d_born(fwi_fd2d* p, const float* wavelet_dev, const float* dv_dev, int nt, float* dtraces_dev, float* traces_dev,
                   void* stream) {
     int rc = check_linearised(p, "fwi_fd2d_born", wavelet_dev, dv_dev, dtraces_dev, nt);
     if (rc) return rc;
-    DeviceGuard g(p->device);
-    cudaStream_t user = (cudaStream_t)stream;
-    int S = 1;
-    if ((rc = prepare_born(p, nt, S))) return rc;
-    const size_t ntr = (size_t)nt * p->nrec;
-    if ((rc = enter(p, user))) return rc;
-    FWI_CUDA(cudaMemcpyAsync(p->wav, wavelet_dev, (size_t)nt * p->nsrc * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if ((rc = stage_dm(p, dv_dev))) return rc;
-    rc = run_cached(p, 2, nt, S, 0, [&](cudaStream_t st) { return record_born(p, nt, S, st); });
-    if (rc) return rc;
-    FWI_CUDA(cudaMemcpyAsync(dtraces_dev, p->resid, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if (traces_dev) FWI_CUDA(cudaMemcpyAsync(traces_dev, p->syn, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    {   // the background ran in segments: a tb2 plan pairs its steps per segment
-        State fs{0, 1};
-        for (int n0 = 0; n0 < nt; n0 += S) fs = advance_state(p, fs, 0, std::min(nt, n0 + S) - n0);
-        p->fwd_c = fs.c; p->fwd_o = fs.o;
-    }
-    return leave(p, user);
+    ShotIO io;
+    io.wavelet = wavelet_dev; io.dv = dv_dev; io.dtraces = dtraces_dev; io.traces = traces_dev;
+    return run_shot(p, kBorn, nt, stream, io);
 }
 
 int fwi_fd2d_gauss_newton(fwi_fd2d* p, const float* wavelet_dev, const float* dv_dev, int nt, float* hv_dev, float* dtraces_dev,
                           void* stream) {
     int rc = check_linearised(p, "fwi_fd2d_gauss_newton", wavelet_dev, dv_dev, hv_dev, nt);
     if (rc) return rc;
-    DeviceGuard g(p->device);
-    cudaStream_t user = (cudaStream_t)stream;
-    int seg = nt, nseg = 1;
-    if ((rc = prepare_gradient(p, nt, seg, nseg))) return rc;
-    if ((rc = ensure_floats(p, &p->dm, &p->dm_cap, p->plane()))) return rc;
-    const size_t ntr = (size_t)nt * p->nrec;
-    if ((rc = enter(p, user))) return rc;
-    FWI_CUDA(cudaMemcpyAsync(p->wav, wavelet_dev, (size_t)nt * p->nsrc * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if ((rc = stage_dm(p, dv_dev))) return rc;
-    rc = run_cached(p, 3, nt, seg, nseg, [&](cudaStream_t st) { return record_gradient(p, nt, seg, nseg, st, true); });
-    if (rc) return rc;
-    { State fs = advance_state(p, State{0, 1}, 0, nt); p->fwd_c = fs.c; p->fwd_o = fs.o; }
-    dim3 grid(p->rows(), (p->nx + 127) / 128);
-    fd_grad_finalize_kernel<<<grid, 128, 0, p->work>>>(p->acc, p->vp, p->rows(), p->nx, p->px, hv_dev);   // H dv = (2 / v) I
-    FWI_CUDA(cudaGetLastError());
-    p->launches += 1;
-    if (dtraces_dev) FWI_CUDA(cudaMemcpyAsync(dtraces_dev, p->resid, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    return leave(p, user);
+    ShotIO io;
+    io.wavelet = wavelet_dev; io.dv = dv_dev; io.image = hv_dev; io.dtraces = dtraces_dev;     // H dv = (2 / v) I
+    return run_shot(p, kGaussNewton, nt, stream, io);
 }
 
 int64_t fwi_fd2d_launch_count(fwi_fd2d* p) { return p ? p->launches : 0; }
@@ -1536,7 +1533,7 @@ int fwi_fd_slab_info(fwi_fd2d* p, void* ipc_handle_out /*64 bytes*/, uint64_t* o
 static int slab_finish_connect(fwi_fd2d* p, int z_own0, int z_own1, int up_ghost_z) {
     p->z_own0 = z_own0; p->z_own1 = z_own1; p->peer_up_z = up_ghost_z;
     if (const char* e = getenv("FWI_SLAB_TIMEOUT_MS")) { const double ms = atof(e); if (ms > 0) p->slab_timeout_cycles = (long long)(ms * 1.9e6); }
-    p->src.release(); p->rec.release(); p->nsrc = p->nrec = 0;         // z chunking (and so the point binning) changes
+    clear_geometry(p);                // z chunking (and so the point binning) changes
     return make_tmaps(p);
 }
 
@@ -1613,10 +1610,7 @@ int fwi_fd_slab_error(fwi_fd2d* p, int* error_out) {
 int fwi_fd_finalize_gradient(fwi_fd2d* p, float* grad_dev, void* stream) {
     FWI_REQUIRE(p && grad_dev, "fwi_fd_finalize_gradient: bad arguments");
     DeviceGuard g(p->device);
-    dim3 grid(p->rows(), (p->nx + 127) / 128);
-    fd_grad_finalize_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(p->acc, p->vp, p->rows(), p->nx, p->px, grad_dev);
-    FWI_CUDA(cudaGetLastError());
-    return FWI_OK;
+    return launch_finalize(p, grad_dev, (cudaStream_t)stream);
 }
 
 

@@ -192,7 +192,10 @@ int fwi_fd2d_set_geometry(fwi_fd2d* plan, int nsrc, const int* src_z_host, const
  * u_{n+1} at the receivers (fd_oracle.Problem.forward).  Source injection and receiver sampling are fused
  * into the step kernel. */
 int fwi_fd2d_forward(fwi_fd2d* plan, const float* wavelet_dev, int nt, float* traces_dev, void* stream);
-/* Copy a field out as dense (nz, nx): which = 0 u_n, 1 u_{n-1} (after the last forward), 2 imaging sum I. */
+/* Copy a field out as dense (nz, nx): which = 0 u_n, 1 u_{n-1} (after the last forward sweep), 2 imaging sum I.
+ * After a forward, a Born call or a gradient / Gauss-Newton product that stored every snapshot, that is u_nt, u_{nt-1};
+ * after a checkpointed gradient / Gauss-Newton product it is u_S, u_{S-1}, where the recompute of the first segment of
+ * S steps ended. */
 int fwi_fd2d_wavefield(fwi_fd2d* plan, int which, float* out_dev, void* stream);
 /* One shot's misfit and gradient (fd_oracle.Problem.misfit_and_gradient): forward with w_n kept in HBM
  * (or checkpointed), residual = synthetic - observed, adjoint back-propagation with the zero-lag

@@ -115,6 +115,12 @@ def test_checkpointed_gradient_matches_stored(ac, kw):
     assert abs(J1 - J0) <= 1e-12 * J0
     # identical up to the pairing of the deferred imaging at the receiver points (segments pair steps differently)
     assert rel_l2(g1.cpu().numpy(), g0.cpu().numpy()) <= 1e-6
+    # the last forward sweep was the recompute of the first segment: wavefield() returns its u_21 and u_20
+    import torch
+    cur, old = prop.wavefield(0), prop.wavefield(1)
+    prop.forward(wav[:21])
+    assert torch.equal(prop.wavefield(0), cur)
+    assert torch.equal(prop.wavefield(1), old)
     prop.set_memory_limit(5 * plane)
     with pytest.raises(ValueError):
         prop.gradient(wav, obs)

@@ -231,7 +231,8 @@ def test_born_is_the_directional_derivative_at_500x1500(ac):
 # ------------------------------------------------------------------------------------------------ 5. exact properties
 @pytest.mark.parametrize("kw", [dict(tile=(32, 4)), dict(tb2=24), "3d"])
 def test_segment_length_changes_no_bit(ac, kw):
-    """Default segment, S = 1 and S = 7 (forced through the memory limit): bit-identical Born and background traces."""
+    """Default segment, S = 1 and S = 7 (forced through the memory limit): bit-identical Born and background traces, and
+    the same final background wavefields u_nt, u_{nt-1}."""
     if kw == "3d":
         shape, nt = (36, 30, 140), 45
         v, h, dt, src, rec, wav, dv = case3d(shape, nt, seed=4)
@@ -241,12 +242,15 @@ def test_segment_length_changes_no_bit(ac, kw):
         v, h, dt, src, rec, wav, dv = case2d(*shape, nt, seed=4)
     p = plan(ac, shape, h, dt, v, src, rec, 8, **kw)
     ref, ref_tr = [t.cpu().numpy() for t in p.born(wav, dv, want_traces=True)]
+    ref_u = [p.wavefield(k).cpu().numpy() for k in (0, 1)]
     assert np.abs(ref).max() > 0
     for planes in (1, 7):
         p.set_memory_limit(planes * plane_bytes(shape))
         got, got_tr = [t.cpu().numpy() for t in p.born(wav, dv, want_traces=True)]
         assert np.array_equal(got, ref), planes
         assert np.array_equal(got_tr, ref_tr), planes
+        for k in (0, 1):
+            assert np.array_equal(p.wavefield(k).cpu().numpy(), ref_u[k]), (planes, k)
     p.set_memory_limit(plane_bytes(shape) - 4)          # not even one snapshot plane
     with pytest.raises(ValueError):
         p.born(wav, dv)
