@@ -8,7 +8,8 @@ device buffers, and ``torch.distributed`` (NCCL) carries the one collective: the
 over shots.
 
 Conventions: velocity grids are (nz, nx) [2-D] or (nz, ny, nx) [3-D] float32, x contiguous;
-a shot is ``(src, rec)`` with integer index arrays of shape (n, ndim) in (z[, y], x) order;
+a shot is ``(src, rec)`` with integer index arrays of shape (n, ndim) in (z[, y], x) order, or float positions in cell
+units (spec B7, tests/offgrid_reference.py: a point between cells is a short list of weighted cells);
 wavelets are (nt,) or (nt, nsrc); traces are (nt, nrec), time-major; a velocity perturbation dv is grid-shaped.
 `free_surface=True` makes grid row (plane) z = 0 a pressure-free surface (spec B6, tests/free_surface_reference.py):
 the field is mirrored oddly above it, the sponge leaves that face undamped, and sources and receivers need z >= 1.
@@ -44,6 +45,8 @@ _lib.register({
     "fwi_fd2d_launch_count": (c_int64, [c_void_p]),
     "fwi_fd3d_create": (c_int, [c_int, c_int, c_int, c_int, c_float, c_float, c_int, c_float, POINTER(c_void_p)]),
     "fwi_fd3d_set_geometry": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "fwi_fd2d_set_positions": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "fwi_fd3d_set_positions": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "fwi_fd_set_profiles": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "fwi_fd_field_ptr": (c_void_p, [c_void_p, c_int]),
     "fwi_fd_pitch": (c_int, [c_void_p]),
@@ -85,9 +88,18 @@ def _dev_f32(x, device):
     return torch.as_tensor(np.ascontiguousarray(x, dtype=np.float32)).to(device)
 
 
-def _points(pts, ndim):
-    a = np.ascontiguousarray(np.asarray(pts, dtype=np.int32).reshape(-1, ndim))
+def _points(pts, ndim, dtype=np.int32):
+    a = np.ascontiguousarray(np.asarray(pts, dtype=dtype).reshape(-1, ndim))
     return [np.ascontiguousarray(a[:, k]) for k in range(ndim)]
+
+
+def _off_grid(*point_sets):
+    """True if any of the point sets is a non-empty array of a floating dtype: positions in cell units (spec B7)."""
+    for pts in point_sets:
+        a = pts.cpu().numpy() if isinstance(pts, torch.Tensor) else np.asarray(pts)
+        if a.size and a.dtype.kind == "f":
+            return True
+    return False
 
 
 class Propagator:
@@ -147,9 +159,17 @@ class Propagator:
         self._v = v
 
     def set_geometry(self, src, rec):
-        s_ = _points(src, self.ndim)
-        r_ = _points(rec, self.ndim)
-        fn = self._lib.fwi_fd2d_set_geometry if self.ndim == 2 else self._lib.fwi_fd3d_set_geometry
+        """Sources and receivers as (n, ndim) arrays in (z[, y], x) order.  Integer arrays (or lists of ints) are grid indices
+        (B2).  If either is a floating array, both are positions in cell units (spec B7): each coordinate in [0, n - 1],
+        z > 0 with a free surface; a point between cells injects into / samples a weighted list of cells."""
+        if _off_grid(src, rec):
+            s_ = _points(src, self.ndim, np.float64)
+            r_ = _points(rec, self.ndim, np.float64)
+            fn = self._lib.fwi_fd2d_set_positions if self.ndim == 2 else self._lib.fwi_fd3d_set_positions
+        else:
+            s_ = _points(src, self.ndim)
+            r_ = _points(rec, self.ndim)
+            fn = self._lib.fwi_fd2d_set_geometry if self.ndim == 2 else self._lib.fwi_fd3d_set_geometry
         check(fn(self._h, len(s_[0]), *[a.ctypes.data_as(c_void_p) for a in s_],
                  len(r_[0]), *[a.ctypes.data_as(c_void_p) for a in r_]))
         self.nsrc, self.nrec = len(s_[0]), len(r_[0])
@@ -428,6 +448,9 @@ class SlabPropagator:
             self.prop.set_model(v[lo:hi])
 
     def set_geometry(self, src, rec):
+        if _off_grid(src, rec):
+            # a point's taps may straddle two slabs, and a rank's residual would miss the part another rank samples
+            raise ValueError("SlabPropagator takes integer grid indices only; off-grid positions need a single-GPU Propagator")
         ndim = len(self.shape)
         src = np.asarray(src, dtype=np.int64).reshape(-1, ndim)
         rec = np.asarray(rec, dtype=np.int64).reshape(-1, ndim)

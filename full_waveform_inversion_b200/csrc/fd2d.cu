@@ -247,6 +247,46 @@ __global__ void fd_residual_kernel(const float* __restrict__ syn, const float* _
     }
 }
 
+// Off-grid points (spec B7, tests/offgrid_reference.py): an operator in CSR form maps time-major rows of one side to the
+// other, out[n][j] = sum_{e in [ptr[j], ptr[j+1])} w[e] * in[n][col[e]], summed in CSR order so that every run gives the
+// same bits.  Gather: point-major CSR, cell rows in, point rows out (traces); spread: cell-major CSR, point rows in, cell
+// rows out (wavelets, residuals).  One kernel serves both; the two names keep them apart in profiles.
+// A thread owns one output column and kInterpRows time rows: the lanes of a warp read their CSR entries 64 taps apart (one
+// L1 wavefront per lane), so each (col, w) is loaded once for kInterpRows rows (measured at 3000 receivers x 64 taps,
+// nt = 5000: 6.8 ms per gather with one row per thread).
+constexpr int kInterpRows = 8;
+__device__ __forceinline__ void interp_rows(const int* __restrict__ ptr, const int* __restrict__ col, const float* __restrict__ w,
+                                            const float* __restrict__ in, int nin, float* __restrict__ out, int nout, int nt) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= nout) return;
+    const int e0 = ptr[j], e1 = ptr[j + 1];
+    for (int n0 = blockIdx.y * kInterpRows; n0 < nt; n0 += gridDim.y * kInterpRows) {
+        const int nn = min(kInterpRows, nt - n0);
+        const float* rows = in + (size_t)n0 * nin;
+        float acc[kInterpRows];
+#pragma unroll
+        for (int k = 0; k < kInterpRows; ++k) acc[k] = 0.f;
+        for (int e = e0; e < e1; ++e) {
+            const float we = w[e];
+            const float* p = rows + col[e];
+#pragma unroll
+            for (int k = 0; k < kInterpRows; ++k)
+                if (k < nn) acc[k] = fmaf(we, p[(size_t)k * nin], acc[k]);
+        }
+#pragma unroll
+        for (int k = 0; k < kInterpRows; ++k)
+            if (k < nn) out[(size_t)(n0 + k) * nout + j] = acc[k];
+    }
+}
+__global__ void fd_interp_gather_kernel(const int* __restrict__ ptr, const int* __restrict__ col, const float* __restrict__ w,
+                                        const float* __restrict__ in, int nin, float* __restrict__ out, int nout, int nt) {
+    interp_rows(ptr, col, w, in, nin, out, nout, nt);
+}
+__global__ void fd_interp_spread_kernel(const int* __restrict__ ptr, const int* __restrict__ col, const float* __restrict__ w,
+                                        const float* __restrict__ in, int nin, float* __restrict__ out, int nout, int nt) {
+    interp_rows(ptr, col, w, in, nin, out, nout, nt);
+}
+
 __global__ void fd_update_kernel(float* __restrict__ v, const float* __restrict__ g, float step, float vmin, float vmax,
                                  int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -313,6 +353,27 @@ struct PointList {
     static PointListDev dev(const PointList* pl) {
         return (pl && pl->n) ? PointListDev{pl->d_tile_ptr, pl->d_off, pl->d_id} : PointListDev{nullptr, nullptr, nullptr};
     }
+};
+
+// A sparse operator in CSR form (fd_interp_*_kernel): rows[j] sums w[e] * in[col[e]] over e in [ptr[j], ptr[j+1]).
+struct Csr {
+    int rows = 0, cap_rows = 0, cap_nnz = 0;
+    int* d_ptr = nullptr; int* d_col = nullptr; float* d_w = nullptr;
+    void release() {
+        if (d_ptr) cudaFree(d_ptr);
+        if (d_col) cudaFree(d_col);
+        if (d_w) cudaFree(d_w);
+        d_ptr = d_col = nullptr; d_w = nullptr; rows = cap_rows = cap_nnz = 0;
+    }
+};
+
+// Off-grid points of one side (spec B7, fwi_fd*_set_positions): `npts` points whose taps land on the side's unique cells,
+// which are what the step kernels' point lists hold.  by_point (point -> cells) gathers traces, by_cell (cell -> points)
+// spreads wavelets and residuals.  npts = -1: the integer geometry is set, and a point is its cell.
+struct Interp {
+    int npts = -1;
+    Csr by_point, by_cell;
+    void release() { by_point.release(); by_cell.release(); npts = -1; }
 };
 
 // The step-kernel families: the one-step tile kernel, the two-steps-per-pass kernel (temporal blocking, "tb2") and the
@@ -382,7 +443,8 @@ struct State { int c, o; };      // fld[] indices of u_n and u_{n-1}
 
 struct GraphEntry {
     Op op;
-    int nt, nsrc, nrec;
+    int nt, nsrc, nrec;          // cells that sources / receivers inject into / sample
+    int psrc, prec;              // off-grid points (Interp::npts; -1 with the integer geometry)
     Split split;
     cudaGraphExec_t exec;
     int64_t kernels;
@@ -431,7 +493,10 @@ struct fwi_fd2d {
     double* d_J = nullptr;
     PointList src, rec;
     PointList src_ext2, src_own2, rec_ext2, rec_own2;   // tb2: binned by the 120 x cz core tiles (+-4 for *_ext2)
-    int nsrc = 0, nrec = 0;
+    int nsrc = 0, nrec = 0;           // source / receiver cells: the columns of p->wav, p->syn, p->resid
+    Interp isrc, irec;                // off-grid points (spec B7) over those cells
+    float* pts = nullptr; size_t pts_cap = 0;     // off grid: gradient synthetics / Gauss-Newton J dv at the receivers
+    float* pres = nullptr; size_t pres_cap = 0;   // off grid: the residual at the receivers
     size_t mem_limit = 0;             // 0 = automatic (fraction of free memory)
     bool pdl = true;                  // chain 2-D steps with programmatic dependent launch (FWI_PDL=0 turns it off)
     bool pdl_chain = false;           // false right after a kernel that rewrites what a step reads BEFORE its dependency wait (m)
@@ -475,8 +540,12 @@ static void drop_graphs(fwi_fd2d* p) {
 static void clear_geometry(fwi_fd2d* p) {
     p->src.release(); p->rec.release();
     p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
+    p->isrc.release(); p->irec.release();
     p->nsrc = p->nrec = 0;
 }
+
+// Receivers as the caller sees them: traces, observed data and residuals have this many columns.
+static int rec_points(const fwi_fd2d* p) { return p->irec.npts >= 0 ? p->irec.npts : p->nrec; }
 
 static int make_tmaps3(fwi_fd2d* p) {
     p->tiles_x = (p->nx + k3BX - 1) / k3BX;
@@ -839,6 +908,18 @@ static int run_born(fwi_fd2d* p, int n0, int n1, size_t snap_base, State& s, flo
     return FWI_OK;
 }
 
+// Off-grid points (spec B7): out (nt, op.rows) = in (nt, nin) through the CSR operator `op`, gathering (cells -> points)
+// or spreading (points -> cells).
+static int launch_interp(fwi_fd2d* p, bool gather, const Csr& op, const float* in, int nin, float* out, int nt, cudaStream_t st) {
+    if (!op.rows || nt < 1) return FWI_OK;
+    const dim3 grid((op.rows + 127) / 128, std::min((nt + kInterpRows - 1) / kInterpRows, 65535));
+    if (gather) fd_interp_gather_kernel<<<grid, 128, 0, st>>>(op.d_ptr, op.d_col, op.d_w, in, nin, out, op.rows, nt);
+    else fd_interp_spread_kernel<<<grid, 128, 0, st>>>(op.d_ptr, op.d_col, op.d_w, in, nin, out, op.rows, nt);
+    FWI_CUDA(cudaGetLastError());
+    p->launches += 1;
+    return FWI_OK;
+}
+
 // ---- peer-memory slabs: what may be overwritten when ---------------------------------------------------------------
 // A neighbour stores its boundary planes of launch k into THIS GPU's ghost planes of the buffer launch k writes.  Before a
 // run (or a checkpointed segment) rewrites wavefields, a one-thread kernel waits until the neighbours have pushed
@@ -930,7 +1011,19 @@ static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t 
         }
     }
     FWI_CUDA(cudaMemsetAsync(p->d_J, 0, sizeof(double), st));
-    if (ntr && !gauss_newton) {
+    if (p->irec.npts >= 0) {
+        // off grid (spec B7): the misfit lives at the receivers and the adjoint sources are W^T r at the cells.  Gather the
+        // synthetics (Gauss-Newton: J dv), take the residual there, spread it (J dv) back into p->resid.
+        const int np = p->irec.npts;
+        const size_t ntp = (size_t)nt * np;
+        if ((rc = launch_interp(p, true, p->irec.by_point, gauss_newton ? p->resid : p->syn, p->nrec, p->pts, nt, st))) return rc;
+        if (ntp && !gauss_newton) {
+            fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntp + 255) / 256), 256, 0, st>>>(p->pts, p->obs, (int64_t)ntp, p->pres, p->d_J);
+            FWI_CUDA(cudaGetLastError());
+            p->launches += 1;
+        }
+        if ((rc = launch_interp(p, false, p->irec.by_cell, gauss_newton ? p->pts : p->pres, np, p->resid, nt, st))) return rc;
+    } else if (ntr && !gauss_newton) {
         fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntr + 255) / 256), 256, 0, st>>>(p->syn, p->obs, (int64_t)ntr, p->resid, p->d_J);
         FWI_CUDA(cudaGetLastError());
         p->launches += 1;
@@ -961,10 +1054,10 @@ static int record(fwi_fd2d* p, Op op, int nt, const Split& split, cudaStream_t s
     return record_gradient(p, nt, split.seg, split.nseg, st, fs, op == kGaussNewton);
 }
 
-// Cached graph of a time loop, keyed by (op, nt, nsrc, nrec, split); captured and instantiated on first use.
+// Cached graph of a time loop, keyed by (op, nt, cells and off-grid points of both sides, split); captured and instantiated on first use.
 static int get_graph(fwi_fd2d* p, Op op, int nt, const Split& split, GraphEntry** out) {
     for (auto& g : p->graphs)
-        if (g.op == op && g.nt == nt && g.nsrc == p->nsrc && g.nrec == p->nrec && g.split.seg == split.seg && g.split.nseg == split.nseg) { *out = &g; return FWI_OK; }
+        if (g.op == op && g.nt == nt && g.nsrc == p->nsrc && g.nrec == p->nrec && g.psrc == p->isrc.npts && g.prec == p->irec.npts && g.split.seg == split.seg && g.split.nseg == split.nseg) { *out = &g; return FWI_OK; }
     cudaGraph_t graph = nullptr;
     FWI_CUDA(cudaStreamBeginCapture(p->work, cudaStreamCaptureModeThreadLocal));
     const int64_t l0 = p->launches;
@@ -980,7 +1073,7 @@ static int get_graph(fwi_fd2d* p, Op op, int nt, const Split& split, GraphEntry*
     cudaGraphDestroy(graph);
     if (e != cudaSuccess) { set_error("cudaGraphInstantiate failed: %s", cudaGetErrorString(e)); return FWI_ECUDA; }
     if (p->graphs.size() >= 6) { cudaGraphExecDestroy(p->graphs.front().exec); p->graphs.erase(p->graphs.begin()); }
-    p->graphs.push_back(GraphEntry{op, nt, p->nsrc, p->nrec, split, exec, kernels, end});
+    p->graphs.push_back(GraphEntry{op, nt, p->nsrc, p->nrec, p->isrc.npts, p->irec.npts, split, exec, kernels, end});
     *out = &p->graphs.back();
     return FWI_OK;
 }
@@ -1148,6 +1241,8 @@ int fwi_fd2d_destroy(fwi_fd2d* p) {
     if (p->obs) cudaFree(p->obs);
     if (p->wav) cudaFree(p->wav);
     if (p->dm) cudaFree(p->dm);
+    if (p->pts) cudaFree(p->pts);
+    if (p->pres) cudaFree(p->pres);
     clear_geometry(p);
     for (int s = 0; s < 2; ++s) if (p->peer_arena[s] && p->peer_ipc[s]) cudaIpcCloseMemHandle(p->peer_arena[s]);
     if (p->ev_in) cudaEventDestroy(p->ev_in);
@@ -1225,17 +1320,18 @@ int fwi_fd2d_set_model(fwi_fd2d* p, const float* v_dev, void* stream) {
     return leave(p, user);
 }
 
-static int set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
-                        const int* rec_z, const int* rec_y, const int* rec_x) {
-    FWI_REQUIRE(p, "fwi_fd_set_geometry: NULL plan");
-    FWI_REQUIRE(nsrc >= 0 && nrec >= 0 && (nsrc == 0 || (src_z && src_x)) && (nrec == 0 || (rec_z && rec_x)), "fwi_fd_set_geometry: bad arguments");
-    DeviceGuard g(p->device);
-    if (nsrc != p->nsrc || nrec != p->nrec) drop_graphs(p);
+// Ints that staging the point lists of `npts` sources and receivers takes: 2 + 4 lists; a tb2 point sits in <= 4 tiles.
+static size_t bin_staging(const fwi_fd2d* p, size_t npts) {
     const size_t bins = (size_t)std::max({p->tiles_x * p->tiles_y * p->nzch, p->tiles_x * p->tiles_z, p->tiles_x2 * p->tiles_z2}) + 1;
-    int rc = stage_begin(p, 6 * bins + 2 * 10 * ((size_t)nsrc + nrec + 16));      // 2 + 4 lists; a tb2 point sits in <= 4 tiles
-    if (rc) return rc;
+    return 6 * bins + 2 * 10 * (npts + 16);
+}
+
+// Bins the source and receiver cells into the point lists of every kernel family the plan runs (uploads staged by the caller).
+static int bin_points(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
+                      const int* rec_z, const int* rec_y, const int* rec_x) {
+    if (nsrc != p->nsrc || nrec != p->nrec) drop_graphs(p);
     const TileGrid step = tile_grid(p, p->family == k3D ? k3D : kTile);     // tb2 plans run the tile kernel for single steps
-    rc = build_point_list(p, p->src, step, 0, nsrc, src_z, src_y, src_x, "source");
+    int rc = build_point_list(p, p->src, step, 0, nsrc, src_z, src_y, src_x, "source");
     if (rc) return rc;
     rc = build_point_list(p, p->rec, step, 0, nrec, rec_z, rec_y, rec_x, "receiver");
     if (rc) return rc;
@@ -1247,7 +1343,156 @@ static int set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_
         if ((rc = build_point_list(p, p->rec_own2, pass, 0, nrec, rec_z, rec_y, rec_x, "receiver"))) return rc;
     }
     p->nsrc = nsrc; p->nrec = nrec;
+    return FWI_OK;
+}
+
+static int set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
+                        const int* rec_z, const int* rec_y, const int* rec_x) {
+    FWI_REQUIRE(p, "fwi_fd_set_geometry: NULL plan");
+    FWI_REQUIRE(nsrc >= 0 && nrec >= 0 && (nsrc == 0 || (src_z && src_x)) && (nrec == 0 || (rec_z && rec_x)), "fwi_fd_set_geometry: bad arguments");
+    DeviceGuard g(p->device);
+    p->isrc.npts = p->irec.npts = -1;         // points are cells again
+    int rc = stage_begin(p, bin_staging(p, (size_t)nsrc + nrec));
+    if (rc || (rc = bin_points(p, nsrc, src_z, src_y, src_x, nrec, rec_z, rec_y, rec_x))) return rc;
     return stage_end(p);
+}
+
+// ---- off-grid points (spec B7, tests/offgrid_reference.py) ---------------------------------------------------------
+// Kaiser window parameter of the windowed-sinc taps: the b on a 0.01 grid that minimises
+// E(b) = max |sum_k w_k(f) exp(i kappa d_k) - 1| over kappa in [0, 2 pi / 3], f in [0, 1)  (E(4.06) = 8.79e-3).
+constexpr double kKaiserB = 4.06;
+
+// One axis's taps of a coordinate x in cell units on n cells: (index, weight) in ascending index, float64.  An integral x is
+// one tap of weight 1; otherwise 8 taps at floor(x) - 3 .. floor(x) + 4 of Hicks' Kaiser-windowed sinc with half-width 4.
+// `fold` (the free-surface z axis): a tap at -k lands on +k with its weight negated, a tap on row 0 is dropped.  Taps
+// outside [0, n) are dropped (the zero halo of B1); taps on one index are summed.
+static std::vector<std::pair<int, double>> axis_taps(double x, int n, bool fold) {
+    std::vector<std::pair<int, double>> t;
+    const double fl = std::floor(x), f = x - fl;
+    const int i = (int)fl;
+    if (f == 0.0) { t.push_back({i, 1.0}); return t; }
+    const double i0b = std::cyl_bessel_i(0.0, kKaiserB);
+    for (int k = -3; k <= 4; ++k) {
+        const double d = k - f, pd = M_PI * d;
+        double w = std::sin(pd) / pd * std::cyl_bessel_i(0.0, kKaiserB * std::sqrt(1.0 - (d / 4) * (d / 4))) / i0b;
+        int j = i + k;
+        if (fold && j < 0) { j = -j; w = -w; }
+        if ((fold && j == 0) || j < 0 || j >= n) continue;
+        auto it = std::find_if(t.begin(), t.end(), [j](const std::pair<int, double>& e) { return e.first == j; });
+        if (it != t.end()) it->second += w;
+        else t.push_back({j, w});
+    }
+    std::sort(t.begin(), t.end());
+    return t;
+}
+
+// One side's off-grid points as cells and the two CSR forms of the operator W (points x cells).
+struct SideTaps {
+    std::vector<int> cz, cy, cx;                          // the unique cells, in ascending linear offset
+    std::vector<int> pt_ptr, pt_col, cell_ptr, cell_col;
+    std::vector<float> pt_w, cell_w;
+};
+
+static int build_side(const fwi_fd2d* p, int n, const double* z, const double* y, const double* x, const char* what, SideTaps& s) {
+    const double dims[3] = {(double)p->nz, (double)p->ny, (double)p->nx};
+    std::vector<std::pair<int64_t, std::pair<int, double>>> taps;        // (cell offset, (point, weight)), point-major
+    s.pt_ptr.assign(1, 0);
+    for (int i = 0; i < n; ++i) {
+        const double c[3] = {z[i], y ? y[i] : 0.0, x[i]};
+        FWI_REQUIRE(std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]), "%s %d at (z=%g, y=%g, x=%g) is not finite", what, i, c[0], c[1], c[2]);
+        for (int d = 0; d < 3; ++d)
+            FWI_REQUIRE(c[d] >= 0.0 && c[d] <= dims[d] - 1, "%s %d at (z=%g, y=%g, x=%g) is outside the %d x %d x %d grid (each coordinate must lie in [0, n - 1])", what, i, c[0], c[1], c[2], p->nz, p->ny, p->nx);
+        FWI_REQUIRE(!p->free_surface || c[0] > 0.0, "%s %d at (z=%g, y=%g, x=%g) lies on the free surface; off-grid points need z > 0", what, i, c[0], c[1], c[2]);
+        const auto tz = axis_taps(c[0], p->nz, p->free_surface), ty = axis_taps(c[1], p->ny, false), tx = axis_taps(c[2], p->nx, false);
+        for (const auto& a : tz)
+            for (const auto& b : ty)
+                for (const auto& e : tx)
+                    taps.push_back({((int64_t)a.first * p->ny + b.first) * p->nx + e.first, {i, a.second * b.second * e.second}});
+        s.pt_ptr.push_back((int)taps.size());
+    }
+    std::vector<int64_t> cells(taps.size());
+    for (size_t e = 0; e < taps.size(); ++e) cells[e] = taps[e].first;
+    std::sort(cells.begin(), cells.end());
+    cells.erase(std::unique(cells.begin(), cells.end()), cells.end());
+    const int nc = (int)cells.size();
+    s.cz.resize(nc); s.cy.resize(nc); s.cx.resize(nc);
+    for (int c = 0; c < nc; ++c) {
+        s.cx[c] = (int)(cells[c] % p->nx);
+        s.cy[c] = (int)(cells[c] / p->nx % p->ny);
+        s.cz[c] = (int)(cells[c] / p->nx / p->ny);
+    }
+    // a point's taps come in ascending cell order and never repeat a cell (axis_taps merged them per axis)
+    s.pt_col.resize(taps.size()); s.pt_w.resize(taps.size());
+    s.cell_ptr.assign(nc + 1, 0);
+    for (size_t e = 0; e < taps.size(); ++e) {
+        s.pt_col[e] = (int)(std::lower_bound(cells.begin(), cells.end(), taps[e].first) - cells.begin());
+        s.pt_w[e] = (float)taps[e].second.second;
+        s.cell_ptr[s.pt_col[e] + 1]++;
+    }
+    for (int c = 0; c < nc; ++c) s.cell_ptr[c + 1] += s.cell_ptr[c];
+    std::vector<int> fill(s.cell_ptr.begin(), s.cell_ptr.end() - 1);
+    s.cell_col.resize(taps.size()); s.cell_w.resize(taps.size());
+    for (size_t e = 0; e < taps.size(); ++e) {                           // points of a cell in ascending order
+        const int k = fill[s.pt_col[e]]++;
+        s.cell_col[k] = taps[e].second.first;
+        s.cell_w[k] = s.pt_w[e];
+    }
+    return FWI_OK;
+}
+
+static size_t csr_staging(const SideTaps& s) { return s.pt_ptr.size() + s.cell_ptr.size() + 4 * s.pt_col.size(); }
+
+static int upload_csr(fwi_fd2d* p, Csr& c, const std::vector<int>& ptr, const std::vector<int>& col, const std::vector<float>& w) {
+    const int rows = (int)ptr.size() - 1, nnz = (int)col.size();
+    if (c.cap_rows < rows || c.cap_nnz < std::max(nnz, 1)) {       // allocations change -> cached graphs hold stale pointers
+        c.release();
+        drop_graphs(p);
+        const int cr = rows + rows / 2 + 16, cn = nnz + nnz / 2 + 16;
+        FWI_CUDA(cudaMalloc(&c.d_ptr, (cr + 1) * sizeof(int)));
+        FWI_CUDA(cudaMalloc(&c.d_col, cn * sizeof(int)));
+        FWI_CUDA(cudaMalloc(&c.d_w, cn * sizeof(float)));
+        c.cap_rows = cr; c.cap_nnz = cn;
+    }
+    int rc = stage_upload(p, c.d_ptr, ptr.data(), ptr.size());
+    // (the weights travel through the int staging buffer bit for bit)
+    if (!rc && nnz) rc = stage_upload(p, c.d_col, col.data(), nnz);
+    if (!rc && nnz) rc = stage_upload(p, (int*)c.d_w, (const int*)w.data(), nnz);
+    c.rows = rows;
+    return rc;
+}
+
+static int set_positions(fwi_fd2d* p, int nsrc, const double* src_z, const double* src_y, const double* src_x, int nrec,
+                         const double* rec_z, const double* rec_y, const double* rec_x) {
+    FWI_REQUIRE(p, "fwi_fd_set_positions: NULL plan");
+    FWI_REQUIRE(nsrc >= 0 && nrec >= 0 && (nsrc == 0 || (src_z && src_x)) && (nrec == 0 || (rec_z && rec_x)), "fwi_fd_set_positions: bad arguments");
+    // a point's taps may straddle two slabs, and a slab's residual would miss the part of a trace another rank samples
+    FWI_REQUIRE(!p->peers(), "fwi_fd_set_positions: not available on a plan connected as a peer-memory slab");
+    SideTaps s, r;
+    int rc = build_side(p, nsrc, src_z, src_y, src_x, "source", s);
+    if (rc || (rc = build_side(p, nrec, rec_z, rec_y, rec_x, "receiver", r))) return rc;
+    DeviceGuard g(p->device);
+    p->isrc.npts = p->irec.npts = -1;
+    const int ncs = (int)s.cz.size(), ncr = (int)r.cz.size();
+    if ((rc = stage_begin(p, bin_staging(p, (size_t)ncs + ncr) + csr_staging(s) + csr_staging(r)))) return rc;
+    if ((rc = bin_points(p, ncs, s.cz.data(), s.cy.data(), s.cx.data(), ncr, r.cz.data(), r.cy.data(), r.cx.data()))) return rc;
+    if ((rc = upload_csr(p, p->isrc.by_point, s.pt_ptr, s.pt_col, s.pt_w)) || (rc = upload_csr(p, p->isrc.by_cell, s.cell_ptr, s.cell_col, s.cell_w)) ||
+        (rc = upload_csr(p, p->irec.by_point, r.pt_ptr, r.pt_col, r.pt_w)) || (rc = upload_csr(p, p->irec.by_cell, r.cell_ptr, r.cell_col, r.cell_w)))
+        return rc;
+    p->isrc.npts = nsrc; p->irec.npts = nrec;
+    return stage_end(p);
+}
+
+int fwi_fd2d_set_positions(fwi_fd2d* p, int nsrc, const double* src_z, const double* src_x, int nrec, const double* rec_z,
+                           const double* rec_x) {
+    FWI_REQUIRE(p && p->ny == 1, "fwi_fd2d_set_positions: needs a 2-D plan");
+    return set_positions(p, nsrc, src_z, nullptr, src_x, nrec, rec_z, nullptr, rec_x);
+}
+
+int fwi_fd3d_set_positions(fwi_fd2d* p, int nsrc, const double* src_z, const double* src_y, const double* src_x, int nrec,
+                           const double* rec_z, const double* rec_y, const double* rec_x) {
+    FWI_REQUIRE(p && p->ny > 1, "fwi_fd3d_set_positions: needs a 3-D plan");
+    FWI_REQUIRE((nsrc == 0 || src_y) && (nrec == 0 || rec_y), "fwi_fd3d_set_positions: y coordinates missing");
+    return set_positions(p, nsrc, src_z, src_y, src_x, nrec, rec_z, rec_y, rec_x);
 }
 
 int fwi_fd2d_set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_x, int nrec, const int* rec_z,
@@ -1287,7 +1532,7 @@ static int storage_budget(fwi_fd2d* p, size_t reclaim, size_t& budget, size_t& p
 // up as sporadic slow shots.  Born runs in segments of S = min(nt, kBornSeg, planes the budget allows) steps; it only
 // queries free memory when the snapshot buffer cannot already hold min(nt, kBornSeg) planes.
 static int prepare(fwi_fd2d* p, Op op, int nt, Split& split) {
-    const size_t pl = p->plane(), ntr = (size_t)nt * p->nrec;
+    const size_t pl = p->plane(), ntr = (size_t)nt * p->nrec, ntp = (size_t)nt * rec_points(p);
     const bool adjoint = op == kGradient || op == kGaussNewton;
     split = Split{nt, 1};
     int rc;
@@ -1314,7 +1559,9 @@ static int prepare(fwi_fd2d* p, Op op, int nt, Split& split) {
     if (adjoint && split.nseg > 1 && (rc = ensure_floats(p, &p->ckpt, &p->ckpt_slots, (size_t)split.nseg * 2 * pl))) return rc;
     if (op != kForward && (rc = ensure_floats(p, &p->resid, &p->resid_cap, ntr))) return rc;
     if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, ntr))) return rc;
-    if (adjoint && (rc = ensure_floats(p, &p->obs, &p->obs_cap, ntr))) return rc;
+    if (adjoint && (rc = ensure_floats(p, &p->obs, &p->obs_cap, ntp))) return rc;
+    if (adjoint && p->irec.npts >= 0 &&
+        ((rc = ensure_floats(p, &p->pts, &p->pts_cap, ntp)) || (rc = ensure_floats(p, &p->pres, &p->pres_cap, ntp)))) return rc;
     if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
     if (adjoint) { p->split_nt = nt; p->split_limit = p->mem_limit; p->split = split; }      // buffers exist now
     if ((op == kBorn || op == kGaussNewton) && (rc = ensure_floats(p, &p->dm, &p->dm_cap, pl))) return rc;
@@ -1350,6 +1597,16 @@ struct ShotIO {
     double* misfit = nullptr;         // J = 1/2 sum r^2; waits for the shot
 };
 
+// Trace rows (nt, receivers) of a shot into the caller's `dst` from the cell rows `cells`: a copy on the grid; off grid
+// (spec B7) gathered to the receivers, or, with `gathered`, copied from p->pts, where the graph already gathered them.
+static int copy_traces(fwi_fd2d* p, float* dst, const float* cells, bool gathered, int nt) {
+    const size_t n = (size_t)nt * rec_points(p);
+    if (!n) return FWI_OK;
+    if (p->irec.npts >= 0 && !gathered) return launch_interp(p, true, p->irec.by_point, cells, p->nrec, dst, nt, p->work);
+    FWI_CUDA(cudaMemcpyAsync(dst, p->irec.npts >= 0 ? p->pts : cells, n * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    return FWI_OK;
+}
+
 // One shot of `op` on the plan's work stream, ordered after everything queued on `stream` and before what follows on it.
 static int run_shot(fwi_fd2d* p, Op op, int nt, void* stream, const ShotIO& io) {
     DeviceGuard g(p->device);
@@ -1357,17 +1614,21 @@ static int run_shot(fwi_fd2d* p, Op op, int nt, void* stream, const ShotIO& io) 
     Split split;
     int rc;
     if ((rc = prepare(p, op, nt, split)) || (rc = enter(p, user))) return rc;
-    const size_t nw = (size_t)nt * p->nsrc, ntr = (size_t)nt * p->nrec;
-    if (nw) FWI_CUDA(cudaMemcpyAsync(p->wav, io.wavelet, nw * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if (io.obs && ntr) FWI_CUDA(cudaMemcpyAsync(p->obs, io.obs, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    const size_t nw = (size_t)nt * p->nsrc, ntp = (size_t)nt * rec_points(p);
+    if (p->isrc.npts >= 0) {          // off grid (spec B7): the cells' wavelets are W_s^T times the points'
+        if ((rc = launch_interp(p, false, p->isrc.by_cell, io.wavelet, p->isrc.npts, p->wav, nt, p->work))) return rc;
+    } else if (nw) {
+        FWI_CUDA(cudaMemcpyAsync(p->wav, io.wavelet, nw * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    }
+    if (io.obs && ntp) FWI_CUDA(cudaMemcpyAsync(p->obs, io.obs, ntp * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
     if (io.dv && (rc = stage_dm(p, io.dv))) return rc;
     if ((rc = run_cached(p, op, nt, split))) return rc;
     if (io.image) {
         if ((rc = launch_finalize(p, io.image, p->work))) return rc;
         p->launches += 1;
     }
-    if (io.dtraces && ntr) FWI_CUDA(cudaMemcpyAsync(io.dtraces, p->resid, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
-    if (io.traces && ntr) FWI_CUDA(cudaMemcpyAsync(io.traces, p->syn, ntr * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (io.dtraces && (rc = copy_traces(p, io.dtraces, p->resid, op == kGaussNewton, nt))) return rc;
+    if (io.traces && (rc = copy_traces(p, io.traces, p->syn, op == kGradient, nt))) return rc;
     if (io.misfit) FWI_CUDA(cudaMemcpyAsync(io.misfit, p->d_J, sizeof(double), cudaMemcpyDeviceToHost, p->work));
     if ((rc = leave(p, user))) return rc;
     if (io.misfit) FWI_CUDA(cudaStreamSynchronize(p->work));
@@ -1497,6 +1758,7 @@ int fwi_fd_reset(fwi_fd2d* p, int pair, void* stream) {
 int fwi_fd_step(fwi_fd2d* p, int mode, int cur, const float* inj_vals_dev, float* rec_out_dev, int64_t snap_index, void* stream) {
     FWI_REQUIRE(p && p->model_set, "fwi_fd_step: set the model first");
     FWI_REQUIRE(mode >= 0 && mode <= 2 && (cur == 0 || cur == 1), "fwi_fd_step: bad mode / cur");
+    FWI_REQUIRE(p->irec.npts < 0, "fwi_fd_step: the plan holds off-grid positions (fwi_fd*_set_positions); single steps take the integer geometry");
     p->pdl_chain = false;             // caller-driven loop: other kernels (halo exchange, resets) sit between the steps
     FWI_REQUIRE(mode == 0 || (snap_index >= 0 && (size_t)(snap_index + 1) * p->plane() <= p->snap_steps), "fwi_fd_step: snapshot %lld not reserved", (long long)snap_index);
     DeviceGuard g(p->device);

@@ -224,6 +224,23 @@ int fwi_fd_reserve(fwi_fd2d* plan, int nt, int gradient);
 int fwi_fd3d_create(int device, int nz, int ny, int nx, float h, float dt, int nabs, float alpha, fwi_fd2d** out);
 int fwi_fd3d_set_geometry(fwi_fd2d* plan, int nsrc, const int* src_z_host, const int* src_y_host, const int* src_x_host,
                           int nrec, const int* rec_z_host, const int* rec_y_host, const int* rec_x_host);     /* step-kernel launches so far (bench bookkeeping) */
+/* Off-grid geometry (spec B7, tests/offgrid_reference.py): sources and receivers at float coordinates in cell units (host
+ * arrays; 10.5 lies half-way between rows 10 and 11), each coordinate in [0, n - 1] of its axis, z > 0 with a free surface.
+ * A point with a fractional coordinate is a tensor product of 8 Kaiser-windowed sinc taps per fractional axis (b = 4.06);
+ * an integral coordinate is one tap.  Taps outside the grid are dropped; with a free surface a tap at row -k folds onto
+ * row k with its weight negated and a tap on row 0 is dropped.  Sources inject wavelet x weight at every tap cell,
+ * receivers record sum weight x u_{n+1} over their taps, and the misfit, gradient, Born and Gauss-Newton products are
+ * taken at the points.  Replaces any geometry; fwi_fd*_set_geometry replaces it in turn.  Wavelets, observed data and
+ * traces keep their (nt, points) layout.  Each shot operation then adds, on top of its step kernels: one spread of the
+ * wavelet; a gradient or Gauss-Newton product one gather and one spread of the residual (J dv) inside its graph; a
+ * forward or Born call one gather per trace array it returns.  FWI_EINVAL, naming the point, for a coordinate that is
+ * not finite, outside the grid or at z <= 0 under a free surface; FWI_EINVAL on a plan connected as a peer-memory slab;
+ * fwi_fd_step is FWI_EINVAL while the plan holds positions. */
+int fwi_fd2d_set_positions(fwi_fd2d* plan, int nsrc, const double* src_z_host, const double* src_x_host,
+                           int nrec, const double* rec_z_host, const double* rec_x_host);
+int fwi_fd3d_set_positions(fwi_fd2d* plan, int nsrc, const double* src_z_host, const double* src_y_host,
+                           const double* src_x_host, int nrec, const double* rec_z_host, const double* rec_y_host,
+                           const double* rec_x_host);
 
 /* Low-level stepping API: the caller drives the time loop, one leapfrog step per call on the caller's stream.
  * Used by the slab-decomposed multi-GPU path (acoustic.SlabPropagator), which exchanges the 4-plane halos of the
