@@ -460,10 +460,11 @@ class SlabPropagator:
             loc = p[keep].copy()
             loc[:, 0] += self.up - self.z0
             return keep, loc
-        self.src_ids, s_loc = mine(src)
-        self.rec_ids, r_loc = mine(rec)
+        src_ids, s_loc = mine(src)
+        rec_ids, r_loc = mine(rec)
+        self.prop.set_geometry(s_loc, r_loc)            # a rejected geometry raises here and leaves the rank's state as it was
+        self.src_ids, self.rec_ids = src_ids, rec_ids
         self.nsrc_global, self.nrec_global = len(src), len(rec)
-        self.prop.set_geometry(s_loc, r_loc)
         self._graphs = {}                               # captured loops hold the old list sizes
 
     def _exchange(self, idx):

@@ -340,31 +340,32 @@ using namespace fwi;
 // (set_geometry rewrites their contents in place).
 namespace {
 
+// A device array the plan owns, `cap` elements.  ensure() is the one place that reallocates plan memory: captured graphs
+// hold the old address, so every reallocation drops them.  `slack`: allocate n + n/2 + 16 elements, so that a later
+// geometry of similar size reuses the array; otherwise exactly max(n, 1).
+template <typename T> struct DevArray {
+    T* d = nullptr;
+    size_t cap = 0;
+    int ensure(fwi_fd2d* p, size_t n, bool slack = false);
+    void release() { if (d) cudaFree(d); d = nullptr; cap = 0; }
+};
+
 struct PointList {
-    int n = 0, cap = 0, nbins = 0;
-    int* d_tile_ptr = nullptr; int* d_off = nullptr; int* d_id = nullptr;
-    void release() {
-        if (d_tile_ptr) cudaFree(d_tile_ptr);
-        if (d_off) cudaFree(d_off);
-        if (d_id) cudaFree(d_id);
-        d_tile_ptr = d_off = d_id = nullptr; n = cap = nbins = 0;
-    }
+    int n = 0;
+    DevArray<int> tile_ptr, off, id;
+    void release() { tile_ptr.release(); off.release(); id.release(); n = 0; }
     // what a kernel reads; an absent or empty list is all null, which the kernels skip
     static PointListDev dev(const PointList* pl) {
-        return (pl && pl->n) ? PointListDev{pl->d_tile_ptr, pl->d_off, pl->d_id} : PointListDev{nullptr, nullptr, nullptr};
+        return (pl && pl->n) ? PointListDev{pl->tile_ptr.d, pl->off.d, pl->id.d} : PointListDev{nullptr, nullptr, nullptr};
     }
 };
 
 // A sparse operator in CSR form (fd_interp_*_kernel): rows[j] sums w[e] * in[col[e]] over e in [ptr[j], ptr[j+1]).
 struct Csr {
-    int rows = 0, cap_rows = 0, cap_nnz = 0;
-    int* d_ptr = nullptr; int* d_col = nullptr; float* d_w = nullptr;
-    void release() {
-        if (d_ptr) cudaFree(d_ptr);
-        if (d_col) cudaFree(d_col);
-        if (d_w) cudaFree(d_w);
-        d_ptr = d_col = nullptr; d_w = nullptr; rows = cap_rows = cap_nnz = 0;
-    }
+    int rows = 0;
+    DevArray<int> ptr, col;
+    DevArray<float> w;
+    void release() { ptr.release(); col.release(); w.release(); rows = 0; }
 };
 
 // Off-grid points of one side (spec B7, fwi_fd*_set_positions): `npts` points whose taps land on the side's unique cells,
@@ -483,20 +484,15 @@ struct fwi_fd2d {
     float* fld[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // forward 0..3, adjoint 4..7 (one-step kernels use 0/1 and 4/5)
     CUtensorMap tmap[8];
     float* acc = nullptr;
-    float* snap = nullptr; size_t snap_steps = 0;
-    float* ckpt = nullptr; size_t ckpt_slots = 0;
-    float* resid = nullptr; size_t resid_cap = 0;
-    float* syn = nullptr; size_t syn_cap = 0;
-    float* obs = nullptr; size_t obs_cap = 0;
-    float* wav = nullptr; size_t wav_cap = 0;
-    float* dm = nullptr; size_t dm_cap = 0;   // Born: pitched dm = (2 m / v) dv
+    DevArray<float> snap, ckpt, resid, syn, obs, wav;
+    DevArray<float> dm;               // Born: pitched dm = (2 m / v) dv
     double* d_J = nullptr;
     PointList src, rec;
     PointList src_ext2, src_own2, rec_ext2, rec_own2;   // tb2: binned by the 120 x cz core tiles (+-4 for *_ext2)
     int nsrc = 0, nrec = 0;           // source / receiver cells: the columns of p->wav, p->syn, p->resid
     Interp isrc, irec;                // off-grid points (spec B7) over those cells
-    float* pts = nullptr; size_t pts_cap = 0;     // off grid: gradient synthetics / Gauss-Newton J dv at the receivers
-    float* pres = nullptr; size_t pres_cap = 0;   // off grid: the residual at the receivers
+    DevArray<float> pts;              // off grid: gradient synthetics / Gauss-Newton J dv at the receivers
+    DevArray<float> pres;             // off grid: the residual at the receivers
     size_t mem_limit = 0;             // 0 = automatic (fraction of free memory)
     bool pdl = true;                  // chain 2-D steps with programmatic dependent launch (FWI_PDL=0 turns it off)
     bool pdl_chain = false;           // false right after a kernel that rewrites what a step reads BEFORE its dependency wait (m)
@@ -537,7 +533,18 @@ static void drop_graphs(fwi_fd2d* p) {
     p->graphs.clear();
 }
 
+template <typename T> int DevArray<T>::ensure(fwi_fd2d* p, size_t n, bool slack) {
+    if (d && n <= cap) return FWI_OK;
+    release();
+    drop_graphs(p);
+    const size_t want = slack ? n + n / 2 + 16 : std::max<size_t>(n, 1);
+    FWI_CUDA(cudaMalloc(&d, want * sizeof(T)));
+    cap = want;
+    return FWI_OK;
+}
+
 static void clear_geometry(fwi_fd2d* p) {
+    drop_graphs(p);                   // they hold the addresses of the lists released here
     p->src.release(); p->rec.release();
     p->src_ext2.release(); p->src_own2.release(); p->rec_ext2.release(); p->rec_own2.release();
     p->isrc.release(); p->irec.release();
@@ -644,17 +651,17 @@ static int stage_begin(fwi_fd2d* p, size_t need_ints) {
     sl.used = 0;
     return FWI_OK;
 }
-static int stage_upload(fwi_fd2d* p, int* dst_dev, const int* src, size_t n) {
+// Ensures `a` holds v.size() elements and queues their upload through the slot stage_begin sized (floats travel through
+// the int slot bit for bit).  Contents are rewritten in place on the work stream, ordered after the previous shot's graph.
+template <typename T> static int stage_upload(fwi_fd2d* p, DevArray<T>& a, const std::vector<T>& v, bool slack) {
+    static_assert(sizeof(T) == sizeof(int), "the staging slots hold 4-byte words");
+    int rc = a.ensure(p, v.size(), slack);
+    if (rc || v.empty()) return rc;
     auto& sl = p->stage[p->stage_cur];
-    if (sl.used + n > sl.cap) {          // (bound computed by set_geometry was too small: fall back to a synchronous copy)
-        FWI_CUDA(cudaStreamSynchronize(p->work));
-        FWI_CUDA(cudaMemcpy(dst_dev, src, n * sizeof(int), cudaMemcpyHostToDevice));
-        return FWI_OK;
-    }
     int* h = sl.host + sl.used;
-    memcpy(h, src, n * sizeof(int));
-    sl.used += n;
-    FWI_CUDA(cudaMemcpyAsync(dst_dev, h, n * sizeof(int), cudaMemcpyHostToDevice, p->work));
+    memcpy(h, v.data(), v.size() * sizeof(T));
+    sl.used += v.size();
+    FWI_CUDA(cudaMemcpyAsync(a.d, h, v.size() * sizeof(T), cudaMemcpyHostToDevice, p->work));
     return FWI_OK;
 }
 static int stage_end(fwi_fd2d* p) {
@@ -676,15 +683,8 @@ static TileGrid tile_grid(const fwi_fd2d* p, Family f) {
     return {{p->tile->rows, 1, kBX}, {p->tiles_z, 1, p->tiles_x}, 0};
 }
 
-// Lists each point in every tile whose core widened by `reach` on each side holds it: reach 0 gives the single owning tile,
-// kHalo the tb2 kernel's extended list.  A counting sort keeps the points of a bin in input order.
-static int build_point_list(fwi_fd2d* p, PointList& pl, const TileGrid& g, int reach, int n, const int* iz, const int* iy,
-                            const int* ix, const char* what) {
-    const int nbins = g.count[0] * g.count[1] * g.count[2];
+static int check_points(const fwi_fd2d* p, int n, const int* iz, const int* iy, const int* ix, const char* what) {
     const int z_own1 = p->z_own1 > 0 ? p->z_own1 : p->nz;
-    std::vector<int> tile_ptr(nbins + 1, 0);
-    std::vector<std::pair<int, int>> hits;      // (bin, point) in input order
-    hits.reserve(n);
     for (int i = 0; i < n; ++i) {
         const int yy = iy ? iy[i] : 0;
         FWI_REQUIRE(iz[i] >= 0 && iz[i] < p->nz && ix[i] >= 0 && ix[i] < p->nx && yy >= 0 && yy < p->ny, "%s %d at (z=%d, y=%d, x=%d) is outside the %d x %d x %d grid", what, i, iz[i], yy, ix[i], p->nz, p->ny, p->nx);
@@ -692,7 +692,23 @@ static int build_point_list(fwi_fd2d* p, PointList& pl, const TileGrid& g, int r
         FWI_REQUIRE(iz[i] >= p->z_own0 && iz[i] < z_own1, "%s %d at z=%d is outside the planes [%d, %d) this slab owns", what, i, iz[i], p->z_own0, z_own1);
         // the free surface holds p = 0: a point on it would inject into, or record, a row that stays 0
         FWI_REQUIRE(!p->free_surface || iz[i] >= 1, "%s %d at (z=%d, y=%d, x=%d) lies on the free surface; sources and receivers need z >= 1", what, i, iz[i], yy, ix[i]);
-        const int c[3] = {iz[i] - g.z0, yy, ix[i]};
+    }
+    return FWI_OK;
+}
+
+struct HostList { std::vector<int> tile_ptr, off, id; };
+
+// Lists each (checked) point in every tile whose core widened by `reach` on each side holds it: reach 0 gives the single
+// owning tile, kHalo the tb2 kernel's extended list.  A counting sort keeps the points of a bin in input order.
+static void bin_points(const fwi_fd2d* p, const TileGrid& g, int reach, int n, const int* iz, const int* iy, const int* ix,
+                       HostList& out) {
+    const int nbins = g.count[0] * g.count[1] * g.count[2];
+    std::vector<int>& tile_ptr = out.tile_ptr;
+    tile_ptr.assign(nbins + 1, 0);
+    std::vector<std::pair<int, int>> hits;      // (bin, point) in input order
+    hits.reserve(n);
+    for (int i = 0; i < n; ++i) {
+        const int c[3] = {iz[i] - g.z0, iy ? iy[i] : 0, ix[i]};
         int lo[3], hi[3];
         for (int d = 0; d < 3; ++d) {
             lo[d] = std::max(0, (c[d] - reach) / g.size[d]);
@@ -707,29 +723,14 @@ static int build_point_list(fwi_fd2d* p, PointList& pl, const TileGrid& g, int r
                 }
     }
     for (int t = 0; t < nbins; ++t) tile_ptr[t + 1] += tile_ptr[t];
-    const int tot = std::max(1, tile_ptr[nbins]);
-    std::vector<int> fill(tile_ptr.begin(), tile_ptr.end() - 1), off(tot), id(tot);
+    std::vector<int> fill(tile_ptr.begin(), tile_ptr.end() - 1);
+    out.off.resize(tile_ptr[nbins]);
+    out.id.resize(tile_ptr[nbins]);
     for (const auto& h : hits) {
         const int i = h.second, e = fill[h.first]++;
-        off[e] = (iz[i] * p->ny + (iy ? iy[i] : 0)) * p->px + ix[i];
-        id[e] = i;
+        out.off[e] = (iz[i] * p->ny + (iy ? iy[i] : 0)) * p->px + ix[i];
+        out.id[e] = i;
     }
-    if (pl.nbins != nbins || pl.cap < tot) {     // allocations change -> cached graphs hold stale pointers
-        pl.release();
-        drop_graphs(p);
-        const int cap = tot + tot / 2 + 16;      // slack: the tb2 extended lists vary a little from shot to shot
-        FWI_CUDA(cudaMalloc(&pl.d_tile_ptr, (nbins + 1) * sizeof(int)));
-        FWI_CUDA(cudaMalloc(&pl.d_off, cap * sizeof(int)));
-        FWI_CUDA(cudaMalloc(&pl.d_id, cap * sizeof(int)));
-        pl.cap = cap; pl.nbins = nbins;
-    }
-    // contents are rewritten in place on the work stream, ordered after the previous shot's graph
-    int rc = stage_upload(p, pl.d_tile_ptr, tile_ptr.data(), nbins + 1);
-    if (!rc) rc = stage_upload(p, pl.d_off, off.data(), tot);
-    if (!rc) rc = stage_upload(p, pl.d_id, id.data(), tot);
-    if (rc) return rc;
-    pl.n = tile_ptr[nbins];
-    return FWI_OK;
 }
 
 // Launches the kernel of `mode` of a step-kernel shape, its free-surface instance when `fs`.  With `pdl` it is chained to
@@ -759,7 +760,7 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
         a.inj_vals = inj_vals;
         a.rec = PointList::dev(rec);
         a.rec_out = rec_out;
-        a.dm = p->dm;
+        a.dm = p->dm.d;
         const bool pdl = p->pdl && p->pdl_chain;
         p->pdl_chain = true;
         return launch_shape(*p->tile, mode, p->free_surface, dim3(p->tiles_x, p->tiles_z), pdl, st, p->tmap[cur], a);
@@ -783,19 +784,9 @@ static int launch_step(fwi_fd2d* p, int mode, int cur, float* oldnew, const Poin
     a.flag_peer_up = p->peer_arena[0] ? (int*)((char*)p->peer_arena[0] + p->peer_flags_off[0]) + kSyncFlagDn : nullptr;   // I am its lower neighbour
     a.flag_peer_dn = p->peer_arena[1] ? (int*)((char*)p->peer_arena[1] + p->peer_flags_off[1]) + kSyncFlagUp : nullptr;   // I am its upper neighbour
     a.timeout_cycles = p->slab_timeout_cycles;
-    a.dm = p->dm;
+    a.dm = p->dm.d;
     // (programmatic dependent launch was measured on this kernel too: 2 % at 128^3, nothing from 256^3 up - not used)
     return launch_shape(*p->fd3, mode, p->free_surface, dim3(p->tiles_x, p->tiles_y, p->nzch), false, st, p->tm3[cur], p->tm3_old[oi], p->tm3_m, a);
-}
-
-static int ensure_floats(fwi_fd2d* p, float** ptr, size_t* cap, size_t need_floats) {
-    if (*cap >= need_floats && *ptr) return FWI_OK;
-    if (*ptr) cudaFree(*ptr);
-    *ptr = nullptr; *cap = 0;
-    drop_graphs(p);
-    FWI_CUDA(cudaMalloc(ptr, std::max<size_t>(need_floats, 1) * sizeof(float)));
-    *cap = need_floats;
-    return FWI_OK;
 }
 
 static void other_two(const State& s, int base, int& a, int& b) {
@@ -831,7 +822,7 @@ static int run_forward(fwi_fd2d* p, const float* wavelet, int n0, int n1, float*
         for (; n + 1 < n1; n += 2) {
             int jc, jd;
             other_two(s, 0, jc, jd);
-            float* s1 = save ? p->snap + (size_t)(n - snap_base) * pl : nullptr;
+            float* s1 = save ? p->snap.d + (size_t)(n - snap_base) * pl : nullptr;
             int rc = launch_tb2(p, save ? STEP_FWD_SAVE : STEP_FWD, s, jc, jd, &p->src_ext2, &p->src_own2, wavelet + (size_t)n * p->nsrc,
                                 wavelet + (size_t)(n + 1) * p->nsrc, traces ? &p->rec_own2 : nullptr,
                                 traces ? traces + (size_t)n * p->nrec : nullptr, traces ? traces + (size_t)(n + 1) * p->nrec : nullptr,
@@ -843,7 +834,7 @@ static int run_forward(fwi_fd2d* p, const float* wavelet, int n0, int n1, float*
     // a leftover single step behind a two-steps-per-pass launch reads u_{n-1} written by that very pass: no chaining
     if (p->family == kTb2) p->pdl_chain = false;
     for (; n < n1; ++n) {
-        float* snap = save ? p->snap + (size_t)(n - snap_base) * pl : nullptr;
+        float* snap = save ? p->snap.d + (size_t)(n - snap_base) * pl : nullptr;
         int rc = launch_step(p, save ? STEP_FWD_SAVE : STEP_FWD, s.c, p->fld[s.o], &p->src, wavelet + (size_t)n * p->nsrc,
                              traces ? &p->rec : nullptr, traces ? traces + (size_t)n * p->nrec : nullptr, snap, st);
         if (rc) return rc;
@@ -863,7 +854,7 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
             int jc, jd;
             other_two(s, 4, jc, jd);
             int rc = launch_tb2(p, STEP_ADJ, s, jc, jd, &p->rec_ext2, &p->rec_own2, resid + (size_t)n * p->nrec, resid + (size_t)(n - 1) * p->nrec,
-                                nullptr, nullptr, nullptr, p->snap + (size_t)(n - snap_base) * pl, p->snap + (size_t)(n - 1 - snap_base) * pl, st);
+                                nullptr, nullptr, nullptr, p->snap.d + (size_t)(n - snap_base) * pl, p->snap.d + (size_t)(n - 1 - snap_base) * pl, st);
             if (rc) return rc;
             s = State{jc, jd};
         }
@@ -876,7 +867,7 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
             if (rc) return rc;
             s = State{s.o, s.c};
             rc = launch_step(p, STEP_ADJ2, s.c, p->fld[s.o], &p->rec, resid + (size_t)(n - 1) * p->nrec, nullptr, nullptr,
-                             p->snap + (size_t)(n - 1 - snap_base) * pl, st, p->snap + (size_t)(n - snap_base) * pl);
+                             p->snap.d + (size_t)(n - 1 - snap_base) * pl, st, p->snap.d + (size_t)(n - snap_base) * pl);
             if (rc) return rc;
             s = State{s.o, s.c};
         }
@@ -884,7 +875,7 @@ static int run_adjoint(fwi_fd2d* p, const float* resid, int n0, int n1, size_t s
     if (p->family == kTb2) p->pdl_chain = false;          // see run_forward: leftover step behind a two-step pass
     for (; n >= n0; --n) {
         int rc = launch_step(p, STEP_ADJ, s.c, p->fld[s.o], &p->rec, resid + (size_t)n * p->nrec, nullptr, nullptr,
-                             p->snap + (size_t)(n - snap_base) * pl, st);
+                             p->snap.d + (size_t)(n - snap_base) * pl, st);
         if (rc) return rc;
         s = State{s.o, s.c};
     }
@@ -900,7 +891,7 @@ static int run_born(fwi_fd2d* p, int n0, int n1, size_t snap_base, State& s, flo
     const size_t pl = p->plane();
     for (int n = n0; n < n1; ++n) {
         int rc = launch_step(p, STEP_BORN, s.c, p->fld[s.o], nullptr, nullptr, &p->rec, traces + (size_t)n * p->nrec,
-                             p->snap + (size_t)(n - snap_base) * pl, st);
+                             p->snap.d + (size_t)(n - snap_base) * pl, st);
         if (rc) return rc;
         s = State{s.o, s.c};
     }
@@ -913,8 +904,8 @@ static int run_born(fwi_fd2d* p, int n0, int n1, size_t snap_base, State& s, flo
 static int launch_interp(fwi_fd2d* p, bool gather, const Csr& op, const float* in, int nin, float* out, int nt, cudaStream_t st) {
     if (!op.rows || nt < 1) return FWI_OK;
     const dim3 grid((op.rows + 127) / 128, std::min((nt + kInterpRows - 1) / kInterpRows, 65535));
-    if (gather) fd_interp_gather_kernel<<<grid, 128, 0, st>>>(op.d_ptr, op.d_col, op.d_w, in, nin, out, op.rows, nt);
-    else fd_interp_spread_kernel<<<grid, 128, 0, st>>>(op.d_ptr, op.d_col, op.d_w, in, nin, out, op.rows, nt);
+    if (gather) fd_interp_gather_kernel<<<grid, 128, 0, st>>>(op.ptr.d, op.col.d, op.w.d, in, nin, out, op.rows, nt);
+    else fd_interp_spread_kernel<<<grid, 128, 0, st>>>(op.ptr.d, op.col.d, op.w.d, in, nin, out, op.rows, nt);
     FWI_CUDA(cudaGetLastError());
     p->launches += 1;
     return FWI_OK;
@@ -961,7 +952,7 @@ static int record_forward(fwi_fd2d* p, int nt, cudaStream_t st, State& fs) {
     int rc = zero_state(p, 0, 1, st);
     if (rc) return rc;
     fs = State{0, 1};
-    return run_forward(p, p->wav, 0, nt, p->nrec ? p->syn : nullptr, false, 0, fs, st);
+    return run_forward(p, p->wav.d, 0, nt, p->nrec ? p->syn.d : nullptr, false, 0, fs, st);
 }
 
 // Born modelling of one shot: per segment of S steps the background forward saves its S snapshots (traces -> p->syn)
@@ -974,8 +965,8 @@ static int record_born(fwi_fd2d* p, int nt, int S, cudaStream_t st, State& fs) {
     State bs{4, 5};
     for (int n0 = 0; n0 < nt; n0 += S) {
         const int n1 = std::min(nt, n0 + S);
-        if ((rc = run_forward(p, p->wav, n0, n1, p->syn, true, n0, fs, st))) return rc;
-        if ((rc = run_born(p, n0, n1, n0, bs, p->resid, st))) return rc;
+        if ((rc = run_forward(p, p->wav.d, n0, n1, p->syn.d, true, n0, fs, st))) return rc;
+        if ((rc = run_born(p, n0, n1, n0, bs, p->resid.d, st))) return rc;
     }
     return FWI_OK;
 }
@@ -995,19 +986,19 @@ static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t 
     std::vector<State> seg_state(nseg, fs);
     if (gauss_newton && (rc = zero_state(p, 4, 5, st))) return rc;
     if (nseg == 1) {
-        rc = run_forward(p, p->wav, 0, nt, p->nrec ? p->syn : nullptr, true, 0, fs, st);
+        rc = run_forward(p, p->wav.d, 0, nt, p->nrec ? p->syn.d : nullptr, true, 0, fs, st);
         if (rc) return rc;
-        if (gauss_newton && (rc = run_born(p, 0, nt, 0, bs, p->resid, st))) return rc;
+        if (gauss_newton && (rc = run_born(p, 0, nt, 0, bs, p->resid.d, st))) return rc;
     } else {
         for (int s = 0; s < nseg; ++s) {
             if ((rc = slab_fence(p, st))) return rc;       // the ghost planes of u_n must have arrived before they are saved
-            FWI_CUDA(cudaMemcpyAsync(p->ckpt + (size_t)(2 * s) * pl, p->fld[fs.c], pl * sizeof(float), cudaMemcpyDeviceToDevice, st));
-            FWI_CUDA(cudaMemcpyAsync(p->ckpt + (size_t)(2 * s + 1) * pl, p->fld[fs.o], pl * sizeof(float), cudaMemcpyDeviceToDevice, st));
+            FWI_CUDA(cudaMemcpyAsync(p->ckpt.d + (size_t)(2 * s) * pl, p->fld[fs.c], pl * sizeof(float), cudaMemcpyDeviceToDevice, st));
+            FWI_CUDA(cudaMemcpyAsync(p->ckpt.d + (size_t)(2 * s + 1) * pl, p->fld[fs.o], pl * sizeof(float), cudaMemcpyDeviceToDevice, st));
             seg_state[s] = fs;
             const int n0 = s * seg, n1 = std::min(nt, (s + 1) * seg);
-            rc = run_forward(p, p->wav, n0, n1, p->nrec ? p->syn : nullptr, gauss_newton, n0, fs, st);
+            rc = run_forward(p, p->wav.d, n0, n1, p->nrec ? p->syn.d : nullptr, gauss_newton, n0, fs, st);
             if (rc) return rc;
-            if (gauss_newton && (rc = run_born(p, n0, n1, n0, bs, p->resid, st))) return rc;
+            if (gauss_newton && (rc = run_born(p, n0, n1, n0, bs, p->resid.d, st))) return rc;
         }
     }
     FWI_CUDA(cudaMemsetAsync(p->d_J, 0, sizeof(double), st));
@@ -1016,15 +1007,15 @@ static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t 
         // synthetics (Gauss-Newton: J dv), take the residual there, spread it (J dv) back into p->resid.
         const int np = p->irec.npts;
         const size_t ntp = (size_t)nt * np;
-        if ((rc = launch_interp(p, true, p->irec.by_point, gauss_newton ? p->resid : p->syn, p->nrec, p->pts, nt, st))) return rc;
+        if ((rc = launch_interp(p, true, p->irec.by_point, gauss_newton ? p->resid.d : p->syn.d, p->nrec, p->pts.d, nt, st))) return rc;
         if (ntp && !gauss_newton) {
-            fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntp + 255) / 256), 256, 0, st>>>(p->pts, p->obs, (int64_t)ntp, p->pres, p->d_J);
+            fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntp + 255) / 256), 256, 0, st>>>(p->pts.d, p->obs.d, (int64_t)ntp, p->pres.d, p->d_J);
             FWI_CUDA(cudaGetLastError());
             p->launches += 1;
         }
-        if ((rc = launch_interp(p, false, p->irec.by_cell, gauss_newton ? p->pts : p->pres, np, p->resid, nt, st))) return rc;
+        if ((rc = launch_interp(p, false, p->irec.by_cell, gauss_newton ? p->pts.d : p->pres.d, np, p->resid.d, nt, st))) return rc;
     } else if (ntr && !gauss_newton) {
-        fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntr + 255) / 256), 256, 0, st>>>(p->syn, p->obs, (int64_t)ntr, p->resid, p->d_J);
+        fd_residual_kernel<<<(unsigned)std::min<size_t>(1024, (ntr + 255) / 256), 256, 0, st>>>(p->syn.d, p->obs.d, (int64_t)ntr, p->resid.d, p->d_J);
         FWI_CUDA(cudaGetLastError());
         p->launches += 1;
     }
@@ -1032,16 +1023,16 @@ static int record_gradient(fwi_fd2d* p, int nt, int seg, int nseg, cudaStream_t 
     FWI_CUDA(cudaMemsetAsync(p->acc, 0, pl * sizeof(float), st));
     State as{4, 5};
     if (nseg == 1) {
-        rc = run_adjoint(p, p->resid, 0, nt, 0, as, st);
+        rc = run_adjoint(p, p->resid.d, 0, nt, 0, as, st);
         if (rc) return rc;
     } else {
         for (int s = nseg - 1; s >= 0; --s) {
             const int n0 = s * seg, n1 = std::min(nt, (s + 1) * seg);
             fs = seg_state[s];
-            if ((rc = restore_state(p, fs, p->ckpt + (size_t)(2 * s) * pl, p->ckpt + (size_t)(2 * s + 1) * pl, st))) return rc;
-            rc = run_forward(p, p->wav, n0, n1, nullptr, true, n0, fs, st);     // recompute w_n for this segment
+            if ((rc = restore_state(p, fs, p->ckpt.d + (size_t)(2 * s) * pl, p->ckpt.d + (size_t)(2 * s + 1) * pl, st))) return rc;
+            rc = run_forward(p, p->wav.d, n0, n1, nullptr, true, n0, fs, st);     // recompute w_n for this segment
             if (rc) return rc;
-            rc = run_adjoint(p, p->resid, n0, n1, n0, as, st);
+            rc = run_adjoint(p, p->resid.d, n0, n1, n0, as, st);
             if (rc) return rc;
         }
     }
@@ -1234,15 +1225,7 @@ int fwi_fd2d_destroy(fwi_fd2d* p) {
     if (p->work) cudaStreamSynchronize(p->work);
     drop_graphs(p);
     cudaFree(p->arena); cudaFree(p->gx); cudaFree(p->gz); cudaFree(p->gy); cudaFree(p->d_J);
-    if (p->snap) cudaFree(p->snap);
-    if (p->ckpt) cudaFree(p->ckpt);
-    if (p->resid) cudaFree(p->resid);
-    if (p->syn) cudaFree(p->syn);
-    if (p->obs) cudaFree(p->obs);
-    if (p->wav) cudaFree(p->wav);
-    if (p->dm) cudaFree(p->dm);
-    if (p->pts) cudaFree(p->pts);
-    if (p->pres) cudaFree(p->pres);
+    for (DevArray<float>* a : {&p->snap, &p->ckpt, &p->resid, &p->syn, &p->obs, &p->wav, &p->dm, &p->pts, &p->pres}) a->release();
     clear_geometry(p);
     for (int s = 0; s < 2; ++s) if (p->peer_arena[s] && p->peer_ipc[s]) cudaIpcCloseMemHandle(p->peer_arena[s]);
     if (p->ev_in) cudaEventDestroy(p->ev_in);
@@ -1320,43 +1303,6 @@ int fwi_fd2d_set_model(fwi_fd2d* p, const float* v_dev, void* stream) {
     return leave(p, user);
 }
 
-// Ints that staging the point lists of `npts` sources and receivers takes: 2 + 4 lists; a tb2 point sits in <= 4 tiles.
-static size_t bin_staging(const fwi_fd2d* p, size_t npts) {
-    const size_t bins = (size_t)std::max({p->tiles_x * p->tiles_y * p->nzch, p->tiles_x * p->tiles_z, p->tiles_x2 * p->tiles_z2}) + 1;
-    return 6 * bins + 2 * 10 * (npts + 16);
-}
-
-// Bins the source and receiver cells into the point lists of every kernel family the plan runs (uploads staged by the caller).
-static int bin_points(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
-                      const int* rec_z, const int* rec_y, const int* rec_x) {
-    if (nsrc != p->nsrc || nrec != p->nrec) drop_graphs(p);
-    const TileGrid step = tile_grid(p, p->family == k3D ? k3D : kTile);     // tb2 plans run the tile kernel for single steps
-    int rc = build_point_list(p, p->src, step, 0, nsrc, src_z, src_y, src_x, "source");
-    if (rc) return rc;
-    rc = build_point_list(p, p->rec, step, 0, nrec, rec_z, rec_y, rec_x, "receiver");
-    if (rc) return rc;
-    if (p->family == kTb2) {
-        const TileGrid pass = tile_grid(p, kTb2);
-        if ((rc = build_point_list(p, p->src_ext2, pass, kHalo, nsrc, src_z, src_y, src_x, "source"))) return rc;
-        if ((rc = build_point_list(p, p->src_own2, pass, 0, nsrc, src_z, src_y, src_x, "source"))) return rc;
-        if ((rc = build_point_list(p, p->rec_ext2, pass, kHalo, nrec, rec_z, rec_y, rec_x, "receiver"))) return rc;
-        if ((rc = build_point_list(p, p->rec_own2, pass, 0, nrec, rec_z, rec_y, rec_x, "receiver"))) return rc;
-    }
-    p->nsrc = nsrc; p->nrec = nrec;
-    return FWI_OK;
-}
-
-static int set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
-                        const int* rec_z, const int* rec_y, const int* rec_x) {
-    FWI_REQUIRE(p, "fwi_fd_set_geometry: NULL plan");
-    FWI_REQUIRE(nsrc >= 0 && nrec >= 0 && (nsrc == 0 || (src_z && src_x)) && (nrec == 0 || (rec_z && rec_x)), "fwi_fd_set_geometry: bad arguments");
-    DeviceGuard g(p->device);
-    p->isrc.npts = p->irec.npts = -1;         // points are cells again
-    int rc = stage_begin(p, bin_staging(p, (size_t)nsrc + nrec));
-    if (rc || (rc = bin_points(p, nsrc, src_z, src_y, src_x, nrec, rec_z, rec_y, rec_x))) return rc;
-    return stage_end(p);
-}
-
 // ---- off-grid points (spec B7, tests/offgrid_reference.py) ---------------------------------------------------------
 // Kaiser window parameter of the windowed-sinc taps: the b on a 0.01 grid that minimises
 // E(b) = max |sum_k w_k(f) exp(i kappa d_k) - 1| over kappa in [0, 2 pi / 3], f in [0, 1)  (E(4.06) = 8.79e-3).
@@ -1386,17 +1332,18 @@ static std::vector<std::pair<int, double>> axis_taps(double x, int n, bool fold)
     return t;
 }
 
+struct HostCsr { std::vector<int> ptr, col; std::vector<float> w; };
+
 // One side's off-grid points as cells and the two CSR forms of the operator W (points x cells).
 struct SideTaps {
     std::vector<int> cz, cy, cx;                          // the unique cells, in ascending linear offset
-    std::vector<int> pt_ptr, pt_col, cell_ptr, cell_col;
-    std::vector<float> pt_w, cell_w;
+    HostCsr by_point, by_cell;
 };
 
 static int build_side(const fwi_fd2d* p, int n, const double* z, const double* y, const double* x, const char* what, SideTaps& s) {
     const double dims[3] = {(double)p->nz, (double)p->ny, (double)p->nx};
     std::vector<std::pair<int64_t, std::pair<int, double>>> taps;        // (cell offset, (point, weight)), point-major
-    s.pt_ptr.assign(1, 0);
+    s.by_point.ptr.assign(1, 0);
     for (int i = 0; i < n; ++i) {
         const double c[3] = {z[i], y ? y[i] : 0.0, x[i]};
         FWI_REQUIRE(std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]), "%s %d at (z=%g, y=%g, x=%g) is not finite", what, i, c[0], c[1], c[2]);
@@ -1408,7 +1355,7 @@ static int build_side(const fwi_fd2d* p, int n, const double* z, const double* y
             for (const auto& b : ty)
                 for (const auto& e : tx)
                     taps.push_back({((int64_t)a.first * p->ny + b.first) * p->nx + e.first, {i, a.second * b.second * e.second}});
-        s.pt_ptr.push_back((int)taps.size());
+        s.by_point.ptr.push_back((int)taps.size());
     }
     std::vector<int64_t> cells(taps.size());
     for (size_t e = 0; e < taps.size(); ++e) cells[e] = taps[e].first;
@@ -1422,43 +1369,100 @@ static int build_side(const fwi_fd2d* p, int n, const double* z, const double* y
         s.cz[c] = (int)(cells[c] / p->nx / p->ny);
     }
     // a point's taps come in ascending cell order and never repeat a cell (axis_taps merged them per axis)
-    s.pt_col.resize(taps.size()); s.pt_w.resize(taps.size());
-    s.cell_ptr.assign(nc + 1, 0);
+    s.by_point.col.resize(taps.size()); s.by_point.w.resize(taps.size());
+    s.by_cell.ptr.assign(nc + 1, 0);
     for (size_t e = 0; e < taps.size(); ++e) {
-        s.pt_col[e] = (int)(std::lower_bound(cells.begin(), cells.end(), taps[e].first) - cells.begin());
-        s.pt_w[e] = (float)taps[e].second.second;
-        s.cell_ptr[s.pt_col[e] + 1]++;
+        s.by_point.col[e] = (int)(std::lower_bound(cells.begin(), cells.end(), taps[e].first) - cells.begin());
+        s.by_point.w[e] = (float)taps[e].second.second;
+        s.by_cell.ptr[s.by_point.col[e] + 1]++;
     }
-    for (int c = 0; c < nc; ++c) s.cell_ptr[c + 1] += s.cell_ptr[c];
-    std::vector<int> fill(s.cell_ptr.begin(), s.cell_ptr.end() - 1);
-    s.cell_col.resize(taps.size()); s.cell_w.resize(taps.size());
+    for (int c = 0; c < nc; ++c) s.by_cell.ptr[c + 1] += s.by_cell.ptr[c];
+    std::vector<int> fill(s.by_cell.ptr.begin(), s.by_cell.ptr.end() - 1);
+    s.by_cell.col.resize(taps.size()); s.by_cell.w.resize(taps.size());
     for (size_t e = 0; e < taps.size(); ++e) {                           // points of a cell in ascending order
-        const int k = fill[s.pt_col[e]]++;
-        s.cell_col[k] = taps[e].second.first;
-        s.cell_w[k] = s.pt_w[e];
+        const int k = fill[s.by_point.col[e]]++;
+        s.by_cell.col[k] = taps[e].second.first;
+        s.by_cell.w[k] = s.by_point.w[e];
     }
     return FWI_OK;
 }
 
-static size_t csr_staging(const SideTaps& s) { return s.pt_ptr.size() + s.cell_ptr.size() + 4 * s.pt_col.size(); }
+// ---- installing a geometry: build it on the host, then commit it, so that a rejected one leaves the plan as it was ----
+// The cells of both sides binned into every point list the plan's family runs and, off grid, both sides' operators.
+struct HostGeometry {
+    int nsrc = 0, nrec = 0;                   // cells
+    int psrc = -1, prec = -1;                 // off-grid points (Interp::npts)
+    HostList src, rec, src_ext2, src_own2, rec_ext2, rec_own2;
+    SideTaps s, r;
+};
 
-static int upload_csr(fwi_fd2d* p, Csr& c, const std::vector<int>& ptr, const std::vector<int>& col, const std::vector<float>& w) {
-    const int rows = (int)ptr.size() - 1, nnz = (int)col.size();
-    if (c.cap_rows < rows || c.cap_nnz < std::max(nnz, 1)) {       // allocations change -> cached graphs hold stale pointers
-        c.release();
-        drop_graphs(p);
-        const int cr = rows + rows / 2 + 16, cn = nnz + nnz / 2 + 16;
-        FWI_CUDA(cudaMalloc(&c.d_ptr, (cr + 1) * sizeof(int)));
-        FWI_CUDA(cudaMalloc(&c.d_col, cn * sizeof(int)));
-        FWI_CUDA(cudaMalloc(&c.d_w, cn * sizeof(float)));
-        c.cap_rows = cr; c.cap_nnz = cn;
+// Checks the cells, all sources and then all receivers, and bins them for every kernel family the plan runs.
+static int bin_geometry(const fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
+                        const int* rec_z, const int* rec_y, const int* rec_x, HostGeometry& g) {
+    int rc = check_points(p, nsrc, src_z, src_y, src_x, "source");
+    if (rc || (rc = check_points(p, nrec, rec_z, rec_y, rec_x, "receiver"))) return rc;
+    g.nsrc = nsrc; g.nrec = nrec;
+    const TileGrid step = tile_grid(p, p->family == k3D ? k3D : kTile);     // tb2 plans run the tile kernel for single steps
+    bin_points(p, step, 0, nsrc, src_z, src_y, src_x, g.src);
+    bin_points(p, step, 0, nrec, rec_z, rec_y, rec_x, g.rec);
+    if (p->family == kTb2) {
+        const TileGrid pass = tile_grid(p, kTb2);
+        bin_points(p, pass, kHalo, nsrc, src_z, src_y, src_x, g.src_ext2);
+        bin_points(p, pass, 0, nsrc, src_z, src_y, src_x, g.src_own2);
+        bin_points(p, pass, kHalo, nrec, rec_z, rec_y, rec_x, g.rec_ext2);
+        bin_points(p, pass, 0, nrec, rec_z, rec_y, rec_x, g.rec_own2);
     }
-    int rc = stage_upload(p, c.d_ptr, ptr.data(), ptr.size());
-    // (the weights travel through the int staging buffer bit for bit)
-    if (!rc && nnz) rc = stage_upload(p, c.d_col, col.data(), nnz);
-    if (!rc && nnz) rc = stage_upload(p, (int*)c.d_w, (const int*)w.data(), nnz);
-    c.rows = rows;
+    return FWI_OK;
+}
+
+// (slack: the tb2 extended lists vary a little from shot to shot)
+static int upload_list(fwi_fd2d* p, PointList& pl, const HostList& h) {
+    int rc = stage_upload(p, pl.tile_ptr, h.tile_ptr, false);
+    if (!rc) rc = stage_upload(p, pl.off, h.off, true);
+    if (!rc) rc = stage_upload(p, pl.id, h.id, true);
     return rc;
+}
+static int upload_csr(fwi_fd2d* p, Csr& c, const HostCsr& h) {
+    int rc = stage_upload(p, c.ptr, h.ptr, true);
+    if (!rc) rc = stage_upload(p, c.col, h.col, true);
+    if (!rc) rc = stage_upload(p, c.w, h.w, true);
+    return rc;
+}
+
+// Uploads every array of a built geometry through one staging slot, then switches the plan to it.  A failed CUDA call
+// leaves the plan without a geometry rather than with parts of two.
+static int commit_geometry(fwi_fd2d* p, const HostGeometry& g) {
+    DeviceGuard dg(p->device);
+    const std::pair<PointList*, const HostList*> lists[] = {{&p->src, &g.src}, {&p->rec, &g.rec}, {&p->src_ext2, &g.src_ext2},
+                                                            {&p->src_own2, &g.src_own2}, {&p->rec_ext2, &g.rec_ext2}, {&p->rec_own2, &g.rec_own2}};
+    const std::pair<Csr*, const HostCsr*> ops[] = {{&p->isrc.by_point, &g.s.by_point}, {&p->isrc.by_cell, &g.s.by_cell},
+                                                   {&p->irec.by_point, &g.r.by_point}, {&p->irec.by_cell, &g.r.by_cell}};
+    const int nlists = p->family == kTb2 ? 6 : 2, nops = g.psrc >= 0 ? 4 : 0;
+    size_t ints = 0;
+    for (int k = 0; k < nlists; ++k) ints += lists[k].second->tile_ptr.size() + lists[k].second->off.size() + lists[k].second->id.size();
+    for (int k = 0; k < nops; ++k) ints += ops[k].second->ptr.size() + ops[k].second->col.size() + ops[k].second->w.size();
+    if (g.nsrc != p->nsrc || g.nrec != p->nrec) drop_graphs(p);
+    int rc = stage_begin(p, ints);
+    for (int k = 0; k < nlists && !rc; ++k) rc = upload_list(p, *lists[k].first, *lists[k].second);
+    for (int k = 0; k < nops && !rc; ++k) rc = upload_csr(p, *ops[k].first, *ops[k].second);
+    if (!rc) {
+        for (int k = 0; k < nlists; ++k) lists[k].first->n = lists[k].second->tile_ptr.back();
+        for (int k = 0; k < nops; ++k) ops[k].first->rows = (int)ops[k].second->ptr.size() - 1;
+        p->nsrc = g.nsrc; p->nrec = g.nrec;
+        p->isrc.npts = g.psrc; p->irec.npts = g.prec;
+        rc = stage_end(p);
+    }
+    if (rc) clear_geometry(p);
+    return rc;
+}
+
+static int set_geometry(fwi_fd2d* p, int nsrc, const int* src_z, const int* src_y, const int* src_x, int nrec,
+                        const int* rec_z, const int* rec_y, const int* rec_x) {
+    FWI_REQUIRE(p, "fwi_fd_set_geometry: NULL plan");
+    FWI_REQUIRE(nsrc >= 0 && nrec >= 0 && (nsrc == 0 || (src_z && src_x)) && (nrec == 0 || (rec_z && rec_x)), "fwi_fd_set_geometry: bad arguments");
+    HostGeometry g;                           // (psrc = prec = -1: points are cells again)
+    const int rc = bin_geometry(p, nsrc, src_z, src_y, src_x, nrec, rec_z, rec_y, rec_x, g);
+    return rc ? rc : commit_geometry(p, g);
 }
 
 static int set_positions(fwi_fd2d* p, int nsrc, const double* src_z, const double* src_y, const double* src_x, int nrec,
@@ -1467,19 +1471,14 @@ static int set_positions(fwi_fd2d* p, int nsrc, const double* src_z, const doubl
     FWI_REQUIRE(nsrc >= 0 && nrec >= 0 && (nsrc == 0 || (src_z && src_x)) && (nrec == 0 || (rec_z && rec_x)), "fwi_fd_set_positions: bad arguments");
     // a point's taps may straddle two slabs, and a slab's residual would miss the part of a trace another rank samples
     FWI_REQUIRE(!p->peers(), "fwi_fd_set_positions: not available on a plan connected as a peer-memory slab");
-    SideTaps s, r;
-    int rc = build_side(p, nsrc, src_z, src_y, src_x, "source", s);
-    if (rc || (rc = build_side(p, nrec, rec_z, rec_y, rec_x, "receiver", r))) return rc;
-    DeviceGuard g(p->device);
-    p->isrc.npts = p->irec.npts = -1;
-    const int ncs = (int)s.cz.size(), ncr = (int)r.cz.size();
-    if ((rc = stage_begin(p, bin_staging(p, (size_t)ncs + ncr) + csr_staging(s) + csr_staging(r)))) return rc;
-    if ((rc = bin_points(p, ncs, s.cz.data(), s.cy.data(), s.cx.data(), ncr, r.cz.data(), r.cy.data(), r.cx.data()))) return rc;
-    if ((rc = upload_csr(p, p->isrc.by_point, s.pt_ptr, s.pt_col, s.pt_w)) || (rc = upload_csr(p, p->isrc.by_cell, s.cell_ptr, s.cell_col, s.cell_w)) ||
-        (rc = upload_csr(p, p->irec.by_point, r.pt_ptr, r.pt_col, r.pt_w)) || (rc = upload_csr(p, p->irec.by_cell, r.cell_ptr, r.cell_col, r.cell_w)))
+    HostGeometry g;
+    int rc = build_side(p, nsrc, src_z, src_y, src_x, "source", g.s);
+    if (rc || (rc = build_side(p, nrec, rec_z, rec_y, rec_x, "receiver", g.r)) ||
+        (rc = bin_geometry(p, (int)g.s.cz.size(), g.s.cz.data(), g.s.cy.data(), g.s.cx.data(), (int)g.r.cz.size(), g.r.cz.data(),
+                           g.r.cy.data(), g.r.cx.data(), g)))
         return rc;
-    p->isrc.npts = nsrc; p->irec.npts = nrec;
-    return stage_end(p);
+    g.psrc = nsrc; g.prec = nrec;
+    return commit_geometry(p, g);
 }
 
 int fwi_fd2d_set_positions(fwi_fd2d* p, int nsrc, const double* src_z, const double* src_x, int nrec, const double* rec_z,
@@ -1540,7 +1539,7 @@ static int prepare(fwi_fd2d* p, Op op, int nt, Split& split) {
         split = p->split;
     } else if (adjoint) {
         size_t budget = 0, planes = 0;
-        if ((rc = storage_budget(p, p->snap_steps + p->ckpt_slots, budget, planes))) return rc;     // both in floats
+        if ((rc = storage_budget(p, p->snap.cap + p->ckpt.cap, budget, planes))) return rc;
         if ((size_t)nt > planes) {
             // segment length S with S + 2*ceil(nt/S) planes minimal-ish: start from sqrt(2 nt)
             split.seg = std::max(1, (int)std::ceil(std::sqrt(2.0 * nt)));
@@ -1550,21 +1549,21 @@ static int prepare(fwi_fd2d* p, Op op, int nt, Split& split) {
     } else if (op == kBorn) {
         const int S = std::min(nt, kBornSeg);
         size_t budget = 0, planes = (size_t)S;
-        if ((p->mem_limit || p->snap_steps < (size_t)S * pl) && (rc = storage_budget(p, p->snap_steps, budget, planes))) return rc;
+        if ((p->mem_limit || p->snap.cap < (size_t)S * pl) && (rc = storage_budget(p, p->snap.cap, budget, planes))) return rc;
         FWI_REQUIRE(planes >= 1, "fwi_fd2d_born: the memory limit holds no snapshot plane of %zu bytes", pl * sizeof(float));
         split.seg = (int)std::min<size_t>((size_t)S, planes);
         split.nseg = (nt + split.seg - 1) / split.seg;
     }
-    if (op != kForward && (rc = ensure_floats(p, &p->snap, &p->snap_steps, (size_t)split.seg * pl))) return rc;   // snap_steps counts floats
-    if (adjoint && split.nseg > 1 && (rc = ensure_floats(p, &p->ckpt, &p->ckpt_slots, (size_t)split.nseg * 2 * pl))) return rc;
-    if (op != kForward && (rc = ensure_floats(p, &p->resid, &p->resid_cap, ntr))) return rc;
-    if ((rc = ensure_floats(p, &p->syn, &p->syn_cap, ntr))) return rc;
-    if (adjoint && (rc = ensure_floats(p, &p->obs, &p->obs_cap, ntp))) return rc;
+    if (op != kForward && (rc = p->snap.ensure(p, (size_t)split.seg * pl))) return rc;
+    if (adjoint && split.nseg > 1 && (rc = p->ckpt.ensure(p, (size_t)split.nseg * 2 * pl))) return rc;
+    if (op != kForward && (rc = p->resid.ensure(p, ntr))) return rc;
+    if ((rc = p->syn.ensure(p, ntr))) return rc;
+    if (adjoint && (rc = p->obs.ensure(p, ntp))) return rc;
     if (adjoint && p->irec.npts >= 0 &&
-        ((rc = ensure_floats(p, &p->pts, &p->pts_cap, ntp)) || (rc = ensure_floats(p, &p->pres, &p->pres_cap, ntp)))) return rc;
-    if ((rc = ensure_floats(p, &p->wav, &p->wav_cap, (size_t)nt * p->nsrc))) return rc;
+        ((rc = p->pts.ensure(p, ntp)) || (rc = p->pres.ensure(p, ntp)))) return rc;
+    if ((rc = p->wav.ensure(p, (size_t)nt * p->nsrc))) return rc;
     if (adjoint) { p->split_nt = nt; p->split_limit = p->mem_limit; p->split = split; }      // buffers exist now
-    if ((op == kBorn || op == kGaussNewton) && (rc = ensure_floats(p, &p->dm, &p->dm_cap, pl))) return rc;
+    if ((op == kBorn || op == kGaussNewton) && (rc = p->dm.ensure(p, pl))) return rc;
     return FWI_OK;
 }
 
@@ -1580,7 +1579,7 @@ static int launch_finalize(fwi_fd2d* p, float* grad, cudaStream_t st) {
 // the buffer's address)
 static int stage_dm(fwi_fd2d* p, const float* dv_dev) {
     dim3 grid(p->rows(), (p->px + 127) / 128);
-    fd_dm_kernel<<<grid, 128, 0, p->work>>>(dv_dev, p->m, p->vp, p->rows(), p->nx, p->px, p->dm);
+    fd_dm_kernel<<<grid, 128, 0, p->work>>>(dv_dev, p->m, p->vp, p->rows(), p->nx, p->px, p->dm.d);
     FWI_CUDA(cudaGetLastError());
     return FWI_OK;
 }
@@ -1603,7 +1602,7 @@ static int copy_traces(fwi_fd2d* p, float* dst, const float* cells, bool gathere
     const size_t n = (size_t)nt * rec_points(p);
     if (!n) return FWI_OK;
     if (p->irec.npts >= 0 && !gathered) return launch_interp(p, true, p->irec.by_point, cells, p->nrec, dst, nt, p->work);
-    FWI_CUDA(cudaMemcpyAsync(dst, p->irec.npts >= 0 ? p->pts : cells, n * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    FWI_CUDA(cudaMemcpyAsync(dst, p->irec.npts >= 0 ? p->pts.d : cells, n * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
     return FWI_OK;
 }
 
@@ -1616,19 +1615,19 @@ static int run_shot(fwi_fd2d* p, Op op, int nt, void* stream, const ShotIO& io) 
     if ((rc = prepare(p, op, nt, split)) || (rc = enter(p, user))) return rc;
     const size_t nw = (size_t)nt * p->nsrc, ntp = (size_t)nt * rec_points(p);
     if (p->isrc.npts >= 0) {          // off grid (spec B7): the cells' wavelets are W_s^T times the points'
-        if ((rc = launch_interp(p, false, p->isrc.by_cell, io.wavelet, p->isrc.npts, p->wav, nt, p->work))) return rc;
+        if ((rc = launch_interp(p, false, p->isrc.by_cell, io.wavelet, p->isrc.npts, p->wav.d, nt, p->work))) return rc;
     } else if (nw) {
-        FWI_CUDA(cudaMemcpyAsync(p->wav, io.wavelet, nw * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+        FWI_CUDA(cudaMemcpyAsync(p->wav.d, io.wavelet, nw * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
     }
-    if (io.obs && ntp) FWI_CUDA(cudaMemcpyAsync(p->obs, io.obs, ntp * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
+    if (io.obs && ntp) FWI_CUDA(cudaMemcpyAsync(p->obs.d, io.obs, ntp * sizeof(float), cudaMemcpyDeviceToDevice, p->work));
     if (io.dv && (rc = stage_dm(p, io.dv))) return rc;
     if ((rc = run_cached(p, op, nt, split))) return rc;
     if (io.image) {
         if ((rc = launch_finalize(p, io.image, p->work))) return rc;
         p->launches += 1;
     }
-    if (io.dtraces && (rc = copy_traces(p, io.dtraces, p->resid, op == kGaussNewton, nt))) return rc;
-    if (io.traces && (rc = copy_traces(p, io.traces, p->syn, op == kGradient, nt))) return rc;
+    if (io.dtraces && (rc = copy_traces(p, io.dtraces, p->resid.d, op == kGaussNewton, nt))) return rc;
+    if (io.traces && (rc = copy_traces(p, io.traces, p->syn.d, op == kGradient, nt))) return rc;
     if (io.misfit) FWI_CUDA(cudaMemcpyAsync(io.misfit, p->d_J, sizeof(double), cudaMemcpyDeviceToHost, p->work));
     if ((rc = leave(p, user))) return rc;
     if (io.misfit) FWI_CUDA(cudaStreamSynchronize(p->work));
@@ -1736,7 +1735,7 @@ int fwi_fd_reserve_snapshots(fwi_fd2d* p, int nsteps) {
     FWI_REQUIRE(p && nsteps >= 0, "fwi_fd_reserve_snapshots: bad arguments");
     DeviceGuard g(p->device);
     FWI_CUDA(cudaStreamSynchronize(p->work));
-    return ensure_floats(p, &p->snap, &p->snap_steps, (size_t)nsteps * p->plane());
+    return p->snap.ensure(p, (size_t)nsteps * p->plane());
 }
 
 // Zero the wavefield pair (0 = forward, 1 = adjoint; the adjoint pair also clears the imaging accumulator).
@@ -1760,7 +1759,7 @@ int fwi_fd_step(fwi_fd2d* p, int mode, int cur, const float* inj_vals_dev, float
     FWI_REQUIRE(mode >= 0 && mode <= 2 && (cur == 0 || cur == 1), "fwi_fd_step: bad mode / cur");
     FWI_REQUIRE(p->irec.npts < 0, "fwi_fd_step: the plan holds off-grid positions (fwi_fd*_set_positions); single steps take the integer geometry");
     p->pdl_chain = false;             // caller-driven loop: other kernels (halo exchange, resets) sit between the steps
-    FWI_REQUIRE(mode == 0 || (snap_index >= 0 && (size_t)(snap_index + 1) * p->plane() <= p->snap_steps), "fwi_fd_step: snapshot %lld not reserved", (long long)snap_index);
+    FWI_REQUIRE(mode == 0 || (snap_index >= 0 && (size_t)(snap_index + 1) * p->plane() <= p->snap.cap), "fwi_fd_step: snapshot %lld not reserved", (long long)snap_index);
     DeviceGuard g(p->device);
     if (p->geom_pending) {
         // (not while the caller captures a graph: it synchronised before starting the capture, and an event recorded
@@ -1770,7 +1769,7 @@ int fwi_fd_step(fwi_fd2d* p, int mode, int cur, const float* inj_vals_dev, float
         if (cs == cudaStreamCaptureStatusNone) { FWI_CUDA(cudaStreamWaitEvent((cudaStream_t)stream, p->ev_geom, 0)); p->geom_pending = false; }
     }
     const int base = (mode == STEP_ADJ) ? 4 : 0;
-    float* snap = (mode == 0) ? nullptr : p->snap + (size_t)snap_index * p->plane();
+    float* snap = (mode == 0) ? nullptr : p->snap.d + (size_t)snap_index * p->plane();
     int rc = launch_step(p, mode, base + cur, p->fld[base + (cur ^ 1)], mode == STEP_ADJ ? &p->rec : &p->src, inj_vals_dev,
                          (mode != STEP_ADJ && rec_out_dev) ? &p->rec : nullptr, rec_out_dev, snap, (cudaStream_t)stream);
     if (rc) return rc;

@@ -185,7 +185,8 @@ int fwi_fd2d_set_graphs(fwi_fd2d* plan, int enable);
 int fwi_fd2d_set_memory_limit(fwi_fd2d* plan, uint64_t bytes);
 /* v_dev: (nz, nx) fp32 velocities, dense.  Builds m = (v dt / h)^2 in the pitched layout (fd_oracle B1). */
 int fwi_fd2d_set_model(fwi_fd2d* plan, const float* v_dev, void* stream);
-/* One shot's acquisition: integer grid indices of sources and receivers (host arrays; fd_oracle B2). */
+/* One shot's acquisition: integer grid indices of sources and receivers (host arrays; fd_oracle B2).
+ * On FWI_EINVAL the plan keeps the geometry it had. */
 int fwi_fd2d_set_geometry(fwi_fd2d* plan, int nsrc, const int* src_z_host, const int* src_x_host,
                           int nrec, const int* rec_z_host, const int* rec_x_host);
 /* Forward model: nt leapfrog steps from rest; wavelet_dev (nt, nsrc); traces_dev (nt, nrec) receives
@@ -235,7 +236,7 @@ int fwi_fd3d_set_geometry(fwi_fd2d* plan, int nsrc, const int* src_z_host, const
  * wavelet; a gradient or Gauss-Newton product one gather and one spread of the residual (J dv) inside its graph; a
  * forward or Born call one gather per trace array it returns.  FWI_EINVAL, naming the point, for a coordinate that is
  * not finite, outside the grid or at z <= 0 under a free surface; FWI_EINVAL on a plan connected as a peer-memory slab;
- * fwi_fd_step is FWI_EINVAL while the plan holds positions. */
+ * fwi_fd_step is FWI_EINVAL while the plan holds positions.  On FWI_EINVAL the plan keeps the geometry it had. */
 int fwi_fd2d_set_positions(fwi_fd2d* plan, int nsrc, const double* src_z_host, const double* src_x_host,
                            int nrec, const double* rec_z_host, const double* rec_x_host);
 int fwi_fd3d_set_positions(fwi_fd2d* plan, int nsrc, const double* src_z_host, const double* src_y_host,
